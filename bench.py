@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the reference's headline workload on B200, measured as the driver contract asks.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--bases G]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--bases G] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): synthetic hg19-sized genome (3.1 Gb, 22 chromosomes, ~3 % N,
 50 % lower case), 10 kb windows (310 k), pentanucleotide AND trinucleotide context maps with genome
@@ -55,10 +55,17 @@ def emit_json(line):
     out.flush()
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=30)
+    ap.add_argument("--steps", type=positive_int, default=30, help="timed steps of each timed leg")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--bases", type=float, default=3.1e9, help="genome size per GPU (debug override)")
@@ -70,6 +77,8 @@ def parse_args():
                          "(fused, falls back to nccl when symmetric memory is unavailable) or one NCCL all-gather")
     ap.add_argument("--scaling", default="auto", choices=["auto", "strong", "weak"],
                     help="N > 1: strong = ONE 3.1 Gb genome range-sharded over the ranks (default), weak = one genome per rank")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="single process only: after the timed steps, write what the last one computed to DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -183,8 +192,28 @@ def build_workload(total_bases, seed, device):
     g_chrom, g_strand, g_ptr, g_bs, g_be = pipeline.synth_genes(N_GENES, lengths, WINDOW, seed + 200)
     owner = np.repeat(np.arange(N_GENES), np.diff(g_ptr))
     # L from the CDS content itself (K4, strand-aware; half-open block ends = inclusive end + 1)
-    bc, _ = kernels.count_contexts(dg, g_chrom[owner], g_bs, g_be + 1, 1, 1, strand=g_strand[owner])
-    L = pipeline.synth_gene_L(bc.cpu().numpy(), g_ptr, seed + 300)
+    cds_counts = lambda: kernels.count_contexts(dg, g_chrom[owner], g_bs, g_be + 1, 1, 1,
+                                                strand=g_strand[owner])[0].cpu().numpy()
+    bc = cds_counts()
+    # A gene drawn inside one of the genome's N runs (10-51 kb) has no countable context, in its CDS or in its windows:
+    # R_SIZE = 0 makes its Pi_INDEL infinite, and the reference's sum over genes then zeroes the indel scale factor of
+    # every gene.  Real CDS never lie in assembly gaps, so such a gene is moved 64 kb along its chromosome (further in
+    # than the longest N run) until its CDS holds a countable context.
+    lim = np.maximum((lengths - 1) // WINDOW * WINDOW - 1, 0) - 1          # last CDS position synth_genes allows
+    for _ in range(16):
+        empty = np.flatnonzero(np.add.reduceat(bc.sum(axis=1), g_ptr[:-1]) == 0)
+        if len(empty) == 0:
+            break
+        for g in empty:
+            a, b = g_ptr[g], g_ptr[g + 1]
+            shift = 1 << 16 if g_be[a:b].max() + (1 << 16) <= lim[g_chrom[g]] else -(1 << 16)
+            g_bs[a:b] += shift
+            g_be[a:b] += shift
+        assert g_bs.min() >= 5, "a gene was moved off the start of its chromosome"
+        bc = cds_counts()
+    else:
+        raise RuntimeError("synthetic genes without countable context remain after 16 moves")
+    L = pipeline.synth_gene_L(bc, g_ptr, seed + 300)
     # mutations: 30 % coding SNVs, 63 % non-coding SNVs, 7 % indels; Zipf-weighted samples
     rng = np.random.default_rng(seed + 400)
     n_cds = int(0.30 * N_MUT)
@@ -643,6 +672,36 @@ def parity_sample(dg, d, di, res, seed, n_windows=500, n_genes=200):
     return out
 
 
+DUMP_WINDOWS = 8192          # count-table rows written by --dump-outputs (the whole pentanucleotide table is 1.27 GB)
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, di, res):
+    """What the last timed step computed, as out_dir/<name>.npy, for comparing two builds output for output: the rows
+    of both count tables for a fixed, seeded sample of DUMP_WINDOWS windows (their indices in sample_windows), the
+    genome totals, and every array of the test stage's result (per-gene columns, scale-factor sums, sequence model,
+    mutation contexts).  Integer arrays whose values float32 holds exactly (the counts, the contexts) are written as
+    float32, all others as float64."""
+    import torch
+    n_win = di.win_chrom.numel()
+    rows = np.sort(np.random.default_rng(0).choice(n_win, size=min(DUMP_WINDOWS, n_win), replace=False))
+    idx = torch.from_numpy(rows).to(di.counts5.device)
+    arrays = {"sample_windows": rows, "counts5_sample": di.counts5[idx], "counts3_sample": di.counts3[idx],
+              "totals5": di.totals5, "totals3": di.totals3}
+    arrays.update(res)
+    out = {}
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        exact32 = a.dtype.kind in "iub" and (a.size == 0 or int(np.abs(a).max()) < 1 << 24)
+        out[name] = a.astype(np.float32 if exact32 else np.float64)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # FP64 side of the test stage at the sizes where it binds (BASELINE configs 5 and 3), outside the step's timing
 # ------------------------------------------------------------------------------------------------
@@ -928,11 +987,10 @@ def run_reference(args):
     import multiprocessing as mp
     n_proc = max(1, min((os.cpu_count() or 2) - 2, 64))
     n_steps = args.warmup + args.steps
-    # about 3 s of pool work per step (1000 windows = 10 Mb per worker and context size), the whole run bounded
-    # to ~2.5 minutes
+    # about 3 s of pool work per step (1000 windows = 10 Mb per worker and context size)
     wpp = 1000
     pool = mp.Pool(n_proc) if n_proc > 1 else None
-    vals, t0, sample = [], time.perf_counter(), ""
+    vals, sample = [], ""
     stages = None
     for i in range(n_steps):
         v, st, secs = reference_value(args.bases, n_proc, 1000 + i, pool, wpp)
@@ -948,8 +1006,6 @@ def run_reference(args):
                      st["observed"][1], st["observed"][0], st["transfer"][1], st["transfer"][0], N_GENES, st["test"][0],
                      args.bases, N_MUT - int(0.07 * N_MUT), N_GENES))
         stages = {k: round(v_, 3) for k, v_ in secs.items()}
-        if time.perf_counter() - t0 > 150.0 and vals:
-            break
     if pool is not None:
         pool.close()
     v = float(np.median(vals))
@@ -997,6 +1053,8 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     assert torch.cuda.is_available(), "bench.py needs a GPU (no CPU fallback)"
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of a single-process run; it is not supported under torchrun")
     torch.cuda.set_device(local_rank)
     device = torch.device("cuda", local_rank)
     placement = bind_to_gpu_numa_node(local_rank) if world > 1 else "single process, not bound"
@@ -1063,6 +1121,8 @@ def main():
         elapsed_ms, k5_ms = float(t[0]), float(t[1])
     ms_per_step = elapsed_ms / args.steps
     value = n_total / (ms_per_step * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, di, res)
 
     # ---- the all-gathered result rows (range-sharded runs): every rank's block, as it arrived on EVERY rank, against the
     #      rows that rank computed (bitwise, NaN = NaN); outside the timed region
@@ -1121,8 +1181,7 @@ def main():
         # (1) the steady state: the packed-genome cache as the source (every run after the first one)
         hg_packed = host_pipeline.HostGenome.from_device(dg)
         hp = HostPath(hg_packed, d, di, device, shard=shard)
-        n_e2e = max(3, min(args.steps, 5))
-        e2e_s = timed(hp, n_e2e)
+        e2e_s = timed(hp, args.steps)
         h2d, d2h = totals_over_ranks(hp.h2d_bytes, hp.d2h_bytes)
         e2e = {"value": n_total / e2e_s, "unit": "bases/s", "ms_per_step": e2e_s * 1e3,
                "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h, "gpu_launches_per_step": hp.launches,
@@ -1139,7 +1198,7 @@ def main():
         hg_ascii = host_pipeline.HostGenome.from_device(dg, ascii_d)
         del ascii_d
         hp = HostPath(hg_ascii, d, di, device, shard=shard)
-        cold_s = timed(hp, 3)
+        cold_s = timed(hp, args.steps)
         h2d, d2h = totals_over_ranks(hp.h2d_bytes, hp.d2h_bytes)
         e2e["cold"] = {"value": n_total / cold_s, "ms_per_step": cold_s * 1e3, "h2d_bytes_per_step": h2d,
                        "d2h_bytes_per_step": d2h, "source": "pinned host ASCII genome (1 B/base), K1 pack on the device"}

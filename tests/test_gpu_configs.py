@@ -357,6 +357,11 @@ def test_config2_parity_sample_at_full_size(oracle):
     torch.cuda.synchronize()
     out = bench.parity_sample(dg, d, di, res, seed=1, n_windows=500, n_genes=200)
     assert out["ok"], out
+    # every synthetic gene holds countable context, so every result is finite: one gene with R_SIZE = 0 (Pi_INDEL = inf)
+    # would zero the indel scale factor, and with it EXP_INDEL, of all genes
+    for k, v in res.items():
+        assert not v.is_floating_point() or bool(torch.isfinite(v).all()), k
+    assert float(res["EXP_INDEL"].min()) > 0
     assert out["windows"] == 500 and out["genes"] == 200
     assert out["windows_beyond_2^31"] > 50, out           # ~30 % of hg19 lies beyond 2^31
     assert out["mutations"] > 500 and out["p_values"] > 500, out

@@ -1,7 +1,6 @@
-"""CPU tier: the built-in HDF5 reader (digdriver_b200/hdf5_lite.py) on the one real HDF5 file of this image (SciPy's
-MATLAB v7.3 test file, written by libhdf5 through MATLAB) and on round trips through its own classic-format writer,
-including the pandas fixed-format layout and the reference's per-element groups (SURVEY.md section 8 f-1)."""
-import glob
+"""CPU tier: the built-in HDF5 reader (digdriver_b200/hdf5_lite.py) on a real HDF5 file (SciPy's MATLAB v7.3 test file,
+written by libhdf5 through MATLAB) and on round trips through its own classic-format writer, including the pandas
+fixed-format layout and the reference's per-element groups (SURVEY.md section 8 f-1)."""
 import os
 import struct
 import zlib
@@ -10,18 +9,15 @@ import numpy as np
 import pandas as pd
 import pytest
 
+from conftest import GOLDEN
 from digdriver_b200 import hdf5_lite, storage
 
-
-def _scipy_mat():
-    import scipy.io
-    hits = glob.glob(os.path.join(os.path.dirname(scipy.io.__file__), "matlab", "tests", "data", "testhdf5_7.4_GLNX86.mat"))
-    return hits[0] if hits else None
+# a copy of scipy/io/matlab/tests/data/testhdf5_7.4_GLNX86.mat from SciPy 1.18.1 (BSD-3-Clause), 4 KB
+SCIPY_MAT = os.path.join(GOLDEN, "testhdf5_7.4_GLNX86.mat")
 
 
-@pytest.mark.skipif(_scipy_mat() is None, reason="SciPy's MATLAB v7.3 test file is not installed")
 def test_reads_a_real_libhdf5_file():
-    with hdf5_lite.File(_scipy_mat()) as f:
+    with hdf5_lite.File(SCIPY_MAT) as f:
         assert f.base == 512 and f.keys("/") == ["testdouble"] and not f.is_group("testdouble")
         assert f.attrs("testdouble") == {"MATLAB_class": "double"}
         x = f["testdouble"]

@@ -275,3 +275,30 @@ def test_mask_runs_round_trip():
     assert np.array_equal(out, words)
     assert not any(f < 1000 < f + c for f, c, _ in runs)   # no run spans the chromosome boundary (word 1000)
     assert mask_runs_of(np.zeros(10, dtype=np.int32), np.array([0]), 320).shape == (0, 3)
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: a seeded, sorted sample of count-table rows with their window indices, whole small arrays,
+    integer arrays as exact float32 and larger integers and floats as float64."""
+    import torch
+    import bench
+    from types import SimpleNamespace
+    n_win = 10_000
+    c5 = torch.randint(0, 10_001, (n_win, 1024), dtype=torch.int32, generator=torch.Generator().manual_seed(0))
+    di = SimpleNamespace(win_chrom=torch.zeros(n_win, dtype=torch.int32), counts5=c5, counts3=c5[:, :64].contiguous(),
+                         totals5=c5.sum(0) * 1000, totals3=c5[:, :64].sum(0))
+    res = {"PVAL_MUT_BURDEN": torch.linspace(0, 1, 7, dtype=torch.float64), "CTX": torch.tensor([-1, 0, 63], dtype=torch.int32)}
+    bench.dump_outputs(str(tmp_path / "a"), di, res)
+    bench.dump_outputs(str(tmp_path / "b"), di, res)
+    got = {f[:-4]: np.load(str(tmp_path / "a" / f)) for f in os.listdir(tmp_path / "a")}
+    assert sorted(got) == sorted(["sample_windows", "counts5_sample", "counts3_sample", "totals5", "totals3",
+                                  "PVAL_MUT_BURDEN", "CTX"])
+    assert sorted(os.listdir(tmp_path / "b")) == sorted(k + ".npy" for k in got)
+    for k, v in got.items():
+        assert np.array_equal(v, np.load(str(tmp_path / "b" / (k + ".npy"))))
+    rows = got["sample_windows"].astype(np.int64)
+    assert len(rows) == bench.DUMP_WINDOWS and np.all(np.diff(rows) > 0)
+    assert got["counts5_sample"].dtype == np.float32 and np.array_equal(got["counts5_sample"], c5[rows].numpy())
+    assert got["totals5"].dtype == np.float64 and np.array_equal(got["totals5"], di.totals5.numpy())
+    assert got["CTX"].dtype == np.float32 and got["CTX"].tolist() == [-1, 0, 63]
+    assert got["PVAL_MUT_BURDEN"].dtype == np.float64 and np.array_equal(got["PVAL_MUT_BURDEN"], res["PVAL_MUT_BURDEN"].numpy())
