@@ -31,6 +31,7 @@ SIGNATURES = {
     "dig_narrow_counts_u16": (_I, [_P, _I64, _P, _P, _P]),
     "dig_peer_broadcast": (_I, [_P, _I64, _P, _I, _P]),
     "dig_nmask_fill_runs": (_I, [_P, _I64, _P, _I64, _I64, _P]),
+    "dig_nmask_summary": (_I, [_P, _I64, _I64, _P, _P]),
     "dig_tabulate_capacity": (_I64, [_I64]),
     "dig_tabulate_elements_workspace_bytes": (_I64, [_I64]),
     "dig_tabulate_genes_workspace_bytes": (_I64, [_I64]),
@@ -75,7 +76,7 @@ class ScanOpts(ctypes.Structure):
     """dig_scan_opts of include/dig_b200.h."""
     _fields_ = [("workspace_d", _c.c_void_p), ("workspace_bytes", _c.c_int64), ("variant", _c.c_int32),
                 ("totals_limit_kb", _c.c_uint32), ("tile_window", _c.c_int64), ("n_peer_counts3", _c.c_int32),
-                ("reserved0", _c.c_int32), ("peer_counts3_d", _c.c_void_p * 8), ("mc_counts3_d", _c.c_void_p)]
+                ("nsum_offset_words", _c.c_int32), ("peer_counts3_d", _c.c_void_p * 8), ("mc_counts3_d", _c.c_void_p)]
 
 
 SCAN_AUTO, SCAN_PER_BASE, SCAN_HEX_PLAIN, SCAN_HEX = 0, 1, 2, 3
@@ -92,6 +93,7 @@ KERNELS_PER_CALL = {
     "dig_window_denominators": 1, "dig_site_test": 1, "dig_gene_dnds_sel": 1, "dig_selection_coefficient": 1, "dig_region_prob_norm": 1, "dig_position_obs": 1, "dig_position_test": 1, "dig_nb_pvalue_exact": 1,
     "dig_nb_pvalue_variant": 1, "dig_loglik": 1, "dig_gene_llr_test": 1, "dig_overlap_count": 1, "dig_overlap_fill": 1,
     "dig_element_region_counts": 1, "dig_element_psum": 1, "dig_narrow_counts_u16": 1, "dig_peer_broadcast": 1, "dig_nmask_fill_runs": 1,
+    "dig_nmask_summary": 1,
 }
 launch_count = 0
 

@@ -49,6 +49,46 @@ __global__ void __launch_bounds__(256) nmask_fill_runs_kernel(const int64_t *__r
     }
 }
 
+// one thread per 128-base block (one 16-byte load of four mask words); a warp covers 32 blocks = two summary words, so
+// each summary word is merged into by exactly one half-warp
+__global__ void __launch_bounds__(256) nmask_summary_kernel(const uint32_t *__restrict__ nmask, int64_t word0, int64_t n_words,
+                                                            uint32_t *__restrict__ nsum)
+{
+    const int lane = threadIdx.x & 31;
+    const int64_t b_lo = word0 >> 2, b_hi = (word0 + n_words + 3) >> 2;    // blocks to rebuild
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < ((b_hi - (b_lo & ~(int64_t)31) + 31) & ~(int64_t)31);
+         t += stride) {
+        const int64_t blk = (b_lo & ~(int64_t)31) + t;
+        const bool in = blk >= b_lo && blk < b_hi;
+        uint32_t v = 0u;
+        if (in) {
+            const int64_t w = blk * 4, wend = word0 + n_words;
+            uint32_t m[4];
+            if (w + 4 <= wend) {
+                const uint4 q = *reinterpret_cast<const uint4 *>(nmask + w);
+                m[0] = q.x; m[1] = q.y; m[2] = q.z; m[3] = q.w;
+            } else {
+#pragma unroll
+                for (int i = 0; i < 4; ++i) m[i] = w + i < wend ? nmask[w + i] : ~0u;
+            }
+            const uint32_t any = m[0] | m[1] | m[2] | m[3], all = m[0] & m[1] & m[2] & m[3];
+            v = (any != 0u ? 1u : 0u) | (all == ~0u ? 2u : 0u);
+        }
+        const int sh = 2 * (lane & 15);
+        uint32_t bits = v << sh, keep = in ? 0u : 3u << sh;
+#pragma unroll
+        for (int o = 8; o > 0; o >>= 1) {
+            bits |= __shfl_xor_sync(0xffffffffu, bits, o);
+            keep |= __shfl_xor_sync(0xffffffffu, keep, o);
+        }
+        if ((lane & 15) == 0 && keep != 0xFFFFFFFFu) {
+            uint32_t *dst = nsum + (blk >> 4);
+            *dst = keep == 0u ? bits : (*dst & keep) | bits;
+        }
+    }
+}
+
 struct PeerDst {
     uint4 *p[8];
 };
@@ -78,6 +118,21 @@ int dig_nmask_fill_runs(const int64_t *runs_d, int64_t n_runs, uint32_t *nmask_d
     int64_t blocks = (n_runs + 7) / 8;
     if (blocks > 1184) blocks = 1184;
     nmask_fill_runs_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(runs_d, n_runs, nmask_d, word0, n_words);
+    DIG_CHECK_LAUNCH();
+    return DIG_OK;
+}
+
+int dig_nmask_summary(const uint32_t *nmask_d, int64_t word0, int64_t n_words, uint32_t *nsum_d, void *stream)
+{
+    DIG_CHECK_ARG(word0 >= 0 && n_words >= 0 && (word0 & 3) == 0, "word0 must be a non-negative multiple of 4, n_words >= 0");
+    if (n_words == 0) return DIG_OK;
+    DIG_CHECK_ARG(nmask_d != nullptr && nsum_d != nullptr, "null pointer");
+    DIG_CHECK_ARG((reinterpret_cast<uintptr_t>(nmask_d) & 15u) == 0, "nmask_d must be 16-byte aligned");
+    const int64_t threads = (((word0 + n_words + 3) >> 2) - ((word0 >> 2) & ~(int64_t)31) + 31) & ~(int64_t)31;
+    int64_t blocks = (threads + 255) / 256;
+    const int64_t cap = (int64_t)dig::sm_count() * 8;
+    if (blocks > cap) blocks = cap;
+    nmask_summary_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(nmask_d, word0, n_words, nsum_d);
     DIG_CHECK_LAUNCH();
     return DIG_OK;
 }

@@ -38,6 +38,7 @@ struct ScanOpts {
     int n_peer = 0;
     void *const *peer3 = nullptr;
     void *mc3 = nullptr;
+    int64_t nsum_off = 0;                   // words from nmask_d to its N summary (0: none)
 };
 
 ScanOpts scan_opts(const dig_scan_opts *o)
@@ -49,6 +50,7 @@ ScanOpts scan_opts(const dig_scan_opts *o)
         r.variant = o->variant;
         if (o->totals_limit_kb != 0u) r.tot_limit_kb = o->totals_limit_kb;
         r.tile_window = o->tile_window;
+        r.nsum_off = o->nsum_offset_words > 0 ? o->nsum_offset_words : 0;
         if (o->n_peer_counts3 > 0) {
             r.n_peer = o->n_peer_counts3 < 8 ? o->n_peer_counts3 : 8;
             r.peer3 = o->peer_counts3_d;
@@ -564,7 +566,7 @@ extern "C" int dig_count_contexts_fused53(const uint32_t *packed2_d, const uint3
     DIG_CHECK_ARG(so.variant >= DIG_SCAN_AUTO && so.variant <= DIG_SCAN_HEX, "unknown scan variant");
     if (so.variant == DIG_SCAN_AUTO &&
         scan_lb_usable(packed2_d, nmask_d, n_bases, counts5_d, so.workspace, so.workspace_bytes, n_reg))
-        return launch_scan_lb(packed2_d, nmask_d, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
+        return launch_scan_lb(packed2_d, nmask_d, so.nsum_off > 0 ? nmask_d + so.nsum_off : nullptr, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
                               n_reg, counts5_d, counts3_d, totals5_d, totals3_d, so.tot_limit_kb, so.workspace,
                               so.tile_window, (cudaStream_t)stream, so.n_peer, so.peer3, so.mc3);
     DIG_CHECK_ARG(so.n_peer == 0, "peer_counts3_d needs the lane-bank kernel (workspace, 128-base aligned genome, variant AUTO)");
@@ -610,14 +612,14 @@ extern "C" int dig_count_contexts(const uint32_t *packed2_d, const uint32_t *nma
     cudaStream_t st = (cudaStream_t)stream;
     if (n_up == 2 && n_down == 2 && reg_strand_d == nullptr && so.variant == DIG_SCAN_AUTO &&
         scan_lb_usable(packed2_d, nmask_d, n_bases, counts_d, so.workspace, so.workspace_bytes, n_reg))
-        return launch_scan_lb(packed2_d, nmask_d, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
+        return launch_scan_lb(packed2_d, nmask_d, so.nsum_off > 0 ? nmask_d + so.nsum_off : nullptr, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
                               n_reg, counts_d, nullptr, totals_d, nullptr, so.tot_limit_kb, so.workspace, so.tile_window, st);
     // (the lane-bank kernel works in batches of 32 regions, one CTA per batch: with fewer than two batches per SM -- e.g.
     // 3 100 windows of 1 Mb -- the per-warp kernel spreads the work better)
     if (n_up == 1 && n_down == 1 && reg_strand_d == nullptr && so.variant == DIG_SCAN_AUTO &&
         n_reg >= (int64_t)64 * dig::sm_count() &&
         scan_lb_usable(packed2_d, nmask_d, n_bases, counts_d, so.workspace, so.workspace_bytes, n_reg))
-        return launch_scan_lb(packed2_d, nmask_d, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
+        return launch_scan_lb(packed2_d, nmask_d, so.nsum_off > 0 ? nmask_d + so.nsum_off : nullptr, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
                               n_reg, nullptr, counts_d, nullptr, totals_d, so.tot_limit_kb, so.workspace, so.tile_window, st,
                               so.n_peer, so.peer3, so.mc3);
     DIG_CHECK_ARG(so.n_peer == 0, "peer_counts3_d needs the trinucleotide lane-bank kernel (n_up = n_down = 1, plus strand, "

@@ -158,11 +158,12 @@ int launch_scan_tri_list(const uint32_t *p2, const uint32_t *nm, int64_t n_bases
                          unsigned int tot_limit_kb, const int32_t *rlist, const int32_t *rlist_n, cudaStream_t stream);
 
 // scan_lb.cu: the same tables through the lane-bank kernel (one window per lane, conflict-free atomics), followed by
-// launch_scan_hex over the regions it could not take.  `workspace` holds that list (scan_lb_workspace_bytes).
+// launch_scan_hex over the regions it could not take.  `workspace` holds that list (scan_lb_workspace_bytes).  `nsum`
+// (nullable): the per-128-base N summary of nm (dig_nmask_summary); with it the kernel stages the bases alone.
 size_t scan_lb_workspace_bytes(int64_t n_reg);
 bool scan_lb_usable(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int32_t *counts5, const void *workspace,
                     size_t workspace_bytes, int64_t n_reg);
-int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int64_t *chrom_off,
+int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, const uint32_t *nsum, int64_t n_bases, const int64_t *chrom_off,
                    const int64_t *chrom_len, const int32_t *reg_chrom, const int64_t *reg_start, const int64_t *reg_end,
                    int64_t n_reg, int32_t *counts5, int32_t *counts3, unsigned long long *totals5,
                    unsigned long long *totals3, unsigned int tot_limit_kb, void *workspace, int64_t tile_window,

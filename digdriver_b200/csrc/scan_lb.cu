@@ -18,7 +18,8 @@
 //     LB_MAX_CHUNKS chunks.
 //   * genome staging: the 16 consumer warps split each 2048-base chunk of every window into 128-base spans; the
 //     chunk (+ one 16-byte granule of halo) of each of the 32 windows is brought into shared memory by TMA bulk
-//     copies (cp.async.bulk, mbarrier completion), two stages deep; consumer warp w issues the copies of windows
+//     copies (cp.async.bulk, mbarrier completion), two stages deep (plus slots aliased onto the slice buffers; with
+//     the per-128-base N summary only the bases are staged, see lb_span_states); consumer warp w issues the copies of windows
 //     2w and 2w+1 (ptxas serialises per-lane bulk copies, so they are spread over the warps).  Window strides of
 //     33 / 17 granules keep the 128-bit shared-memory reads of a quarter-warp on distinct banks.
 //   * write-out: pentanucleotide m gets dp4a(row m) (hexamers that START with m) plus byte f of the rows
@@ -93,6 +94,14 @@ constexpr uint32_t LB_SMEM = OFF_BAR + 256u;                       // 17 barrier
 static_assert(OFF_BAR % 16u == 0u, "barrier block alignment");
 static_assert(LB_SMEM <= 232448u, "shared memory budget");
 
+// With the per-128-base N summary (LbArgs::nsum) a stage holds the bases alone: 8 x LB_DGROUP = 17 KB instead of 26 KB, so
+// THREE stages fit where two stood, and a fourth ring slot is aliased onto the slice buffers as before.  The span states
+// of every window and slot (one word per window, see lb_span_states) sit in the 1 KB left between the third stage and
+// the slice buffers.  Every other offset is the same in both layouts.
+constexpr uint32_t LB_BSTAGE = 8u * LB_DGROUP;                    // 17408 B: a stage of bases only
+constexpr uint32_t OFF_SUM = OFF_STG + 3u * LB_BSTAGE;             // [4 slots][32 windows] span-state words
+static_assert(OFF_SUM + 4u * 128u <= OFF_OUT && LB_BSTAGE <= LB_NOUT * OUT_BYTES, "bases-only ring layout");
+
 enum { BAR_FULL = 0, BAR_EMPTY = 2, BAR_OUTFULL = 4, BAR_OUTEMPTY = 8, BAR_DONE = 12, BAR_CLEAN = 13 };
 
 // Third staging slot of the pentanucleotide modes.  Two stages are all that fits beside the 128 KB table and the four
@@ -106,9 +115,29 @@ enum { BAR_FULL = 0, BAR_EMPTY = 2, BAR_OUTFULL = 4, BAR_OUTEMPTY = 8, BAR_DONE 
 #define DIG_LB_STAGE3 1
 #endif
 constexpr bool LB_ST3 = DIG_LB_STAGE3 != 0;
-enum { BAR_FULL2 = 14, BAR_EMPTY2 = 15, BAR_OUTFREE = 16 };           // OUTFREE: the four writer warps have shipped their last tile of the batch
-__device__ __forceinline__ uint32_t lb3_full(uint32_t stage) { return stage < 2u ? (uint32_t)BAR_FULL + stage : (uint32_t)BAR_FULL2; }
-__device__ __forceinline__ uint32_t lb3_empty(uint32_t stage) { return stage < 2u ? (uint32_t)BAR_EMPTY + stage : (uint32_t)BAR_EMPTY2; }
+// With the N summary (bases-only stages) the ring has FOUR slots, chunk kq going to slot kq % 4: slots 0-2 are real
+// stages and slot 3 is the slice buffers, under the same BAR_OUTFREE rule.
+enum { BAR_FULL2 = 14, BAR_EMPTY2 = 15, BAR_OUTFREE = 16, BAR_FULL3 = 17, BAR_EMPTY3 = 18 };   // OUTFREE: the four writer warps have shipped their last tile of the batch
+__device__ __forceinline__ uint32_t lb3_full(uint32_t stage)
+{
+    return stage < 2u ? (uint32_t)BAR_FULL + stage : (stage == 2u ? (uint32_t)BAR_FULL2 : (uint32_t)BAR_FULL3);
+}
+__device__ __forceinline__ uint32_t lb3_empty(uint32_t stage)
+{
+    return stage < 2u ? (uint32_t)BAR_EMPTY + stage : (stage == 2u ? (uint32_t)BAR_EMPTY2 : (uint32_t)BAR_EMPTY3);
+}
+// slots of the pentanucleotide ring, the last one being the slice buffers; stg0 = sbase + OFF_STG
+template <bool NS>
+struct LbSlots {
+    static constexpr uint32_t N = NS ? 4u : 3u;
+};
+template <bool NS>
+__device__ __forceinline__ uint32_t lb_slot(uint32_t stg0, uint32_t stage)
+{
+    if constexpr (NS) return stage < 3u ? stg0 + stage * LB_BSTAGE : stg0 + (OFF_OUT - OFF_STG);
+    else return stg0 + stage * LB_STAGE_BYTES;                    // slot 2 = OFF_OUT
+}
+__device__ __forceinline__ uint32_t lb_slot_sum(uint32_t stg0, uint32_t stage) { return stg0 + (OFF_SUM - OFF_STG) + stage * 128u; }
 
 // Staging ring per mode.  The pentanucleotide modes have room for two stages next to their 128 KB table and the slice
 // buffers; the trinucleotide-only mode (32 KB table, no slice buffers) runs FOUR, which hides the ~3 k cycles between a
@@ -421,6 +450,41 @@ __device__ __forceinline__ void lb_pairs(const uint32_t (&D)[9], uint32_t tabl, 
     }
 }
 
+// ---- the per-128-base N summary (dig_nmask_summary): two bits per aligned block of 128 bases, block j at bits 2 (j & 15)
+// and 2 (j & 15) + 1 of word j >> 4: bit 0 = the block holds an N, bit 1 = every base of it is N (00 clean, 01 mixed,
+// 11 all-N).  A consumer span covers block b and the first four bases of block b + 1 (its last centres reach base 131),
+// so its state is taken from both blocks:
+//   * clean (00): neither block holds an N;
+//   * all-N (11): both blocks are all N -- no centre of the span has a valid 3- or 5-mer (a span whose own block is all N
+//     but whose halo block is not can still hold the trinucleotide centre 129), no atomics;
+//   * mixed (01): anything else; the span's five mask words are read from global memory.
+// Blocks outside [0, n_bases / 128) -- the lead-in span of a region at the genome start has origin -128 -- count as all N.
+// Returns the states of the sixteen spans of the chunk starting at base G0 (a multiple of 128): span s at bits 2s, 2s + 1.
+__device__ __forceinline__ uint32_t lb_span_states(const uint32_t *__restrict__ nsum, int64_t n_bases, int64_t G0)
+{
+    const int64_t B0 = G0 >> 7, nw = ((n_bases >> 7) + 15) >> 4, w0 = B0 >> 4;       // arithmetic shifts: floor
+    const uint32_t lo = (w0 >= 0 && w0 < nw) ? __ldg(nsum + w0) : ~0u;
+    const uint32_t hi = (w0 + 1 >= 0 && w0 + 1 < nw) ? __ldg(nsum + w0 + 1) : ~0u;
+    const unsigned long long v = (((unsigned long long)hi << 32) | lo) >> (2 * (B0 & 15));   // blocks B0 .. B0 + 16
+    const unsigned long long hn = v & 0x5555555555555555ull, an = (v >> 1) & 0x5555555555555555ull;
+    const uint32_t nc = (uint32_t)(hn | (hn >> 2)) & 0x55555555u;                   // an N in block s or s + 1
+    const uint32_t aa = (uint32_t)(an & (an >> 2)) & 0x55555555u;                   // blocks s and s + 1 all N
+    return nc | (aa << 1);
+}
+// the five mask words of the span starting at base G (a multiple of 128, >= -128) straight from global memory; words
+// outside the genome read as all N
+__device__ __forceinline__ void lb_mask_global(const uint32_t *__restrict__ nmask, int64_t n_bases, int64_t G, uint32_t (&M)[5])
+{
+    const int64_t w = G >> 5, nw = n_bases >> 5;
+    if (w >= 0 && w + 4 <= nw) {
+        const uint4 m = __ldg(reinterpret_cast<const uint4 *>(nmask + w));
+        M[0] = m.x; M[1] = m.y; M[2] = m.z; M[3] = m.w;
+    } else {
+        M[0] = M[1] = M[2] = M[3] = ~0u;
+    }
+    M[4] = (w + 4 >= 0 && w + 4 < nw) ? __ldg(nmask + w + 4) : ~0u;
+}
+
 #ifdef DIG_LB_TIMING
 #define LB_T(var) const long long var = clock64()
 #define LB_ACC(slot, t0, t1) tacc[slot] += (unsigned long long)((t1) - (t0))
@@ -432,6 +496,7 @@ __device__ __forceinline__ void lb_pairs(const uint32_t (&D)[9], uint32_t tabl, 
 struct LbArgs {
     const uint32_t *p2;
     const uint32_t *nmask;
+    const uint32_t *nsum;     // per-128-base N summary (kernels instantiated with NS = true only)
     int64_t n_bases;
     const int64_t *chrom_off;
     const int64_t *chrom_len;
@@ -492,7 +557,8 @@ __device__ __forceinline__ int lb_chunk_order(int kq, int nch) { return kq == 0 
 // The chunk sequence of a CTA is the concatenation of the chunks of its batches (each batch in lb_chunk_order).  In the
 // trinucleotide-only rings chunk number ci lands in stage ci & (NST - 1) once the chunk that used the stage before has
 // been read into registers by all consumer warps of the team; in the pentanucleotide modes chunk kq of a batch lands in
-// slot kq % 3 (slot 2 = the slice buffers, see BAR_FULL2 / BAR_OUTFREE above), with one fill-parity bit per slot.
+// slot kq % 3 (kq % 4 with the N summary; the last slot = the slice buffers, see BAR_FULL2 / BAR_OUTFREE above), with one
+// fill-parity bit per slot.
 //   * Regular group (the four windows lie at a pitch of 8 tile windows in one chromosome, nothing clipped): the group
 //     leader issues TWO 2-D TMA box loads per chunk (4 rows x 528 B of bases, 4 rows x 272 B of mask) through tensor
 //     maps that view each genome array as rows of one pitch (lb_input_maps).
@@ -503,7 +569,7 @@ struct LbMaps {
     CUtensorMap d[2], m[2];   // bases / mask, each with two row phases (a box must not cross the end of a row)
 };
 
-template <int GM>
+template <int GM, bool NS>
 __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps, const LbTeam T, int pw, int lane)
 {
     const uint32_t bar = T.bar;
@@ -511,7 +577,8 @@ __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps,
     const int m = lane & 3;                                // row of the group's box
     const bool mine = (lane >> T.lane_shift) == pw;
     uint32_t ci = 0u;
-    constexpr bool ST3 = LB_ST3 && GM < 2;                 // three slots, the third one aliasing the slice buffers
+    constexpr bool ST3 = LB_ST3 && GM < 2;                 // three (NS: four) slots, the last one aliasing the slice buffers
+    constexpr uint32_t NSL = LbSlots<NS>::N;
     uint32_t uses = 0u, pbi = 0u;                          // bit s of uses: parity of the number of fills of slot s
     for (int64_t b = T.b0; b < n_batches; b += T.bstep, ++pbi) {
         const LbGeom g = lb_geom<GM>(b * 32 + lb_win(lane), A.n_reg, A.chrom_off, A.chrom_len, A.reg_chrom, A.reg_start, A.reg_end);
@@ -548,7 +615,7 @@ __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps,
             uint32_t stage, fpar, full_i, empty_i;
             if constexpr (ST3) {
                 stage = st3;
-                st3 = st3 == 2u ? 0u : st3 + 1u;
+                st3 = st3 == NSL - 1u ? 0u : st3 + 1u;
                 fpar = (uses >> stage) & 1u;
                 uses ^= 1u << stage;
                 full_i = lb3_full(stage);
@@ -559,15 +626,25 @@ __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps,
                 full_i = R::FULL0 + stage;
                 empty_i = R::EMPTY0 + stage;
             }
+            // span states of this window's chunk: read (read-only data) before the wait for the slot hides the load
+            uint32_t sw = 0u;
+            if constexpr (NS) {
+                if (mine && k < g.nch) sw = lb_span_states(A.nsum, A.n_bases, g.O + (int64_t)k * LB_CHUNK);
+            }
             LB_T(t_e0);
             mbar_wait_idle(bar + 8u * empty_i, fpar ^ 1u);
             if constexpr (ST3) {
                 // the slice buffers are free once the previous batch's last tiles have left them
-                if (stage == 2u && pbi >= 1u) mbar_wait_idle(bar + 8u * BAR_OUTFREE, (pbi - 1u) & 1u);
+                if (stage == NSL - 1u && pbi >= 1u) mbar_wait_idle(bar + 8u * BAR_OUTFREE, (pbi - 1u) & 1u);
             }
             LB_T(t_e1);
             const uint32_t full = bar + 8u * full_i;
-            const uint32_t stg = T.stg0 + stage * LB_STAGE_BYTES;
+            const uint32_t stg = ST3 ? lb_slot<NS>(T.stg0, stage) : T.stg0 + stage * LB_STAGE_BYTES;
+            if constexpr (NS) {
+                // the state word goes where the mask strips went (trinucleotide-only rings, whose stages keep their size)
+                // or into the state block of the pentanucleotide ring; this lane's FULL arrival below releases it
+                if (mine) sts32((ST3 ? lb_slot_sum(T.stg0, stage) : stg + LB_MBASE) + (uint32_t)lb_win(lane) * 4u, sw);
+            }
             if (!mine) {
                 // another producer warp's window
             } else if (regular && k < g.nch) {
@@ -582,9 +659,9 @@ __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps,
                     int bxd = (int)xd - lead, bxm = (int)xm - lead, sd = 0, sm = 0;
                     if (bxd + (int)(LB_DROW / 4) > (int)ped) { bxd -= (int)A.dshift; sd = 1; }     // the box would cross the row end:
                     if (bxm + (int)(LB_MROW / 4) > (int)pem) { bxm -= (int)A.mshift; sm = 1; }     // same row of the shifted view
-                    mbar_arrive_tx(full, 4u * (LB_DROW + LB_MROW));
+                    mbar_arrive_tx(full, 4u * (NS ? LB_DROW : LB_DROW + LB_MROW));
                     tensor_g2s(&maps->d[sd], stg + lb_dgroup(lane), bxd, (int)yd, full);
-                    tensor_g2s(&maps->m[sm], stg + lb_mgroup(lane), bxm, (int)ym, full);
+                    if constexpr (!NS) tensor_g2s(&maps->m[sm], stg + lb_mgroup(lane), bxm, (int)ym, full);
                 } else {
                     mbar_arrive(full);
                 }
@@ -600,9 +677,9 @@ __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps,
                 const int64_t davail = (A.n_bases >> 2) - dsrc, mavail = (A.n_bases >> 3) - msrc;
                 if (dbytes > davail) dbytes = davail;
                 if (mbytes > mavail) mbytes = mavail;
-                mbar_arrive_tx(full, (uint32_t)(dbytes + mbytes));
+                mbar_arrive_tx(full, (uint32_t)(NS ? dbytes : dbytes + mbytes));
                 bulk_g2s(ddst, reinterpret_cast<const unsigned char *>(A.p2) + dsrc, (uint32_t)dbytes, full);
-                bulk_g2s(mdst, reinterpret_cast<const unsigned char *>(A.nmask) + msrc, (uint32_t)mbytes, full);
+                if constexpr (!NS) bulk_g2s(mdst, reinterpret_cast<const unsigned char *>(A.nmask) + msrc, (uint32_t)mbytes, full);
             } else {
                 mbar_arrive(full);
             }
@@ -633,9 +710,10 @@ __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps,
 // ahead for the slice buffers' OUTEMPTY barriers -- a barrier look is a round trip through the shared-memory pipe behind
 // the other warps' atomics.  Measured on one box, twice each: 0.925 ms without, 0.933-0.936 ms with the FULL probe,
 // 0.941-0.944 ms with the OUTEMPTY probe: the extra shared-memory operation costs more than the hidden latency.
-template <bool TRI>
+template <bool TRI, bool NS>
 __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int warp, int lane)
 {
+    constexpr uint32_t NSL = LbSlots<NS>::N;
     const uint32_t bar = sbase + OFF_BAR;
     const uint32_t tabl = sbase + OFF_TAB + (uint32_t)lane * 4u;
     const int64_t n_batches = (A.n_reg + 31) >> 5;
@@ -667,9 +745,9 @@ __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int
         for (int kq = 0; kq < nch; ++kq, ++cit) {
             const int k = lb_chunk_order(kq, nch);
             uint32_t stage, fpar, full_i, empty_i;
-            if constexpr (LB_ST3) {                        // slot kq % 3 (see BAR_FULL2); the producers count the same way
+            if constexpr (LB_ST3) {                        // slot kq % 3 (NS: kq % 4, see BAR_FULL2); the producers count the same way
                 stage = st3;
-                st3 = st3 == 2u ? 0u : st3 + 1u;
+                st3 = st3 == NSL - 1u ? 0u : st3 + 1u;
                 fpar = (uses >> stage) & 1u;
                 uses ^= 1u << stage;
                 full_i = lb3_full(stage);
@@ -685,7 +763,7 @@ __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int
             LB_T(t_b);
             LB_ACC(0, t_a, t_b);
             LB_ACC((kq == 0 ? 8 : (kq == 1 ? 9 : 10)), t_a, t_b);
-            const uint32_t stg = sbase + OFF_STG + stage * LB_STAGE_BYTES;
+            const uint32_t stg = LB_ST3 ? lb_slot<NS>(sbase + OFF_STG, stage) : sbase + OFF_STG + stage * LB_STAGE_BYTES;
             {
                 // a span that holds no centre of any lane's window (the lead-in span, the tail of the last chunk)
                 const int base0 = k * LB_CHUNK + warp * LB_SPAN;
@@ -696,20 +774,29 @@ __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int
                 }
             }
             const uint32_t dptr = stg + lb_dstrip(lane) + (uint32_t)warp * 32u;
-            const uint32_t mptr = stg + lb_mstrip(lane) + (uint32_t)warp * 16u;
-            uint32_t D[9], M[5];
+            uint32_t D[9], M[5] = {0u, 0u, 0u, 0u, 0u}, sst = 0u;
+            uint32_t dep;
             {
-                const uint4 a = lds128(dptr), c = lds128(dptr + 16u), m = lds128(mptr);
+                const uint4 a = lds128(dptr), c = lds128(dptr + 16u);
                 D[0] = a.x; D[1] = a.y; D[2] = a.z; D[3] = a.w;
                 D[4] = c.x; D[5] = c.y; D[6] = c.z; D[7] = c.w;
                 D[8] = lds32(dptr + 32u);
-                M[0] = m.x; M[1] = m.y; M[2] = m.z; M[3] = m.w;
-                M[4] = lds32(mptr + 16u);
+                if constexpr (NS) {
+                    // this span's state (lb_span_states): one word per window, written by its producer lane
+                    const uint32_t sa = LB_ST3 ? lb_slot_sum(sbase + OFF_STG, stage) : stg + LB_MBASE;
+                    sst = (lds32(sa + (uint32_t)lb_win(lane) * 4u) >> (2 * warp)) & 3u;
+                    dep = (D[0] | D[4]) ^ (D[8] | sst);
+                } else {
+                    const uint32_t mptr = stg + lb_mstrip(lane) + (uint32_t)warp * 16u;
+                    const uint4 m = lds128(mptr);
+                    M[0] = m.x; M[1] = m.y; M[2] = m.z; M[3] = m.w;
+                    M[4] = lds32(mptr + 16u);
+                    dep = (D[0] | D[4]) ^ (D[8] | M[0]) ^ M[4];
+                }
             }
             // the stage may be refilled as soon as all sixteen warps have arrived: only after the loads have RETURNED
-            // (one register of each of the five load instructions is enough: a warp's load instruction releases its
-            // scoreboard when the data of ALL lanes has been written, so lane 0's dependence covers the warp)
-            const uint32_t dep = (D[0] | D[4]) ^ (D[8] | M[0]) ^ M[4];
+            // (one register of each load instruction is enough: a warp's load instruction releases its scoreboard when
+            // the data of ALL lanes has been written, so lane 0's dependence covers the warp)
             __syncwarp();
             if (lane == 0) mbar_arrive_after_loads(bar + 8u * empty_i, dep, A.zero);
             if (!clean) {                                                    // the writer warps have re-zeroed the tables
@@ -722,7 +809,7 @@ __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int
             LB_T(t_p0);
             const int base = k * LB_CHUNK + warp * LB_SPAN;                  // local base 0 relative to the origin
             const int lo5 = g.lo5 - base, hi5 = g.hi5 - base;                // centre c (local base index) valid: lo5 <= c < hi5
-            const uint32_t any_n = M[0] | M[1] | M[2] | M[3] | (M[4] & 0xF0000000u);
+            const uint32_t any_n = NS ? sst : M[0] | M[1] | M[2] | M[3] | (M[4] & 0xF0000000u);
             uint32_t PV[4] = {0u, 0u, 0u, 0u};
 #ifdef DIG_LB_UNIFORM_PATH
             if (__all_sync(0xffffffffu, any_n == 0u && lo5 <= 2 && hi5 >= 130)) {
@@ -733,7 +820,10 @@ __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int
 #endif
                 lb_pairs<false>(D, tabl, A.k32, top_r, PV);
                 npairs += 64u;
-            } else if (k < g.nch) {
+            } else if (k < g.nch && (!NS || sst != 3u)) {                    // (an all-N span has no valid centre)
+                if constexpr (NS) {
+                    if (sst != 0u) lb_mask_global(A.nmask, A.n_bases, g.O + base, M);       // mixed: rare, N-run edges
+                }
                 const int lo3 = g.lo3 - base, hi3 = g.hi3 - base;
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
@@ -1046,7 +1136,7 @@ __device__ __forceinline__ void lb_pairs4(const uint32_t (&D)[9], uint32_t tabl,
     }
 }
 
-template <int TEAMS>
+template <int TEAMS, bool NS>
 __device__ __forceinline__ void lb_consumer_tri(const LbArgs &A, uint32_t sbase, int team, int warp, int lane)
 {
     using L = TriL<TEAMS>;                                     // `warp` = index inside the team
@@ -1097,17 +1187,24 @@ __device__ __forceinline__ void lb_consumer_tri(const LbArgs &A, uint32_t sbase,
                 continue;
             }
             const uint32_t dptr = stg + lb_dstrip(lane) + (uint32_t)span * 32u;
-            const uint32_t mptr = stg + lb_mstrip(lane) + (uint32_t)span * 16u;
-            uint32_t D[9], M[5];
+            uint32_t D[9], M[5] = {0u, 0u, 0u, 0u, 0u}, sst = 0u;
+            uint32_t dep;
             {
-                const uint4 a = lds128(dptr), c = lds128(dptr + 16u), m = lds128(mptr);
+                const uint4 a = lds128(dptr), c = lds128(dptr + 16u);
                 D[0] = a.x; D[1] = a.y; D[2] = a.z; D[3] = a.w;
                 D[4] = c.x; D[5] = c.y; D[6] = c.z; D[7] = c.w;
                 D[8] = lds32(dptr + 32u);
-                M[0] = m.x; M[1] = m.y; M[2] = m.z; M[3] = m.w;
-                M[4] = lds32(mptr + 16u);
+                if constexpr (NS) {                                          // span state (lb_span_states), in the mask's place
+                    sst = (lds32(stg + LB_MBASE + (uint32_t)lb_win(lane) * 4u) >> (2 * span)) & 3u;
+                    dep = (D[0] | D[4]) ^ (D[8] | sst);
+                } else {
+                    const uint32_t mptr = stg + lb_mstrip(lane) + (uint32_t)span * 16u;
+                    const uint4 m = lds128(mptr);
+                    M[0] = m.x; M[1] = m.y; M[2] = m.z; M[3] = m.w;
+                    M[4] = lds32(mptr + 16u);
+                    dep = (D[0] | D[4]) ^ (D[8] | M[0]) ^ M[4];
+                }
             }
-            const uint32_t dep = (D[0] | D[4]) ^ (D[8] | M[0]) ^ M[4];
             __syncwarp();
             if (lane == 0) mbar_arrive_after_loads(bar + 8u * (R::EMPTY0 + stage), dep, A.zero);
             if (!clean) {
@@ -1120,11 +1217,14 @@ __device__ __forceinline__ void lb_consumer_tri(const LbArgs &A, uint32_t sbase,
             LB_T(t_p0);
             const int base = k * LB_CHUNK + span * LB_SPAN;
             const int lo3 = g.lo3 - base, hi3 = g.hi3 - base;                // centre c (local base index) valid: lo3 <= c < hi3
-            const uint32_t any_n = M[0] | M[1] | M[2] | M[3] | (M[4] & 0xF0000000u);
+            const uint32_t any_n = NS ? sst : M[0] | M[1] | M[2] | M[3] | (M[4] & 0xF0000000u);
             uint32_t PV[4] = {0u, 0u, 0u, 0u};
             if (any_n == 0u && lo3 <= 2 && hi3 >= 130) {
                 lb_pairs4<false>(D, tabl, k128, PV);
-            } else if (k < g.nch) {
+            } else if (k < g.nch && (!NS || sst != 3u)) {
+                if constexpr (NS) {
+                    if (sst != 0u) lb_mask_global(A.nmask, A.n_bases, g.O + base, M);
+                }
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     // bit 31 - t of word j <-> centre at local base 32 j + t + 2, its trinucleotide = bases 32 j + t + 1 .. + 3
@@ -1274,7 +1374,7 @@ __device__ __forceinline__ void lb_writer_tri(const LbArgs &A, uint32_t sbase, i
     }
 }
 
-template <bool TOT, int TEAMS>
+template <bool TOT, int TEAMS, bool NS>
 __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_tri_kernel(const LbArgs A, const __grid_constant__ LbMaps imaps)
 {
     using L = TriL<TEAMS>;
@@ -1302,7 +1402,7 @@ __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_tri_kernel(const LbArgs
     __syncthreads();
     if (warp >= LB_CW + LB_WW) {
         const int pw = warp - LB_CW - LB_WW, team = pw / L::PW;
-        lb_producer<L::GM>(A, &imaps,
+        lb_producer<L::GM, NS>(A, &imaps,
                            LbTeam{(int64_t)blockIdx.x * TEAMS + team, (int64_t)gridDim.x * TEAMS, sbase + L::BAR + (uint32_t)team * 128u,
                                   sbase + L::STG + (uint32_t)team * R::NST * LB_STAGE_BYTES, TEAMS == 1 ? 3 : 4},
                            pw % L::PW, lane);
@@ -1310,11 +1410,11 @@ __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_tri_kernel(const LbArgs
         const int ww = warp - LB_CW;
         lb_writer_tri<TOT, TEAMS>(A, sbase, ww / L::WW, ww % L::WW, lane);
     } else {
-        lb_consumer_tri<TEAMS>(A, sbase, warp / L::CW, warp % L::CW, lane);
+        lb_consumer_tri<TEAMS, NS>(A, sbase, warp / L::CW, warp % L::CW, lane);
     }
 }
 
-template <bool TRI, bool TOT>
+template <bool TRI, bool TOT, bool NS>
 __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_kernel(const LbArgs A, const __grid_constant__ CUtensorMap tmap,
                                                                 const __grid_constant__ LbMaps imaps)
 {
@@ -1333,6 +1433,8 @@ __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_kernel(const LbArgs A, 
         mbar_init(bar + 8u * (BAR_EMPTY + 1), LB_CW);
         mbar_init(bar + 8u * BAR_FULL2, 32u);
         mbar_init(bar + 8u * BAR_EMPTY2, LB_CW);
+        mbar_init(bar + 8u * BAR_FULL3, 32u);
+        mbar_init(bar + 8u * BAR_EMPTY3, LB_CW);
         mbar_init(bar + 8u * BAR_OUTFREE, LB_WW);
 #pragma unroll
         for (int i = 0; i < LB_NOUT; ++i) {
@@ -1346,10 +1448,10 @@ __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_kernel(const LbArgs A, 
     }
     __syncthreads();
     if (warp >= LB_CW + LB_WW)
-        lb_producer<TRI>(A, &imaps, LbTeam{(int64_t)blockIdx.x, (int64_t)gridDim.x, sbase + OFF_BAR, sbase + LbRing<TRI>::STG0, 3},
+        lb_producer<TRI, NS>(A, &imaps, LbTeam{(int64_t)blockIdx.x, (int64_t)gridDim.x, sbase + OFF_BAR, sbase + LbRing<TRI>::STG0, 3},
                          warp - LB_CW - LB_WW, lane);
     else if (warp >= LB_CW) lb_writer<TRI, TOT>(A, &tmap, sbase, warp - LB_CW, lane);
-    else lb_consumer<TRI>(A, sbase, warp, lane);
+    else lb_consumer<TRI, NS>(A, sbase, warp, lane);
 }
 
 typedef CUresult (*LbEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
@@ -1428,11 +1530,11 @@ int lb_input_maps(LbMaps *maps, LbArgs &A, int64_t tile_w)
 #ifndef DIG_LB_TRI_TEAMS
 #define DIG_LB_TRI_TEAMS 2
 #endif
-template <bool TOT>
+template <bool TOT, bool NS>
 int launch_lb_tri(const LbArgs &A, const LbMaps &imaps, cudaStream_t stream)
 {
     constexpr int TEAMS = DIG_LB_TRI_TEAMS;
-    auto kern = scan_lb_tri_kernel<TOT, TEAMS>;
+    auto kern = scan_lb_tri_kernel<TOT, TEAMS, NS>;
     static thread_local bool attr_set = false;
     if (!attr_set) {
         DIG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TriL<TEAMS>::SMEM));
@@ -1446,10 +1548,10 @@ int launch_lb_tri(const LbArgs &A, const LbMaps &imaps, cudaStream_t stream)
     return DIG_OK;
 }
 
-template <bool TRI, bool TOT>
+template <bool TRI, bool TOT, bool NS>
 int launch_lb(const LbArgs &A, const CUtensorMap &tmap, const LbMaps &imaps, cudaStream_t stream)
 {
-    auto kern = scan_lb_kernel<TRI, TOT>;
+    auto kern = scan_lb_kernel<TRI, TOT, NS>;
     static thread_local bool attr_set = false;
     if (!attr_set) {
         DIG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LB_SMEM));
@@ -1485,7 +1587,7 @@ bool scan_lb_usable(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, con
 
 // Lane-bank scan of all regions, then the per-warp hexamer kernel over the regions it listed (overflowed batches,
 // regions longer than LB_MAX_CHUNKS chunks).  The list lives in the caller's workspace; no host synchronisation.
-int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int64_t *chrom_off,
+int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, const uint32_t *nsum, int64_t n_bases, const int64_t *chrom_off,
                    const int64_t *chrom_len, const int32_t *reg_chrom, const int64_t *reg_start, const int64_t *reg_end,
                    int64_t n_reg, int32_t *counts5, int32_t *counts3, unsigned long long *totals5,
                    unsigned long long *totals3, unsigned int tot_limit_kb, void *workspace, int64_t tile_window,
@@ -1501,7 +1603,7 @@ int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, cons
     }
     DIG_CUDA(cudaMemsetAsync(fb_count, 0, 16, stream));
     LbArgs A;
-    A.p2 = p2; A.nmask = nm; A.n_bases = n_bases; A.chrom_off = chrom_off; A.chrom_len = chrom_len;
+    A.p2 = p2; A.nmask = nm; A.nsum = nsum; A.n_bases = n_bases; A.chrom_off = chrom_off; A.chrom_len = chrom_len;
     A.reg_chrom = reg_chrom; A.reg_start = reg_start; A.reg_end = reg_end; A.n_reg = n_reg;
     A.counts5 = counts5; A.counts3 = counts3; A.totals5 = totals5; A.totals3 = totals3;
     A.k32 = 32u; A.top = 0x01000000u; A.zero = 0u;
@@ -1521,7 +1623,10 @@ int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, cons
     if (counts5 == nullptr) {
         // trinucleotide table alone: 4-mer pairs in 32-bit lane-bank counters, then the per-warp kernel over the list
         // (regions beyond LB_MAX_CHUNKS_TRI chunks, batches whose exception list overflowed)
-        rc = totals3 != nullptr ? launch_lb_tri<true>(A, imaps, stream) : launch_lb_tri<false>(A, imaps, stream);
+        if (nsum != nullptr)
+            rc = totals3 != nullptr ? launch_lb_tri<true, true>(A, imaps, stream) : launch_lb_tri<false, true>(A, imaps, stream);
+        else
+            rc = totals3 != nullptr ? launch_lb_tri<true, false>(A, imaps, stream) : launch_lb_tri<false, false>(A, imaps, stream);
         if (rc != DIG_OK) return rc;
         rc = launch_scan_tri_list(p2, nm, n_bases, chrom_off, chrom_len, reg_chrom, reg_start, reg_end, n_reg, counts3,
                                   totals3, tot_limit_kb, fb_list, fb_count, stream);
@@ -1531,10 +1636,17 @@ int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, cons
         }
         return rc;
     }
-    if (counts3 != nullptr)
-        rc = totals5 != nullptr ? launch_lb<true, true>(A, tmap, imaps, stream) : launch_lb<true, false>(A, tmap, imaps, stream);
-    else
-        rc = totals5 != nullptr ? launch_lb<false, true>(A, tmap, imaps, stream) : launch_lb<false, false>(A, tmap, imaps, stream);
+    if (nsum != nullptr) {
+        if (counts3 != nullptr)
+            rc = totals5 != nullptr ? launch_lb<true, true, true>(A, tmap, imaps, stream) : launch_lb<true, false, true>(A, tmap, imaps, stream);
+        else
+            rc = totals5 != nullptr ? launch_lb<false, true, true>(A, tmap, imaps, stream) : launch_lb<false, false, true>(A, tmap, imaps, stream);
+    } else {
+        if (counts3 != nullptr)
+            rc = totals5 != nullptr ? launch_lb<true, true, false>(A, tmap, imaps, stream) : launch_lb<true, false, false>(A, tmap, imaps, stream);
+        else
+            rc = totals5 != nullptr ? launch_lb<false, true, false>(A, tmap, imaps, stream) : launch_lb<false, false, false>(A, tmap, imaps, stream);
+    }
     if (rc != DIG_OK) return rc;
     rc = launch_scan_hex(p2, nm, n_bases, chrom_off, chrom_len, reg_chrom, reg_start, reg_end, n_reg, counts5, counts3,
                          totals5, totals3, tot_limit_kb, false, fb_list, fb_count, stream);

@@ -66,6 +66,20 @@ class Genome:
         return (s if start is None else s[start:end]).tobytes().decode()
 
 
+def nsum_layout(n_mask_words):
+    """(offset in words, number of words) of the per-128-base N summary that follows a mask of n_mask_words words in
+    the same allocation (dig_scan_opts.nsum_offset_words)."""
+    return (n_mask_words + 3) // 4 * 4, max(((n_mask_words + 3) // 4 + 15) // 16, 1)
+
+
+def alloc_nmask(n_mask_words, device):
+    """An int32 N mask of n_mask_words words with room for its N summary behind it (summary blocks read as all N)."""
+    off, nsw = nsum_layout(n_mask_words)
+    buf = torch.empty(off + nsw, dtype=torch.int32, device=device)
+    buf[off:].fill_(-1)
+    return buf[:n_mask_words]
+
+
 def _layout(lengths):
     lengths = np.asarray(lengths, dtype=np.int64)
     padded = (lengths + ALIGN - 1) // ALIGN * ALIGN
@@ -77,20 +91,40 @@ def _layout(lengths):
 
 
 class DeviceGenome:
-    """2-bit packed genome + N mask in HBM, with per-chromosome offsets (global coordinates)."""
+    """2-bit packed genome + N mask in HBM, with per-chromosome offsets (global coordinates).
 
-    def __init__(self, names, chrom_len, chrom_off, n_bases, packed2, nmask, n_other, device):
+    ``nsum`` is the per-128-base N summary of ``nmask`` (dig_nmask_summary, 2 bits per block), stored ``nsum_offset``
+    words behind the mask in the same allocation (alloc_nmask; a mask without that room is copied into such a buffer):
+    the lane-bank scan reads it instead of staging the mask.  It is built here from ``nmask``; whoever rewrites words of
+    ``nmask`` afterwards calls ``rebuild_nsum`` over the same words (build_nsum=False: the mask is filled later)."""
+
+    def __init__(self, names, chrom_len, chrom_off, n_bases, packed2, nmask, n_other, device, build_nsum=True):
         self.names = list(names)
         self._index = {n: i for i, n in enumerate(self.names)}
         self.chrom_len = np.asarray(chrom_len, dtype=np.int64)
         self.chrom_off = np.asarray(chrom_off, dtype=np.int64)
         self.n_bases = int(n_bases)
         self.packed2 = packed2
+        self.nsum_offset, nsw = nsum_layout(nmask.numel())
+        if not nmask.is_contiguous() or nmask.untyped_storage().nbytes() < (nmask.storage_offset() + self.nsum_offset + nsw) * 4:
+            m = alloc_nmask(nmask.numel(), nmask.device)
+            m.copy_(nmask)
+            nmask = m
         self.nmask = nmask
+        self.nsum = nmask.as_strided((nsw,), (1,), nmask.storage_offset() + self.nsum_offset)
         self.n_other = int(n_other)
         self.device = device
         self.chrom_len_d = torch.from_numpy(self.chrom_len).to(device)
         self.chrom_off_d = torch.from_numpy(self.chrom_off).to(device)
+        if build_nsum:
+            self.rebuild_nsum(0, nmask.numel())
+
+    def rebuild_nsum(self, word0, n_words, stream=None):
+        """Rebuild the summary of mask words [word0, word0 + n_words) (word0 a multiple of 4) on `stream`."""
+        st = stream if stream is not None else torch.cuda.current_stream(self.nmask.device)
+        with torch.cuda.device(self.nmask.device):
+            _lib.call("dig_nmask_summary", self.nmask.data_ptr(), int(word0), int(n_words), self.nsum.data_ptr(),
+                      st.cuda_stream)
 
     def index(self, name):
         return self._index[name]
@@ -122,7 +156,7 @@ class DeviceGenome:
         n = ascii_d.numel()
         dev = ascii_d.device
         packed2 = torch.empty(max(int(lib.dig_packed_words(n)), 2), dtype=torch.int32, device=dev)
-        nmask = torch.empty(max(int(lib.dig_nmask_words(n)), 1), dtype=torch.int32, device=dev)
+        nmask = alloc_nmask(max(int(lib.dig_nmask_words(n)), 1), dev)
         n_other = torch.zeros(1, dtype=torch.int64, device=dev)
         st = stream if stream is not None else torch.cuda.current_stream(dev)
         with torch.cuda.device(dev):

@@ -24,7 +24,7 @@ import numpy as np
 import torch
 
 from . import _lib, kernels
-from .genome import DeviceGenome, Genome, _layout
+from .genome import DeviceGenome, Genome, _layout, alloc_nmask
 
 CACHE_VERSION = 2
 
@@ -233,7 +233,7 @@ class HostScan:
         lib = _lib.load()
         # device: the packed genome (kept), the ASCII landing buffer (ASCII sources), the count tables
         self.packed2 = torch.empty(max(int(lib.dig_packed_words(n)), 2), dtype=torch.int32, device=dev)
-        self.nmask = torch.empty(max(int(lib.dig_nmask_words(n)), 1), dtype=torch.int32, device=dev)
+        self.nmask = alloc_nmask(max(int(lib.dig_nmask_words(n)), 1), dev)       # with room for its N summary
         self.n_other_d = torch.zeros(1, dtype=torch.int64, device=dev)
         self.dev_ascii = None if hg.is_packed else torch.empty(max(n, 1), dtype=torch.uint8, device=dev)
         self.runs_d, self.run_lo = None, None
@@ -245,7 +245,8 @@ class HostScan:
             word_off = np.append(hg.chrom_off // 32, (n + 31) // 32)
             self.run_lo = np.searchsorted(runs[:, 0], word_off, side="left") if len(runs) else np.zeros(len(word_off), dtype=np.int64)
             self.word_off = word_off
-        self.genome = DeviceGenome(hg.names, hg.chrom_len, hg.chrom_off, n, self.packed2, self.nmask, hg.n_other, dev)
+        self.genome = DeviceGenome(hg.names, hg.chrom_len, hg.chrom_off, n, self.packed2, self.nmask, hg.n_other, dev,
+                                   build_nsum=False)
         self.win_chrom = torch.from_numpy(w[:, 0].astype(np.int32)).to(dev)
         self.win_start = torch.from_numpy(np.ascontiguousarray(w[:, 1])).to(dev)
         self.win_end = torch.from_numpy(np.ascontiguousarray(w[:, 2])).to(dev)
@@ -293,14 +294,17 @@ class HostScan:
         hg = self.hg
         a = int(hg.chrom_off[c])
         b = int(hg.chrom_off[c + 1]) if c + 1 < len(hg.chrom_off) else hg.n_bases
-        if hg.is_packed and self.runs_d is not None and b > a:
+        if b <= a:
+            return
+        if hg.is_packed and self.runs_d is not None:
             lo, hi = int(self.run_lo[c]), int(self.run_lo[c + 1])
             _lib.call("dig_nmask_fill_runs", self.runs_d.data_ptr() + lo * 24, hi - lo, self.nmask.data_ptr(),
                       int(self.word_off[c]), int(self.word_off[c + 1] - self.word_off[c]), stream.cuda_stream)
-        if hg.is_packed or b <= a:
-            return
-        _lib.call("dig_pack_genome", self.dev_ascii.data_ptr() + a, b - a, self.packed2.data_ptr() + a // 16 * 4,
-                  self.nmask.data_ptr() + a // 32 * 4, self.n_other_d.data_ptr(), stream.cuda_stream)
+        elif not hg.is_packed:
+            _lib.call("dig_pack_genome", self.dev_ascii.data_ptr() + a, b - a, self.packed2.data_ptr() + a // 16 * 4,
+                      self.nmask.data_ptr() + a // 32 * 4, self.n_other_d.data_ptr(), stream.cuda_stream)
+        # this chromosome's mask words were just rewritten (copy, runs or pack): its part of the N summary follows them
+        self.genome.rebuild_nsum(a // 32, (b + 31) // 32 - a // 32, stream)
 
     def _scan(self, lo, hi, stream):
         g = self.genome

@@ -38,10 +38,11 @@ def _tile_hint(reg_start, reg_end, tile_window):
     return w if w > 0 and bool(np.all(e - s == w)) else 0
 
 
-def _scan_opts(dev, n_reg, variant, totals_limit_kb, workspace, tile_window=0, peer_rows=None, mc_rows=None):
+def _scan_opts(dev, n_reg, variant, totals_limit_kb, workspace, tile_window=0, peer_rows=None, mc_rows=None, genome=None):
     """dig_scan_opts for one scan call: the device scratch the lane-bank kernel needs (caller-owned, sized by
     dig_scan_workspace_bytes) plus the A/B knobs.  peer_rows: device addresses (ints) of the trinucleotide row block in
-    every rank's peer-mapped buffer (fused all-gather), mc_rows its multicast alias.
+    every rank's peer-mapped buffer (fused all-gather), mc_rows its multicast alias.  genome: its per-128-base N summary
+    (DeviceGenome.nsum, None = none) goes with the call.
     Returns (struct, byref, workspace tensor to keep alive)."""
     import ctypes
     if workspace is None and n_reg > 0:
@@ -56,6 +57,10 @@ def _scan_opts(dev, n_reg, variant, totals_limit_kb, workspace, tile_window=0, p
         for i, a in enumerate(peer_rows):
             opts.peer_counts3_d[i] = int(a)
         opts.mc_counts3_d = int(mc_rows) if mc_rows else None
+    if genome is not None and getattr(genome, "nsum", None) is not None:
+        # the summary lives in the mask's allocation, nsum_offset words after it
+        assert genome.nsum.data_ptr() == genome.nmask.data_ptr() + 4 * genome.nsum_offset
+        opts.nsum_offset_words = genome.nsum_offset
     return opts, ctypes.byref(opts), workspace
 
 
@@ -97,7 +102,7 @@ def count_contexts(genome, reg_chrom, reg_start, reg_end, n_up=1, n_down=1, stra
     opts, opts_ref, workspace = _scan_opts(dev, n if lane_bank else 0, variant, totals_limit_kb,
                                            workspace if lane_bank else None,
                                            _tile_hint(reg_start, reg_end, tile_window) if lane_bank else 0,
-                                           peer_rows, mc_rows)
+                                           peer_rows, mc_rows, genome)
     with torch.cuda.device(dev):
         _lib.call("dig_count_contexts", genome.packed2.data_ptr(), genome.nmask.data_ptr(), genome.n_bases,
                   genome.chrom_off_d.data_ptr(), genome.chrom_len_d.data_ptr(), rc.data_ptr(), rs.data_ptr(),
@@ -129,7 +134,7 @@ def count_contexts_fused53(genome, reg_chrom, reg_start, reg_end, want_totals=Fa
     opts, opts_ref, workspace = _scan_opts(dev, n if lane_bank else 0, variant, totals_limit_kb,
                                            workspace if lane_bank else None,
                                            _tile_hint(reg_start, reg_end, tile_window) if lane_bank else 0,
-                                           peer_rows, mc_rows)
+                                           peer_rows, mc_rows, genome)
     with torch.cuda.device(dev):
         _lib.call("dig_count_contexts_fused53", genome.packed2.data_ptr(), genome.nmask.data_ptr(), genome.n_bases,
                   genome.chrom_off_d.data_ptr(), genome.chrom_len_d.data_ptr(), rc.data_ptr(), rs.data_ptr(),

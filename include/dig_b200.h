@@ -108,7 +108,13 @@ typedef struct dig_scan_opts {
      * multicast alias of the same block: one multimem store then reaches all ranks.  Up to 8 peers; lane-bank kernel
      * only (DIG_ERR_ARG otherwise).  The caller orders the ranks afterwards (a device barrier) before reading. */
     int32_t n_peer_counts3;
-    int32_t reserved0;
+    /* Per-128-base N summary of nmask_d (dig_nmask_summary): 0 = none.  > 0: the summary starts this many uint32 words
+     * after nmask_d, in the same allocation (a multiple of 4, at least dig_nmask_words(n_bases)).  With it the
+     * lane-bank kernel stages the packed bases alone (no mask) and reads each 128-base span's state -- no N, all N, or
+     * mixed -- from the summary; only mixed spans read their mask words, from global memory.  The summary must describe
+     * nmask_d as it is at the time of the call (rebuild the part that covers any mask words you rewrite).  Results are
+     * identical with and without it. */
+    int32_t nsum_offset_words;
     void *peer_counts3_d[8];
     void *mc_counts3_d;
 } dig_scan_opts;
@@ -145,6 +151,13 @@ int dig_narrow_counts_u16(const int32_t *counts_d, int64_t n_values, uint16_t *o
  * int64: (first word, number of words, 32-bit word value), disjoint.  Words [word0, word0 + n_words) of nmask_d are
  * cleared, then the runs (clipped to that range) are written. */
 int dig_nmask_fill_runs(const int64_t *runs_d, int64_t n_runs, uint32_t *nmask_d, int64_t word0, int64_t n_words, void *stream);
+
+/* Per-128-base N summary of an N mask: two bits per aligned block of 128 bases (four mask words), block j at bits
+ * 2 (j & 15) and 2 (j & 15) + 1 of word j >> 4 of nsum_d: bit 0 = the block holds an N, bit 1 = every base of it is N
+ * (00 clean, 01 mixed, 11 all N).  Rebuilds the blocks of mask words [word0, word0 + n_words) and leaves every other
+ * block's bits as they are; word0 must be a multiple of 4, and mask words past word0 + n_words inside the last block
+ * count as all N.  nsum_d holds ceil(ceil(n_mask_words / 4) / 16) words for the whole mask (3.1 Gb: 6 MB). */
+int dig_nmask_summary(const uint32_t *nmask_d, int64_t word0, int64_t n_words, uint32_t *nsum_d, void *stream);
 
 /* The same nbytes (a multiple of 16; 16-byte aligned pointers) copied from src_d to each of the n_dst <= 8 device
  * pointers in dst_d (a HOST array): peer-mapped buffers of the other ranks.  Used for the partial genome totals of a
