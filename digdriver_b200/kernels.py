@@ -729,3 +729,104 @@ def element_psum(L, region_counts, d_pr, device="cuda:0", stream=None, want_deno
         _lib.call("dig_element_psum", Ld.data_ptr(), Rd.data_ptr(), dp.data_ptr(), n, p.data_ptr(), _ptr(den),
                   _stream(dev, stream))
     return (p[:n], den[:n]) if want_denom else p[:n]
+
+
+# ---------------------------------------------------------------------------------------------
+# K9: gene annotation from a CDS gene set (csrc/cdsannot.cu)
+# ---------------------------------------------------------------------------------------------
+
+CDS_CLASS_NAMES = {0: "Synonymous", 1: "Missense", 2: "Nonsense", 3: "Essential_Splice", 5: "Stop_loss"}
+CDS_NO_HIT = 255
+
+
+def _splice_offsets(donor, acceptor):
+    """ctypes int32 arrays (host) of the donor / acceptor intron offsets."""
+    import ctypes
+    d, a = [int(x) for x in donor], [int(x) for x in acceptor]
+    return (ctypes.c_int32 * max(len(d), 1))(*d), len(d), (ctypes.c_int32 * max(len(a), 1))(*a), len(a)
+
+
+def _check_cds_status(status, what):
+    code = int(status.item())
+    if code:
+        why = [m for bit, m in ((1, "a gene has more than 2048 CDS blocks"),
+                                (2, "a gene's chromosome or block lies outside the genome"),
+                                (4, "a gene's blocks are not strictly ascending")) if code & bit]
+        raise _lib.DigError("%s: %s" % (what, "; ".join(why)))
+
+
+def cds_substitution_table(genome, gene_chrom, gene_strand, blk_ptr, blk_start, blk_end, donor=(1, 2, 5),
+                           acceptor=(1, 2), stream=None):
+    """K9a: per-gene substitution table of the CDS.  Blocks are inclusive [start, end] chromosome coordinates,
+    ascending within each gene; gene_chrom indexes the genome.  Returns (L float64 [E, 192, 4] = silent, missense,
+    nonsense, essential splice; flags int32 [E]) on the device."""
+    dev = genome.device
+    gc, gs = _dev(gene_chrom, torch.int32, dev), _dev(gene_strand, torch.int8, dev)
+    bp, bs, be = (_dev(x, torch.int64, dev) for x in (blk_ptr, blk_start, blk_end))
+    E = gc.numel()
+    L = torch.empty((max(E, 1), 192, 4), dtype=torch.float64, device=dev)
+    flags = torch.empty(max(E, 1), dtype=torch.int32, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    d, nd, a, na = _splice_offsets(donor, acceptor)
+    with torch.cuda.device(dev):
+        _lib.call("dig_cds_substitution_table", genome.packed2.data_ptr(), genome.nmask.data_ptr(), genome.n_bases,
+                  genome.chrom_off_d.data_ptr(), genome.chrom_len_d.data_ptr(), len(genome.chrom_len), gc.data_ptr(),
+                  gs.data_ptr(), bp.data_ptr(), bs.data_ptr(), be.data_ptr(), E, d, nd, a, na, L.data_ptr(),
+                  flags.data_ptr(), status.data_ptr(), _stream(dev, stream))
+        _check_cds_status(status, "dig_cds_substitution_table")
+    return L[:E], flags[:E]
+
+
+def annotate_snvs(genome, gene_chrom, gene_strand, blk_ptr, blk_start, blk_end, mut_chrom, mut_pos, mut_alt,
+                  donor=(1, 2, 5), acceptor=(1, 2), stream=None):
+    """K9b: coding class of SNVs in every gene that holds them.  mut_chrom indexes the genome, mut_pos is the 0-based
+    position, mut_alt 0..3 (A/C/G/T).  The SNVs are joined (dig_overlap_count / dig_overlap_fill) against the CDS blocks
+    widened by the largest splice offset, the (mutation, gene) pairs de-duplicated, then classified.  Returns device
+    tensors (pair_mut int64, pair_gene int32, cls uint8), sorted by mutation, then gene; cls is a DIG_CDS_* code
+    (CDS_CLASS_NAMES, CDS_NO_HIT for a pair that is neither a countable coding site nor a splice position)."""
+    dev = genome.device
+    gc, gs = _dev(gene_chrom, torch.int32, dev), _dev(gene_strand, torch.int8, dev)
+    bp, bs, be = (_dev(x, torch.int64, dev) for x in (blk_ptr, blk_start, blk_end))
+    mc, mp, ma = _dev(mut_chrom, torch.int64, dev), _dev(mut_pos, torch.int64, dev), _dev(mut_alt, torch.uint8, dev)
+    E, n_mut = gc.numel(), mp.numel()
+    pad = max([int(x) for x in donor] + [int(x) for x in acceptor] + [0])
+    owner = torch.repeat_interleave(torch.arange(E, dtype=torch.int64, device=dev), bp[1:] - bp[:-1])
+    kc = gc.to(torch.int64)[owner] << 32
+    ks, order = torch.sort(kc | torch.clamp(bs - pad, min=0), stable=True)
+    ke = (kc | (be + 1 + pad))[order]
+    pmax = torch.cummax(ke, 0).values if ke.numel() else ke
+    owner = owner[order]
+    mks = (mc << 32) | mp
+    mke = mks + 1
+    sptr = _stream(dev, stream)
+    empty = (torch.zeros(0, dtype=torch.int64, device=dev), torch.zeros(0, dtype=torch.int32, device=dev),
+             torch.zeros(0, dtype=torch.uint8, device=dev))
+    if n_mut == 0 or ks.numel() == 0:
+        return empty
+    with torch.cuda.device(dev):
+        cnt = torch.empty(n_mut, dtype=torch.int64, device=dev)
+        _lib.call("dig_overlap_count", ks.data_ptr(), ke.data_ptr(), pmax.data_ptr(), ks.numel(), mks.data_ptr(),
+                  mke.data_ptr(), n_mut, cnt.data_ptr(), sptr)
+        off = torch.zeros(n_mut + 1, dtype=torch.int64, device=dev)
+        off[1:] = torch.cumsum(cnt, 0)
+        total = int(off[-1].item())
+        if total == 0:
+            return empty
+        pm = torch.empty(total, dtype=torch.int64, device=dev)
+        pb = torch.empty(total, dtype=torch.int64, device=dev)
+        _lib.call("dig_overlap_fill", ks.data_ptr(), ke.data_ptr(), pmax.data_ptr(), ks.numel(), mks.data_ptr(),
+                  mke.data_ptr(), n_mut, off.data_ptr(), pm.data_ptr(), pb.data_ptr(), sptr)
+        # blocks of one gene may all reach the same SNV: one pair per (mutation, gene), in (mutation, gene) order
+        key = torch.unique(pm * E + owner[pb])
+        pair_mut = torch.div(key, E, rounding_mode="floor")
+        pair_gene = (key - pair_mut * E).to(torch.int32)
+        cls = torch.empty(key.numel(), dtype=torch.uint8, device=dev)
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        d, nd, a, na = _splice_offsets(donor, acceptor)
+        _lib.call("dig_annotate_snvs", genome.packed2.data_ptr(), genome.nmask.data_ptr(), genome.n_bases,
+                  genome.chrom_off_d.data_ptr(), genome.chrom_len_d.data_ptr(), len(genome.chrom_len), gc.data_ptr(),
+                  gs.data_ptr(), bp.data_ptr(), bs.data_ptr(), be.data_ptr(), E, d, nd, a, na, mp.data_ptr(),
+                  ma.data_ptr(), pair_mut.data_ptr(), pair_gene.data_ptr(), key.numel(), cls.data_ptr(),
+                  status.data_ptr(), sptr)
+        _check_cds_status(status, "dig_annotate_snvs")
+    return pair_mut, pair_gene, cls

@@ -486,6 +486,55 @@ int dig_element_psum(const double *L_d, const int64_t *region_counts_d, const do
                      double *p_out_d, double *denom_out_d, void *stream);
 
 /* ---------------------------------------------------------------------------------
+ * K9  gene annotation from a CDS gene set (csrc/cdsannot.cu states the rules in full; DESIGN.md section 5).
+ * Replaces what the reference takes from outside: the L_data [E,192,4] of the genic store (read by genic_model,
+ * genic_driver_tools.py:86-168, never built there) and the GENE / ANNOT columns of scripts/mutationFunction.R.
+ * Genes are a CSR list: gene e owns blocks [blk_ptr[e], blk_ptr[e+1]) of blk_start_d / blk_end_d (int64, INCLUSIVE
+ * chromosome coordinates, strictly ascending, not overlapping), gene_chrom_d int32 indexes chrom_off_d / chrom_len_d
+ * (n_chrom entries), gene_strand_d int8 (< 0 = minus strand).  donor / acceptor are HOST arrays of intron offsets
+ * (each >= 1, at most DIG_CDS_MAX_SPLICE_OFFSETS of each): donor d = intron base +d after the exon, acceptor a = intron
+ * base -a before the next exon, in transcript order.
+ *
+ * dig_cds_substitution_table: L_d float64 [n_gene, 192, 4] (overwritten; exact integers) = number of possible
+ *   substitutions per (bin, class), bin = 3 ctx + rank(ALT) in sorted 'CTX>CTX2' order (strand-aware), columns
+ *   silent, missense, nonsense, essential splice (Stop_loss is counted in none); flags_d int32 [n_gene] DIG_CDS_FLAG_*.
+ *   status_d [1] int32 is OR-ed with DIG_CDS_ERR_* for genes that could not be processed (their rows are zero).
+ * dig_annotate_snvs: class_out_d uint8 [n_pair] = DIG_CDS_* class of SNV pair_mut_d[i] in gene pair_gene_d[i] (the
+ *   (mutation, gene) pairs of an interval join against the CDS blocks widened by the largest splice offset, e.g.
+ *   dig_overlap_fill, de-duplicated); mut_pos_d int64 0-based chromosome position (on the gene's chromosome), mut_alt_d
+ *   uint8 0..3 = A/C/G/T as written (genomic strand).  A coding hit beats a splice hit; DIG_CDS_NO_HIT when the SNV is
+ *   neither a countable coding site (complete codon free of N) nor an essential-splice position of that gene.
+ */
+#define DIG_CDS_SYNONYMOUS 0
+#define DIG_CDS_MISSENSE 1
+#define DIG_CDS_NONSENSE 2
+#define DIG_CDS_ESSENTIAL_SPLICE 3
+#define DIG_CDS_STOP_LOSS 5
+#define DIG_CDS_NO_HIT 255
+#define DIG_CDS_FLAG_LENGTH 1       /* CDS length not a multiple of 3 */
+#define DIG_CDS_FLAG_N 2            /* an N in the CDS */
+#define DIG_CDS_FLAG_STOP 4         /* a stop codon before the last codon */
+#define DIG_CDS_ERR_BLOCKS 1        /* a gene has more than DIG_CDS_MAX_BLOCKS blocks */
+#define DIG_CDS_ERR_RANGE 2         /* chromosome index or block outside the genome */
+#define DIG_CDS_ERR_ORDER 4         /* blocks not strictly ascending / empty */
+#define DIG_CDS_MAX_BLOCKS 2048
+#define DIG_CDS_MAX_SPLICE_OFFSETS 8
+int dig_cds_substitution_table(const uint32_t *packed2_d, const uint32_t *nmask_d, int64_t n_bases,
+                               const int64_t *chrom_off_d, const int64_t *chrom_len_d, int n_chrom,
+                               const int32_t *gene_chrom_d, const int8_t *gene_strand_d, const int64_t *blk_ptr_d,
+                               const int64_t *blk_start_d, const int64_t *blk_end_d, int64_t n_gene,
+                               const int32_t *donor, int n_donor, const int32_t *acceptor, int n_acceptor,
+                               double *L_d, int32_t *flags_d, int32_t *status_d, void *stream);
+int dig_annotate_snvs(const uint32_t *packed2_d, const uint32_t *nmask_d, int64_t n_bases,
+                      const int64_t *chrom_off_d, const int64_t *chrom_len_d, int n_chrom,
+                      const int32_t *gene_chrom_d, const int8_t *gene_strand_d, const int64_t *blk_ptr_d,
+                      const int64_t *blk_start_d, const int64_t *blk_end_d, int64_t n_gene,
+                      const int32_t *donor, int n_donor, const int32_t *acceptor, int n_acceptor,
+                      const int64_t *mut_pos_d, const uint8_t *mut_alt_d, const int64_t *pair_mut_d,
+                      const int32_t *pair_gene_d, int64_t n_pair, uint8_t *class_out_d, int32_t *status_d,
+                      void *stream);
+
+/* ---------------------------------------------------------------------------------
  * Synthetic genome generator (BASELINE.json configs are synthetic): position g is a pure
  * function of (seed, g); identical to orc_synth_genome in oracle/dig_oracle.c.
  */

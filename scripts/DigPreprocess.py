@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """CLI shim with the sub-commands and arguments of the reference's scripts/DigPreprocess.py that lie on the
 hot path: countGenomeContext (the genome scan), addMutationContext, preprocess_element_model,
-initialize_f_data.  Output files are directory stores (or HDF5 when h5py + PyTables exist), see
+initialize_f_data; and two of its own that build the gene annotation the reference takes from outside:
+buildGenicData (the genic store from a BED12 gene set) and annotateMutations (GENE / ANNOT of raw calls).  Output files are directory stores (or HDF5 when h5py + PyTables exist), see
 digdriver_b200/storage.py."""
 import argparse
 import os
@@ -159,6 +160,43 @@ def preprocess_cds_contexts(args):
     storage.Store(args.out_file, "a").write_table(args.out_key, results)
 
 
+def buildGenicData(args):
+    """The genic store (CDS intervals + L_data) of a BED12 gene set; see data_tools/cds_annotation.py."""
+    from digdriver_b200.data_tools import cds_annotation
+    cds_annotation.build_genic_data(args.bed12, args.fasta, args.f_genic, donor=_offset_list(args.donor, '--donor'),
+                                    acceptor=_offset_list(args.acceptor, '--acceptor'), keep_flagged=args.keep_flagged)
+
+
+def _offset_list(text, flag):
+    try:
+        vals = [int(x) for x in text.split(',') if x.strip()]
+    except ValueError:
+        vals = []
+    if not vals or min(vals) < 1 or len(vals) > 8:
+        raise SystemExit("%s takes 1 to 8 comma-separated intron offsets >= 1, got %r" % (flag, text))
+    return vals
+
+
+def annotateMutations(args):
+    """GENE / ANNOT of a 6-column mutation file (CHROM START END REF ALT SAMPLE); the output is the 8-column input of
+    addMutationContext."""
+    import csv
+    with open(args.fmut) as f:
+        first = next(csv.reader(f, delimiter='\t', skipinitialspace=True), [])
+    if len(first) == 5:
+        raise SystemExit("annotateMutations: %s has 5 columns (CHROM POS REF ALT SAMPLE); its coordinate base is "
+                         "ambiguous, so give the 6-column form CHROM START END REF ALT SAMPLE with a 0-based START "
+                         "and END = START + length of REF" % args.fmut)
+    if len(first) != 6:
+        raise SystemExit("annotateMutations: %s has %d columns; expected 6 (CHROM START END REF ALT SAMPLE)"
+                         % (args.fmut, len(first)))
+    from digdriver_b200.data_tools import cds_annotation
+    df_mut = mutation_tools.read_mutation_file(args.fmut, drop_duplicates=False)
+    df_out = cds_annotation.annotate_mutations(df_mut, args.f_genic, args.fasta)
+    print('Saving annotated mutation file: {}'.format(args.fout))
+    df_out.to_csv(args.fout, sep="\t", index=False, header=False)
+
+
 def parse_args(text=None):
     parser = argparse.ArgumentParser(description='Preprocess genome and mutation files for use with Dig (B200).')
     sub = parser.add_subparsers()
@@ -217,6 +255,21 @@ def parse_args(text=None):
     f.add_argument('f_annot_data')
     f.add_argument('f_genome_counts')
     f.set_defaults(func=initialize_data)
+    h = sub.add_parser('buildGenicData', help='build the genic store (CDS + substitution table L_data) of a BED12 gene set')
+    h.add_argument('bed12', help='gene set: one row per gene, CDS = blocks clipped to [thickStart, thickEnd)')
+    h.add_argument('fasta')
+    h.add_argument('f_genic', help='output store, read by DigPretrain.py genicModel')
+    h.add_argument('--donor', default='1,2,5', help='essential-splice donor offsets, intron bases +d after the exon')
+    h.add_argument('--acceptor', default='1,2', help='essential-splice acceptor offsets, intron bases -a before the exon')
+    h.add_argument('--keep-flagged', action='store_true', default=False,
+                   help='keep genes with a CDS length not a multiple of 3, an N, or an internal stop codon')
+    h.set_defaults(func=buildGenicData)
+    m = sub.add_parser('annotateMutations', help='add GENE / ANNOT to a 6-column mutation file')
+    m.add_argument('fmut', help='CHROM START END REF ALT SAMPLE, tab-separated, 0-based START')
+    m.add_argument('f_genic', help='genic store of buildGenicData')
+    m.add_argument('fasta')
+    m.add_argument('fout', help='8-column output: the input of addMutationContext')
+    m.set_defaults(func=annotateMutations)
     return parser.parse_args(text.split()) if text else parser.parse_args()
 
 
