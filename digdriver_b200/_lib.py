@@ -72,6 +72,10 @@ SIGNATURES = {
                                         _P, _P]),
     "dig_annotate_snvs": (_I, [_P, _P, _I64, _P, _P, _I, _P, _P, _P, _P, _P, _I64, _P, _I, _P, _I, _P, _P, _P, _P,
                                _I64, _P, _P, _P]),
+    "dig_codon_sites": (_I, [_P, _P, _I64, _P, _P, _I, _P, _P, _P, _P, _P, _I64, _P, _I64, _P, _P, _P, _P, _P, _P, _P]),
+    "dig_codon_transfer": (_I, [_P, _P, _P, _I64, _P, _P, _P, _I64, _I64, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P,
+                                _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "dig_snv_codons": (_I, [_P, _P, _P, _P, _P, _I64, _P, _P, _P, _P, _P, _P, _P, _I64, _P, _P, _P, _P]),
 }
 
 
@@ -97,7 +101,8 @@ KERNELS_PER_CALL = {
     "dig_window_denominators": 1, "dig_site_test": 1, "dig_gene_dnds_sel": 1, "dig_selection_coefficient": 1, "dig_region_prob_norm": 1, "dig_position_obs": 1, "dig_position_test": 1, "dig_nb_pvalue_exact": 1,
     "dig_nb_pvalue_variant": 1, "dig_loglik": 1, "dig_gene_llr_test": 1, "dig_overlap_count": 1, "dig_overlap_fill": 1,
     "dig_element_region_counts": 1, "dig_element_psum": 1, "dig_narrow_counts_u16": 1, "dig_peer_broadcast": 1, "dig_nmask_fill_runs": 1,
-    "dig_nmask_summary": 1, "dig_cds_substitution_table": 1, "dig_annotate_snvs": 1,
+    "dig_nmask_summary": 1, "dig_cds_substitution_table": 1, "dig_annotate_snvs": 1, "dig_codon_sites": 1,
+    "dig_codon_transfer": 1, "dig_snv_codons": 1,
 }
 launch_count = 0
 

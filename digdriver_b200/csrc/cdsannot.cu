@@ -29,83 +29,20 @@
 // three blocks), reads each base's trinucleotide with one two-word funnel shift (as K3 does) and adds its nine
 // substitutions to a 192 x 4 uint32 shared histogram; one thread per (intron, offset) adds the splice positions.
 // K9b dig_annotate_snvs: one thread per (mutation, gene) pair of the interval join; classifies the SNV in that gene.
-#include "dig_common.cuh"
+#include "cds_common.cuh"
 
 namespace {
 
-constexpr int kThreads = 256;
-constexpr int kMaxBlocks = DIG_CDS_MAX_BLOCKS;
+using namespace dig_cds;
+
 constexpr int kMaxOffsets = DIG_CDS_MAX_SPLICE_OFFSETS;
 constexpr uint8_t kNoHit = 255;
-
-// NCBI standard code, codons in TCAG order (first base slowest)
-__constant__ char kCodeTCAG[65] = "FFLLSSSSYY**CC*WLLLLPPPPHHQQRRRRIIIMTTTTNNKKSSRRVVVVAAAADDEEGGGG";
 
 struct SpliceOffsets {
     int n_don, n_acc;
     int don[kMaxOffsets];
     int acc[kMaxOffsets];
 };
-
-struct GenomeView {
-    const uint32_t *p2, *nm;
-    const int64_t *chrom_off, *chrom_len;
-    int64_t last_p, last_m;
-    int n_chrom;
-};
-
-// amino acid of a codon of ACGT indices (A0 C1 G2 T3): ACGT -> TCAG index is A2 C1 G3 T0
-__device__ __forceinline__ char amino(uint32_t b0, uint32_t b1, uint32_t b2)
-{
-    const uint32_t m = 0x36u;      // 2 | 1 << 2 | 3 << 4 | 0 << 6
-    return kCodeTCAG[(((m >> (2 * b0)) & 3u) << 4) | (((m >> (2 * b1)) & 3u) << 2) | ((m >> (2 * b2)) & 3u)];
-}
-
-// 0 Synonymous, 1 Missense, 2 Nonsense, 5 Stop_loss (DIG_CDS_* codes)
-__device__ __forceinline__ int consequence(char ref_aa, char alt_aa)
-{
-    if (ref_aa == alt_aa) return DIG_CDS_SYNONYMOUS;
-    if (alt_aa == '*') return DIG_CDS_NONSENSE;
-    if (ref_aa == '*') return DIG_CDS_STOP_LOSS;
-    return DIG_CDS_MISSENSE;
-}
-
-__device__ __forceinline__ uint32_t revcomp3(uint32_t c)
-{
-    return ((3u - (c & 3u)) << 4) | ((3u - ((c >> 2) & 3u)) << 2) | (3u - (c >> 4));
-}
-
-struct Site {
-    uint32_t base;   // genomic base (A0 C1 G2 T3)
-    bool base_n;     // the base is not A/C/G/T
-    int32_t ctx;     // genomic trinucleotide p-1..p+1, -1 if it holds an N or leaves the chromosome
-};
-
-// The trinucleotide lies inside two consecutive packed words and its N bits inside two consecutive mask words: four
-// independent loads (one funnel shift each) give the base, its N bit and the context.
-__device__ __forceinline__ Site read_site(const GenomeView &G, int64_t off, int64_t L, int64_t p)
-{
-    const int64_t g = off + p;
-    const int64_t f = p > 0 ? g - 1 : g;
-    const int64_t w = f >> 4, m = f >> 5;
-    const unsigned long long pk =
-        ((unsigned long long)__ldg(G.p2 + w) << 32) | __ldg(G.p2 + (w < G.last_p ? w + 1 : G.last_p));
-    const unsigned long long mk =
-        ((unsigned long long)__ldg(G.nm + m) << 32) | __ldg(G.nm + (m < G.last_m ? m + 1 : G.last_m));
-    const uint32_t key = (uint32_t)(pk >> (64 - 2 * ((int)(f & 15) + 3))) & 63u;
-    const uint32_t bad = (uint32_t)(mk >> (64 - ((int)(f & 31) + 3))) & 7u;
-    Site s;
-    if (p > 0) {
-        s.base = (key >> 2) & 3u;
-        s.base_n = ((bad >> 1) & 1u) != 0u;
-        s.ctx = (p + 1 < L && bad == 0u) ? (int32_t)key : -1;
-    } else {                       // the first base of a chromosome has no upstream neighbour
-        s.base = key >> 4;
-        s.base_n = (bad >> 2) != 0u;
-        s.ctx = -1;
-    }
-    return s;
-}
 
 // Intron-relative index (0 = first intron base after the exon, in transcript order) of splice offset o, or -1 when it
 // falls outside an intron of glen bases or an earlier offset already names the same base.
@@ -134,68 +71,25 @@ __global__ void __launch_bounds__(kThreads) cds_table_kernel(
     __shared__ int32_t s_warp[kThreads / 32];
     __shared__ int s_flags;
 
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x;
     for (int64_t e = blockIdx.x; e < n_gene; e += gridDim.x) {
-        const int64_t b0 = blk_ptr[e];
-        const int64_t nblk = blk_ptr[e + 1] - b0;
-        const int nb64 = nblk > kMaxBlocks ? kMaxBlocks + 1 : (int)nblk;
-        const int c = gene_chrom[e];
-        const bool plus = gene_strand[e] >= 0;
-        int err = 0;
-        if (nb64 > kMaxBlocks) err = DIG_CDS_ERR_BLOCKS;
-        if (nb64 < 0) err = DIG_CDS_ERR_ORDER;
-        if (c < 0 || c >= G.n_chrom) err |= DIG_CDS_ERR_RANGE;
-        const int nb = err ? 0 : nb64;
-        const int64_t off = err ? 0 : G.chrom_off[c], L = err ? 0 : G.chrom_len[c];
         for (int k = tid; k < 192 * 4; k += kThreads) s_hist[k] = 0u;
         if (tid == 0) s_flags = 0;
-        // blocks -> shared memory; each thread owns a contiguous chunk for the prefix sum
-        const int chunk = (nb + kThreads - 1) / kThreads;
-        const int i0 = min(tid * chunk, nb), i1 = min(i0 + chunk, nb);
-        int32_t local = 0;
-        for (int i = i0; i < i1; ++i) {
-            const int64_t s = blk_start[b0 + i], t = blk_end[b0 + i];
-            if (s < 0 || t >= L) err |= DIG_CDS_ERR_RANGE;
-            if (t < s || (i > 0 && s <= blk_end[b0 + i - 1])) err |= DIG_CDS_ERR_ORDER;
-            s_start[i] = s;
-            local += (int32_t)(t - s + 1);
-        }
-        // block-wide exclusive scan of the chunk sums
-        int32_t incl = local;
-        for (int d = 1; d < 32; d <<= 1) {
-            const int32_t v = __shfl_up_sync(0xffffffffu, incl, d);
-            if (lane >= d) incl += v;
-        }
-        if (lane == 31) s_warp[warp] = incl;
-        const int any_err = __syncthreads_or(err);
-        if (any_err) {
-            if (err) atomicOr(status, err);
+        GeneCds gc;
+        if (load_gene_cds(G, gene_chrom, gene_strand, blk_ptr, blk_start, blk_end, e, s_start, s_cum, s_warp, gc,
+                          status)) {
             for (int k = tid; k < 192 * 4; k += kThreads) L_out[e * 768 + k] = 0.0;
             if (tid == 0) flags_out[e] = 0;
             __syncthreads();
             continue;
         }
-        int32_t base = 0;
-        for (int w = 0; w < warp; ++w) base += s_warp[w];
-        int32_t run = base + incl - local;
-        for (int i = i0; i < i1; ++i) {
-            s_cum[i] = run;
-            run += (int32_t)(blk_end[b0 + i] - s_start[i] + 1);
-        }
-        if (tid == kThreads - 1) s_cum[nb] = base + incl;
-        __syncthreads();
+        const int64_t b0 = blk_ptr[e];
+        const int nb = gc.nb;
+        const bool plus = gc.plus;
+        const int64_t off = gc.off, L = gc.L;
         const int32_t T = s_cum[nb];
         const int32_t n_full = T / 3;
-        // transcript base t -> genomic position
-        auto locate = [&](int32_t t) -> int64_t {
-            const int32_t i = plus ? t : T - 1 - t;
-            int lo = 0, hi = nb - 1;                  // last block with s_cum <= i
-            while (lo < hi) {
-                const int mid = (lo + hi + 1) >> 1;
-                if (s_cum[mid] <= i) lo = mid; else hi = mid - 1;
-            }
-            return s_start[lo] + (i - s_cum[lo]);
-        };
+        auto locate = [&](int32_t t) -> int64_t { return cds_locate(s_start, s_cum, nb, T, plus, t); };
         int flags = (T % 3) ? DIG_CDS_FLAG_LENGTH : 0;
         for (int32_t k = tid; 3 * k < T; k += kThreads) {
             const int nbase = min(3, T - 3 * k);
@@ -314,19 +208,6 @@ __global__ void __launch_bounds__(kThreads) annotate_snvs_kernel(
         }
         cls_out[i] = cls;
     }
-}
-
-int make_view(GenomeView &G, const uint32_t *packed2_d, const uint32_t *nmask_d, int64_t n_bases,
-              const int64_t *chrom_off_d, const int64_t *chrom_len_d, int n_chrom)
-{
-    G.p2 = packed2_d;
-    G.nm = nmask_d;
-    G.chrom_off = chrom_off_d;
-    G.chrom_len = chrom_len_d;
-    G.last_m = ((n_bases + 31) >> 5) - 1;
-    G.last_p = (((n_bases + 31) >> 5) << 1) - 1;
-    G.n_chrom = n_chrom;
-    return DIG_OK;
 }
 
 int make_offsets(SpliceOffsets &S, const int32_t *donor, int n_donor, const int32_t *acceptor, int n_acceptor)

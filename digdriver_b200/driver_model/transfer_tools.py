@@ -384,10 +384,10 @@ def run_element_region_model(f_mut, f_bed, f_h5_pretrain, pretrain_key, scale_fa
     return finish_element_model(df_mut_tab, df_pretrain, cj, cj_indel, skip_pvals=skip_pvals)
 
 
-def run_sites_region_model(f_mut, f_sites, f_h5_pretrain, pretrain_key, scale_factor=None, scale_type="genome",
-                           scale_by_expectation=True):
-    """Run a model on an arbitrary set of sites of interest (reference :1098-1169)."""
-    df_pretrain = load_pretrained_model(f_h5_pretrain, key=pretrain_key, restrict_cols=True)
+def sites_scale_factor(f_mut, f_h5_pretrain, scale_factor=None, scale_type="genome", scale_by_expectation=True):
+    """cj of the site-set models (reference :1098-1169): observed Synonymous outside TP53 over sum(MU * Pi_SYN) of the
+    store's genic_model, else the manual factor, else calc_scale_factor_efficient.  Shared by run_sites_region_model
+    and the codon model."""
     if scale_by_expectation:
         print('scaling by expected synonymous mutations (excluding TP53)')
         df_gene = load_pretrained_model(f_h5_pretrain)
@@ -401,6 +401,14 @@ def run_sites_region_model(f_mut, f_sites, f_h5_pretrain, pretrain_key, scale_fa
         print('Calculating scale factor')
         cj = calc_scale_factor_efficient(f_mut, f_h5_pretrain, scale_type=scale_type)[0]
     print("\tScale factor is: {}".format(cj))
+    return cj
+
+
+def run_sites_region_model(f_mut, f_sites, f_h5_pretrain, pretrain_key, scale_factor=None, scale_type="genome",
+                           scale_by_expectation=True):
+    """Run a model on an arbitrary set of sites of interest (reference :1098-1169)."""
+    df_pretrain = load_pretrained_model(f_h5_pretrain, key=pretrain_key, restrict_cols=True)
+    cj = sites_scale_factor(f_mut, f_h5_pretrain, scale_factor, scale_type, scale_by_expectation)
     print('Tabulating mutations')
     df_mut_tab = mutation_tools.tabulate_sites_in_element(f_sites, f_mut)
     df_model = transfer_element_model(df_mut_tab, df_pretrain, cj, use_chrom=False)

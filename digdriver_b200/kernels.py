@@ -751,7 +751,8 @@ def _check_cds_status(status, what):
     if code:
         why = [m for bit, m in ((1, "a gene has more than 2048 CDS blocks"),
                                 (2, "a gene's chromosome or block lies outside the genome"),
-                                (4, "a gene's blocks are not strictly ascending")) if code & bit]
+                                (4, "a gene's blocks are not strictly ascending"),
+                                (8, "the codon numbering does not fit the CDS lengths")) if code & bit]
         raise _lib.DigError("%s: %s" % (what, "; ".join(why)))
 
 
@@ -787,9 +788,30 @@ def annotate_snvs(genome, gene_chrom, gene_strand, blk_ptr, blk_start, blk_end, 
     dev = genome.device
     gc, gs = _dev(gene_chrom, torch.int32, dev), _dev(gene_strand, torch.int8, dev)
     bp, bs, be = (_dev(x, torch.int64, dev) for x in (blk_ptr, blk_start, blk_end))
-    mc, mp, ma = _dev(mut_chrom, torch.int64, dev), _dev(mut_pos, torch.int64, dev), _dev(mut_alt, torch.uint8, dev)
-    E, n_mut = gc.numel(), mp.numel()
+    mp, ma = _dev(mut_pos, torch.int64, dev), _dev(mut_alt, torch.uint8, dev)
+    E = gc.numel()
     pad = max([int(x) for x in donor] + [int(x) for x in acceptor] + [0])
+    pair_mut, pair_gene = _snv_gene_pairs(dev, gc, bp, bs, be, mut_chrom, mp, pad, stream)
+    if pair_mut.numel() == 0:
+        return pair_mut, pair_gene, torch.zeros(0, dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        cls = torch.empty(pair_mut.numel(), dtype=torch.uint8, device=dev)
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        d, nd, a, na = _splice_offsets(donor, acceptor)
+        _lib.call("dig_annotate_snvs", genome.packed2.data_ptr(), genome.nmask.data_ptr(), genome.n_bases,
+                  genome.chrom_off_d.data_ptr(), genome.chrom_len_d.data_ptr(), len(genome.chrom_len), gc.data_ptr(),
+                  gs.data_ptr(), bp.data_ptr(), bs.data_ptr(), be.data_ptr(), E, d, nd, a, na, mp.data_ptr(),
+                  ma.data_ptr(), pair_mut.data_ptr(), pair_gene.data_ptr(), pair_mut.numel(), cls.data_ptr(),
+                  status.data_ptr(), _stream(dev, stream))
+        _check_cds_status(status, "dig_annotate_snvs")
+    return pair_mut, pair_gene, cls
+
+
+def _snv_gene_pairs(dev, gc, bp, bs, be, mut_chrom, mp, pad, stream):
+    """(mutation, gene) pairs of SNVs against the CDS blocks widened by `pad` bases (dig_overlap_count /
+    dig_overlap_fill), one per pair, sorted by mutation, then gene.  Device tensors (pair_mut int64, pair_gene int32)."""
+    mc = _dev(mut_chrom, torch.int64, dev)
+    E, n_mut = gc.numel(), mp.numel()
     owner = torch.repeat_interleave(torch.arange(E, dtype=torch.int64, device=dev), bp[1:] - bp[:-1])
     kc = gc.to(torch.int64)[owner] << 32
     ks, order = torch.sort(kc | torch.clamp(bs - pad, min=0), stable=True)
@@ -799,8 +821,7 @@ def annotate_snvs(genome, gene_chrom, gene_strand, blk_ptr, blk_start, blk_end, 
     mks = (mc << 32) | mp
     mke = mks + 1
     sptr = _stream(dev, stream)
-    empty = (torch.zeros(0, dtype=torch.int64, device=dev), torch.zeros(0, dtype=torch.int32, device=dev),
-             torch.zeros(0, dtype=torch.uint8, device=dev))
+    empty = (torch.zeros(0, dtype=torch.int64, device=dev), torch.zeros(0, dtype=torch.int32, device=dev))
     if n_mut == 0 or ks.numel() == 0:
         return empty
     with torch.cuda.device(dev):
@@ -820,13 +841,108 @@ def annotate_snvs(genome, gene_chrom, gene_strand, blk_ptr, blk_start, blk_end, 
         key = torch.unique(pm * E + owner[pb])
         pair_mut = torch.div(key, E, rounding_mode="floor")
         pair_gene = (key - pair_mut * E).to(torch.int32)
-        cls = torch.empty(key.numel(), dtype=torch.uint8, device=dev)
-        status = torch.zeros(1, dtype=torch.int32, device=dev)
-        d, nd, a, na = _splice_offsets(donor, acceptor)
-        _lib.call("dig_annotate_snvs", genome.packed2.data_ptr(), genome.nmask.data_ptr(), genome.n_bases,
+    return pair_mut, pair_gene
+
+
+# ---------------------------------------------------------------------------------------------
+# K9c / K10 / K9d: codon-level driver test (csrc/codon.cu)
+# ---------------------------------------------------------------------------------------------
+
+CODON_NO_SITE = 255
+
+
+def codon_ptr(blk_ptr, blk_start, blk_end, device):
+    """int64 [E + 1] device tensor numbering floor(CDS length / 3) codons per gene (the codon_ptr of dig_codon_*)."""
+    bp, bs, be = (_dev(x, torch.int64, device) for x in (blk_ptr, blk_start, blk_end))
+    E = bp.numel() - 1
+    owner = torch.repeat_interleave(torch.arange(E, dtype=torch.int64, device=device), bp[1:] - bp[:-1])
+    T = torch.zeros(E, dtype=torch.int64, device=device).index_add_(0, owner, be - bs + 1)
+    ptr = torch.zeros(E + 1, dtype=torch.int64, device=device)
+    ptr[1:] = torch.cumsum(torch.div(T, 3, rounding_mode="floor"), 0)
+    return ptr
+
+
+def codon_sites(genome, gene_chrom, gene_strand, blk_ptr, blk_start, blk_end, stream=None):
+    """K9c: the 9-slot site record of every complete codon of every gene (dig_codon_sites).  Returns a dict of device
+    tensors: PTR int64 [E+1], POS int64 [n, 3], BIN uint8 [n, 9], CLASS uint8 [n, 9], REF_AA uint8 [n] (ASCII),
+    N_SITES uint8 [n]."""
+    dev = genome.device
+    gc, gs = _dev(gene_chrom, torch.int32, dev), _dev(gene_strand, torch.int8, dev)
+    bp, bs, be = (_dev(x, torch.int64, dev) for x in (blk_ptr, blk_start, blk_end))
+    E = gc.numel()
+    ptr = codon_ptr(bp, bs, be, dev)
+    n = int(ptr[-1].item())
+    out = {"PTR": ptr, "POS": torch.empty((n, 3), dtype=torch.int64, device=dev),
+           "BIN": torch.empty((n, 9), dtype=torch.uint8, device=dev),
+           "CLASS": torch.empty((n, 9), dtype=torch.uint8, device=dev),
+           "REF_AA": torch.empty(n, dtype=torch.uint8, device=dev), "N_SITES": torch.empty(n, dtype=torch.uint8, device=dev)}
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.call("dig_codon_sites", genome.packed2.data_ptr(), genome.nmask.data_ptr(), genome.n_bases,
                   genome.chrom_off_d.data_ptr(), genome.chrom_len_d.data_ptr(), len(genome.chrom_len), gc.data_ptr(),
-                  gs.data_ptr(), bp.data_ptr(), bs.data_ptr(), be.data_ptr(), E, d, nd, a, na, mp.data_ptr(),
-                  ma.data_ptr(), pair_mut.data_ptr(), pair_gene.data_ptr(), key.numel(), cls.data_ptr(),
-                  status.data_ptr(), sptr)
-        _check_cds_status(status, "dig_annotate_snvs")
-    return pair_mut, pair_gene, cls
+                  gs.data_ptr(), bp.data_ptr(), bs.data_ptr(), be.data_ptr(), E, ptr.data_ptr(), n,
+                  out["POS"].data_ptr(), out["BIN"].data_ptr(), out["CLASS"].data_ptr(), out["REF_AA"].data_ptr(),
+                  out["N_SITES"].data_ptr(), status.data_ptr(), _stream(dev, stream))
+        _check_cds_status(status, "dig_codon_sites")
+    return out
+
+
+def codon_transfer(sites, gene_chrom_num, gene_strand, window, win_map_off, win_map, win_counts, y_pred, std, y_true,
+                   flag, d_pr, device, stream=None):
+    """K10 (after dig_window_denominators): MU, SIGMA, R_OBS, FLAG, R_SIZE, PI_NUM, PI_SUM, N_WIN per codon of
+    `sites` (codon_sites output) over the windows of its site-carrying bases.  gene_chrom_num holds chromosome NUMBERS
+    (they index win_map_off).  The device status word is returned as STATUS: 2 = a site-carrying base lies in a window
+    missing from the window map (the reference's KeyError); those codons have NaN MU, so the caller can name them."""
+    dev = torch.device(device)
+    gc, gs = _dev(gene_chrom_num, torch.int32, dev), _dev(gene_strand, torch.int8, dev)
+    wmo, wm = _dev(win_map_off, torch.int64, dev), _dev(win_map, torch.int32, dev)
+    wc = _dev(win_counts, torch.int32, dev).contiguous()
+    yp, sd, yt = (_dev(x, torch.float64, dev).contiguous() for x in (y_pred, std, y_true))
+    fl = _dev(np.asarray(flag).astype(np.uint8) if not isinstance(flag, torch.Tensor) else flag.to(torch.uint8),
+              torch.uint8, dev)
+    dp = _dev(d_pr, torch.float64, dev).contiguous()
+    ptr, pos, bins, ns = sites["PTR"], sites["POS"], sites["BIN"], sites["N_SITES"]
+    n, n_win = ns.numel(), wc.shape[0]
+    f64 = lambda: torch.empty(n, dtype=torch.float64, device=dev)
+    out = {"MU": f64(), "SIGMA": f64(), "R_OBS": f64(), "FLAG": torch.empty(n, dtype=torch.uint8, device=dev),
+           "R_SIZE": torch.empty(n, dtype=torch.int64, device=dev), "PI_NUM": f64(), "PI_SUM": f64(),
+           "N_WIN": torch.empty(n, dtype=torch.int32, device=dev)}
+    den_p = torch.empty(max(n_win, 1), dtype=torch.float64, device=dev)
+    den_m = torch.empty(max(n_win, 1), dtype=torch.float64, device=dev)
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    sptr = _stream(dev, stream)
+    with torch.cuda.device(dev):
+        _lib.call("dig_window_denominators", wc.data_ptr(), dp.data_ptr(), n_win, den_p.data_ptr(), den_m.data_ptr(), sptr)
+        _lib.call("dig_codon_transfer", ptr.data_ptr(), gc.data_ptr(), gs.data_ptr(), gc.numel(), pos.data_ptr(),
+                  bins.data_ptr(), ns.data_ptr(), n, int(window), int(wmo.numel()) - 1, wmo.data_ptr(), wm.data_ptr(),
+                  wc.data_ptr(), yp.data_ptr(), sd.data_ptr(), yt.data_ptr(), fl.data_ptr(), den_p.data_ptr(),
+                  den_m.data_ptr(), dp.data_ptr(), out["MU"].data_ptr(), out["SIGMA"].data_ptr(), out["R_OBS"].data_ptr(),
+                  out["FLAG"].data_ptr(), out["R_SIZE"].data_ptr(), out["PI_NUM"].data_ptr(), out["PI_SUM"].data_ptr(),
+                  out["N_WIN"].data_ptr(), status.data_ptr(), sptr)
+    out["STATUS"] = status
+    return out
+
+
+def snv_codons(genome, gene_chrom, gene_strand, blk_ptr, blk_start, blk_end, sites, mut_chrom, mut_pos, mut_ref,
+               mut_alt, stream=None):
+    """K9d: SNVs (mut_chrom indexes the genome, 0-based mut_pos, mut_ref / mut_alt 0..3 as written) joined against the
+    CDS blocks; per (mutation, gene) pair the codon whose site it is and the slot, -1 / CODON_NO_SITE otherwise.
+    Returns device tensors (pair_mut int64, pair_gene int32, codon int64, slot uint8)."""
+    dev = genome.device
+    gc, gs = _dev(gene_chrom, torch.int32, dev), _dev(gene_strand, torch.int8, dev)
+    bp, bs, be = (_dev(x, torch.int64, dev) for x in (blk_ptr, blk_start, blk_end))
+    mp = _dev(mut_pos, torch.int64, dev)
+    mr, ma = _dev(mut_ref, torch.uint8, dev), _dev(mut_alt, torch.uint8, dev)
+    pair_mut, pair_gene = _snv_gene_pairs(dev, gc, bp, bs, be, mut_chrom, mp, 0, stream)
+    n = pair_mut.numel()
+    codon = torch.empty(n, dtype=torch.int64, device=dev)
+    slot = torch.empty(n, dtype=torch.uint8, device=dev)
+    if n:
+        status = torch.zeros(1, dtype=torch.int32, device=dev)
+        with torch.cuda.device(dev):
+            _lib.call("dig_snv_codons", gs.data_ptr(), bp.data_ptr(), bs.data_ptr(), be.data_ptr(),
+                      sites["PTR"].data_ptr(), gc.numel(), sites["POS"].data_ptr(), sites["BIN"].data_ptr(),
+                      mp.data_ptr(), mr.data_ptr(), ma.data_ptr(), pair_mut.data_ptr(), pair_gene.data_ptr(), n,
+                      codon.data_ptr(), slot.data_ptr(), status.data_ptr(), _stream(dev, stream))
+            _check_cds_status(status, "dig_snv_codons")
+    return pair_mut, pair_gene, codon, slot

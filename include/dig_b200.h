@@ -517,6 +517,7 @@ int dig_element_psum(const double *L_d, const int64_t *region_counts_d, const do
 #define DIG_CDS_ERR_BLOCKS 1        /* a gene has more than DIG_CDS_MAX_BLOCKS blocks */
 #define DIG_CDS_ERR_RANGE 2         /* chromosome index or block outside the genome */
 #define DIG_CDS_ERR_ORDER 4         /* blocks not strictly ascending / empty */
+#define DIG_CDS_ERR_CODONS 8        /* codon_ptr does not number floor(CDS length / 3) codons per gene */
 #define DIG_CDS_MAX_BLOCKS 2048
 #define DIG_CDS_MAX_SPLICE_OFFSETS 8
 int dig_cds_substitution_table(const uint32_t *packed2_d, const uint32_t *nmask_d, int64_t n_bases,
@@ -533,6 +534,48 @@ int dig_annotate_snvs(const uint32_t *packed2_d, const uint32_t *nmask_d, int64_
                       const int64_t *mut_pos_d, const uint8_t *mut_alt_d, const int64_t *pair_mut_d,
                       const int32_t *pair_gene_d, int64_t n_pair, uint8_t *class_out_d, int32_t *status_d,
                       void *stream);
+
+/* ---------------------------------------------------------------------------------
+ * K9c / K10 / K9d  codon-level driver test (csrc/codon.cu states the codon rules in full; DESIGN.md section 5): every
+ * codon is a site set of the sites model, without a 192-column L row per codon.  Genes as for K9.
+ * codon_ptr_d int64 [n_gene + 1]: gene e owns codons [codon_ptr[e], codon_ptr[e+1]), floor(CDS length / 3) of them
+ *   (codon k of the gene = transcript bases 3k .. 3k+2, 0-based); n_codon = codon_ptr[n_gene].
+ *
+ * dig_codon_sites: per codon i, codon_pos_d int64 [n_codon, 3] = genomic positions of its transcript bases 0, 1, 2;
+ *   codon_bin_d / codon_class_d uint8 [n_codon, 9]: slot s = 3 j + rank(transcript ALT among the non-REF bases of base
+ *   j) holds the bin (3 ctx + rank, as K9a) and class (DIG_CDS_MISSENSE / DIG_CDS_NONSENSE) of that SNV when it is a
+ *   site, 255 / 255 when not; codon_ref_aa_d uint8 [n_codon] = reference amino acid (ASCII, '*' = stop; 0 for a codon
+ *   with an N); codon_n_sites_d uint8 [n_codon] = number of sites (0 = not tested).  status_d is OR-ed with
+ *   DIG_CDS_ERR_* (DIG_CDS_ERR_CODONS when codon_ptr does not fit the CDS lengths).
+ * dig_codon_transfer: per codon with sites, the K6 region parameters over the windows floor(p / window) of its bases
+ *   that carry a site: mu_d, sigma_d, r_obs_d, flag_out_d, r_size_d (sum of the 64 window counts), pi_num_d (may be
+ *   NULL) = sum over sites of d_pr[bin], pi_sum_d = pi_num / sum_w denom[w] with denom_plus_d / denom_minus_d of
+ *   dig_window_denominators (by gene strand), n_win_d (may be NULL).  gene_chrom_d indexes win_map_off_d (chromosome
+ *   number, as dig_element_transfer's elt_chrom); win_counts_d int32 [n_win, 64], 16-byte aligned.  Codons without
+ *   sites get zeros.  A missing window sets status 2 (the reference's KeyError) and NaN mu / sigma / pi_sum.
+ * dig_snv_codons: per (mutation, gene) pair of the interval join against the CDS blocks (as dig_annotate_snvs),
+ *   codon_out_d int64 = the codon whose site the SNV is (position, REF and ALT; mut_ref_d / mut_alt_d uint8 0..3 as
+ *   written), slot_out_d uint8 = its slot; -1 / 255 when it is no site of that gene.
+ */
+int dig_codon_sites(const uint32_t *packed2_d, const uint32_t *nmask_d, int64_t n_bases, const int64_t *chrom_off_d,
+                    const int64_t *chrom_len_d, int n_chrom, const int32_t *gene_chrom_d, const int8_t *gene_strand_d,
+                    const int64_t *blk_ptr_d, const int64_t *blk_start_d, const int64_t *blk_end_d, int64_t n_gene,
+                    const int64_t *codon_ptr_d, int64_t n_codon, int64_t *codon_pos_d, uint8_t *codon_bin_d,
+                    uint8_t *codon_class_d, uint8_t *codon_ref_aa_d, uint8_t *codon_n_sites_d, int32_t *status_d,
+                    void *stream);
+int dig_codon_transfer(const int64_t *codon_ptr_d, const int32_t *gene_chrom_d, const int8_t *gene_strand_d,
+                       int64_t n_gene, const int64_t *codon_pos_d, const uint8_t *codon_bin_d,
+                       const uint8_t *codon_n_sites_d, int64_t n_codon, int64_t window, int n_chrom,
+                       const int64_t *win_map_off_d, const int32_t *win_map_d, const int32_t *win_counts_d,
+                       const double *y_pred_d, const double *std_d, const double *y_true_d, const uint8_t *flag_d,
+                       const double *denom_plus_d, const double *denom_minus_d, const double *d_pr_d, double *mu_d,
+                       double *sigma_d, double *r_obs_d, uint8_t *flag_out_d, int64_t *r_size_d, double *pi_num_d,
+                       double *pi_sum_d, int32_t *n_win_d, int32_t *status_d, void *stream);
+int dig_snv_codons(const int8_t *gene_strand_d, const int64_t *blk_ptr_d, const int64_t *blk_start_d,
+                   const int64_t *blk_end_d, const int64_t *codon_ptr_d, int64_t n_gene, const int64_t *codon_pos_d,
+                   const uint8_t *codon_bin_d, const int64_t *mut_pos_d, const uint8_t *mut_ref_d,
+                   const uint8_t *mut_alt_d, const int64_t *pair_mut_d, const int32_t *pair_gene_d, int64_t n_pair,
+                   int64_t *codon_out_d, uint8_t *slot_out_d, int32_t *status_d, void *stream);
 
 /* ---------------------------------------------------------------------------------
  * Synthetic genome generator (BASELINE.json configs are synthetic): position g is a pure

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """CLI shim with the sub-commands of the reference's scripts/DigDriver.py: geneDriver, elementDriver
-(--f-bed / --f-sites) and quickDriver.  Results are written to <outdir>/<outpfx>.results.txt as TSV with
+(--f-bed / --f-sites) and quickDriver; and codonDriver, the codon-level test of a gene set.  Results are written to <outdir>/<outpfx>.results.txt as TSV with
 header and index, like the reference (DigDriver.py:41-43, :115-118)."""
 import argparse
 import os
@@ -84,6 +84,17 @@ def onthefly(args):
     _save(_int_counts(df_dig), args)
 
 
+def codon_driver(args):
+    """Every codon of the genic store's genes as a site set of its Missense / Nonsense SNVs (codon_tools.py)."""
+    from digdriver_b200.driver_model import codon_tools
+    print('Running codon driver detection')
+    os.makedirs(args.outdir, exist_ok=True)
+    df_dig = codon_tools.run_codon_model(args.fmut, args.f_genic, args.model, args.f_fasta,
+                                         scale_factor=args.scale_factor_manual,
+                                         scale_by_expectation=not args.scale_factor_manual, min_obs=args.min_obs)
+    _save(df_dig, args)
+
+
 def _common_out(p):
     p.add_argument('--outpfx', type=str, required=True)
     p.add_argument('--outdir', type=str, required=True)
@@ -141,6 +152,16 @@ def parse_args(text=None):
     _common_out(d)
     _element_opts(d)
     d.set_defaults(func=onthefly)
+    e = sub.add_parser('codonDriver', help='test every codon of a gene set (its missense / nonsense SNVs)')
+    e.add_argument('fmut', type=str, help='annotated mutation file (annotateMutations + addMutationContext)')
+    e.add_argument('model', type=str, help='pretrained model with region_params, sequence_model_192, genic_model')
+    e.add_argument('f_genic', type=str, help='genic store of buildGenicData')
+    e.add_argument('f_fasta', type=str)
+    e.add_argument('--outpfx', type=str, required=True)
+    e.add_argument('--outdir', type=str, required=True)
+    e.add_argument('--scale-factor-manual', default=None, type=float)
+    e.add_argument('--min-obs', default=1, type=int, help='write codons with at least this many observed SNVs')
+    e.set_defaults(func=codon_driver)
     return parser.parse_args(text.split()) if text else parser.parse_args()
 
 

@@ -2,7 +2,8 @@
 """CLI shim with the sub-commands and arguments of the reference's scripts/DigPreprocess.py that lie on the
 hot path: countGenomeContext (the genome scan), addMutationContext, preprocess_element_model,
 initialize_f_data; and two of its own that build the gene annotation the reference takes from outside:
-buildGenicData (the genic store from a BED12 gene set) and annotateMutations (GENE / ANNOT of raw calls).  Output files are directory stores (or HDF5 when h5py + PyTables exist), see
+buildGenicData (the genic store from a BED12 gene set), annotateMutations (GENE / ANNOT of raw calls) and codonSites
+(every codon of a gene set as a sites file).  Output files are directory stores (or HDF5 when h5py + PyTables exist), see
 digdriver_b200/storage.py."""
 import argparse
 import os
@@ -197,6 +198,17 @@ def annotateMutations(args):
     df_out.to_csv(args.fout, sep="\t", index=False, header=False)
 
 
+def codonSites(args):
+    """Every codon of the genic store's genes as a sites file (11 columns, ELT = GENE:CODON) for the --f-sites flow."""
+    from digdriver_b200.driver_model import codon_tools
+    genes = None
+    if args.genes:
+        genes = [x.strip() for x in open(args.genes) if x.strip()]
+    df = codon_tools.codon_table(args.f_genic, args.fasta, genes=genes)
+    codon_tools.write_sites(df, args.fout)
+    print('Wrote {} sites of {} codons to {}'.format(len(df), df.ELT.nunique(), args.fout))
+
+
 def parse_args(text=None):
     parser = argparse.ArgumentParser(description='Preprocess genome and mutation files for use with Dig (B200).')
     sub = parser.add_subparsers()
@@ -270,6 +282,12 @@ def parse_args(text=None):
     m.add_argument('fasta')
     m.add_argument('fout', help='8-column output: the input of addMutationContext')
     m.set_defaults(func=annotateMutations)
+    s = sub.add_parser('codonSites', help='write every codon of a genic store as a site set (its missense / nonsense SNVs)')
+    s.add_argument('f_genic', help='genic store of buildGenicData')
+    s.add_argument('fasta')
+    s.add_argument('fout', help='11-column sites file: CHROM START END REF ALT ELT GENE ANNOT MUT_TYPE CONTEXT STRAND')
+    s.add_argument('--genes', default='', help='file with one gene name per line: only these genes')
+    s.set_defaults(func=codonSites)
     return parser.parse_args(text.split()) if text else parser.parse_args()
 
 
