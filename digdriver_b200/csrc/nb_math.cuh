@@ -65,7 +65,10 @@ __device__ inline double log_dbinom_raw(double x, double n, double p, double q)
     }
     if (x == n) return q < 0.1 ? -bd0(n, n * p) - n * q : n * log(p);
     const double lc = stirlerr(n) - stirlerr(x) - stirlerr(n - x) - bd0(x, n * p) - bd0(n - x, n * q);
-    const double lf = LN_2PI + log(x) + log1p(-x / n);
+    // log(1 - x/n): once x/n is near 1 (k << alpha in the NB density) the rounding of x/n is all that is left of
+    // 1 - x/n, so take it as (n - x)/n, where n - x is exact
+    const double r = x / n;
+    const double lf = LN_2PI + log(x) + (r < 0.5 ? log1p(-r) : log((n - x) / n));
     return lc - 0.5 * lf;
 }
 
@@ -85,12 +88,16 @@ __device__ inline double log_nb_density(double k, double a, double p, double q)
 // needs NO division (Lentz spends six per iteration, each a chain of ~30 dependent FP64 instructions; the gene-test kernel
 // is bound by the latency of exactly that chain).  Same truncation rule as before: stop when two successive convergents
 // agree to 1e-15 (|A_n B_{n-1} - A_{n-1} B_n| <= eps |A_{n-1} B_n|, the `del` of Lentz), checked after each odd step.
-__device__ inline double beta_cf(double a, double b, double x)
+// y is 1 - x as the caller holds it (the NB's p and q = 1 - p), so it carries no cancellation of its own.
+__device__ inline double beta_cf(double a, double b, double x, double y)
 {
     const double EPS = 1e-15, BIG = 0x1p+200, SMALL = 0x1p-200;    // growth per iteration < 2^110 (a + 2m up to ~2^27 squared, twice): products stay finite
     const double qab = a + b, qap = a + 1.0, qam = a - 1.0;
-    // convergents after the leading term d_1 = -qab x / qap:  (R, S) = A_1, B_1 and (P, Q) = A_2, B_2, both times qap
-    double R = qap, S = qap, P = qap, Q = qap - qab * x;
+    // convergents after the leading term d_1 = -qab x / qap:  (R, S) = A_1, B_1 and (P, Q) = A_2, B_2, both times qap.
+    // Q = (a+1) - (a+b) x cancels near the side switch; as a y + 1 - b x with the larger product exact inside the
+    // outer fma it keeps its digits (qap - qab * x lost ~1e-5 relative at alpha = 1e12)
+    const double ay = a * y, bx = b * x;
+    double R = qap, S = qap, P = qap, Q = ay >= bx ? fma(a, y, fma(-b, x, 1.0)) : fma(-b, x, fma(a, y, 1.0));
     for (int m = 1; m < 2000000; ++m) {
         const double dm = (double)m, m2 = 2.0 * dm;
         // even step: d = m (b - m) x / ((a + 2m - 1)(a + 2m))
@@ -120,6 +127,28 @@ __device__ inline double beta_cf(double a, double b, double x)
     return P / Q;
 }
 
+// P(X <= kk) / pmf(kk), the p side of the switch: q (kk+alpha)/alpha CF(alpha, kk+1, p).  While m << alpha every odd
+// step of that fraction has 1 + d ~ q + (m - kk)/alpha, so the recurrence cancels about log10(1/q) digits per step when
+// p is near 1 (3.5e-8 relative lost at alpha = 3e8, q = 3e-8; 1e-5 at alpha = 1e12, q = 3e-11).  For integer kk with
+// q < 1e-4 (the site and codon regime) or kk < 1e-10 alpha, the finite sum is taken downward from kk instead: on this
+// side of the switch its ratios j / ((j-1+alpha) q) stay below 1 and shrink, so it stops as soon as the geometric bound
+// on the rest is below 1e-17 of the sum.  The sum has at most kk terms, so it is taken only for kk < 2e6 (beta_cf's own
+// iteration cap); a larger kk keeps the fraction, and no thread loops on a j that j -= 1 cannot move.
+__device__ inline double nb_lower_over_pmf(double kk, double alpha, double p, double q)
+{
+    if ((q < 1e-4 || kk < 1e-10 * alpha) && kk < 2e6 && kk == floor(kk)) {
+        double t = 1.0, s = 1.0;
+        for (double j = kk; j > 0.0; j -= 1.0) {
+            const double r = j / ((j - 1.0 + alpha) * q);
+            t *= r;
+            s += t;
+            if (r < 1.0 && t * r < 1e-17 * s * (1.0 - r)) break;
+        }
+        return s;
+    }
+    return q * (kk + alpha) / alpha * beta_cf(alpha, kk + 1.0, p, q);
+}
+
 __device__ inline double nb_midp(double k, double alpha, double p)
 {
     const double nan = __longlong_as_double(0x7ff8000000000000LL);
@@ -135,11 +164,10 @@ __device__ inline double nb_midp(double k, double alpha, double p)
     const double a = k + 1.0;
     double sf;
     if (q < (a + 1.0) / (a + alpha + 2.0)) {
-        const double cf = beta_cf(a, alpha, q);
+        const double cf = beta_cf(a, alpha, q, p);
         sf = exp(lg + log(q * (k + alpha) / a * cf));
     } else {
-        const double cf = beta_cf(alpha, a, p);
-        sf = 1.0 - exp(lg + log(q * (k + alpha) / alpha * cf));
+        sf = 1.0 - exp(lg + log(nb_lower_over_pmf(k, alpha, p, q)));
     }
     return (isint ? 0.5 * exp(lg) : 0.0) + sf;
 }
@@ -151,36 +179,16 @@ __device__ inline double nb_tail_upper_from(double kk, double alpha, double p, d
 {
     const double lg = log_nb_density(kk, alpha, p, q);
     const double a = kk + 1.0;
-    if (q < (a + 1.0) / (a + alpha + 2.0)) return exp(lg + log(q * (kk + alpha) / a * beta_cf(a, alpha, q)));
-    return 1.0 - exp(lg + log(q * (kk + alpha) / alpha * beta_cf(alpha, a, p)));
+    if (q < (a + 1.0) / (a + alpha + 2.0)) return exp(lg + log(q * (kk + alpha) / a * beta_cf(a, alpha, q, p)));
+    return 1.0 - exp(lg + log(nb_lower_over_pmf(kk, alpha, p, q)));
 }
 
 __device__ inline double nb_tail_lower_to(double kk, double alpha, double p, double q)       // P(X <= kk) = I_p(alpha, kk+1)
 {
     const double lg = log_nb_density(kk, alpha, p, q);
     const double a = kk + 1.0;
-    if (q < (a + 1.0) / (a + alpha + 2.0)) return 1.0 - exp(lg + log(q * (kk + alpha) / a * beta_cf(a, alpha, q)));
-    return exp(lg + log(q * (kk + alpha) / alpha * beta_cf(alpha, a, p)));
-}
-
-__device__ inline double nb_exact(double k, double alpha, double p)
-{
-    const double nan = __longlong_as_double(0x7ff8000000000000LL);
-    if (isnan(k) || isnan(alpha) || isnan(p)) return nan;
-    if (!(alpha > 0.0) || isinf(alpha) || k < 0.0 || isinf(k) || p < 0.0 || p > 1.0) return nan;
-    const double q = 1.0 - p;
-    const double mean = alpha * q / p;                       // +inf when p == 0
-    if (k < mean) {
-        if (p <= 0.0) return 0.0;                            // betainc(alpha, k+1, 0)
-        if (k == 0.0) return exp(alpha * log(p));            // I_p(alpha, 1) = p^alpha
-        return nb_tail_lower_to(k, alpha, p, q);
-    }
-    // only reached with q < 1
-    if (k == 0.0) return 1.0;                                // betainc(0, alpha, q) = 1 (q > 0), else pmf(0; p = 1) = 1
-    if (q <= 0.0) return 0.0;                                // betainc(k, alpha, 0) = 0 and pmf(k > 0; p = 1) = 0
-    const double up = nb_tail_upper_from(k - 1.0, alpha, p, q);
-    if (up == 0.0) return exp(log_nb_density(k, alpha, p, q));
-    return up;
+    if (q < (a + 1.0) / (a + alpha + 2.0)) return 1.0 - exp(lg + log(q * (kk + alpha) / a * beta_cf(a, alpha, q, p)));
+    return exp(lg + log(nb_lower_over_pmf(kk, alpha, p, q)));
 }
 
 // General regularized incomplete beta I_x(a, b) (lgamma prefactor + the same continued fraction); only used by
@@ -190,8 +198,9 @@ __device__ inline double ibeta_general(double a, double b, double x)
     if (x <= 0.0) return 0.0;
     if (x >= 1.0) return 1.0;
     const double lf = lgamma(a + b) - lgamma(a) - lgamma(b) + a * log(x) + b * log1p(-x);
-    if (x < (a + 1.0) / (a + b + 2.0)) return exp(lf + log(beta_cf(a, b, x) / a));
-    return 1.0 - exp(lf + log(beta_cf(b, a, 1.0 - x) / b));
+    const double y = 1.0 - x;
+    if (x < (a + 1.0) / (a + b + 2.0)) return exp(lf + log(beta_cf(a, b, x, y) / a));
+    return 1.0 - exp(lf + log(beta_cf(b, a, y, x) / b));
 }
 
 // The other tail conventions of nb_model.py, selected by `mode` (include/dig_b200.h DIG_NB_*):
@@ -217,6 +226,26 @@ __device__ inline double nb_lower_excl(double k, double alpha, double p, double 
     if (p <= 0.0) return 0.0;
     if (k < 1.0) return ibeta_general(alpha, k, p);
     return nb_tail_lower_to(k - 1.0, alpha, p, q);
+}
+
+__device__ inline double nb_exact(double k, double alpha, double p)
+{
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    if (isnan(k) || isnan(alpha) || isnan(p)) return nan;
+    if (!(alpha > 0.0) || isinf(alpha) || k < 0.0 || isinf(k) || p < 0.0 || p > 1.0) return nan;
+    const double q = 1.0 - p;
+    const double mean = alpha * q / p;                       // +inf when p == 0
+    if (k < mean) {
+        if (p <= 0.0) return 0.0;                            // betainc(alpha, k+1, 0)
+        if (k == 0.0) return exp(alpha * log(p));            // I_p(alpha, 1) = p^alpha
+        return nb_tail_lower_to(k, alpha, p, q);
+    }
+    // only reached with q < 1
+    if (k == 0.0) return 1.0;                                // betainc(0, alpha, q) = 1 (q > 0), else pmf(0; p = 1) = 1
+    if (q <= 0.0) return 0.0;                                // betainc(k, alpha, 0) = 0 and pmf(k > 0; p = 1) = 0
+    const double up = nb_upper_incl(k, alpha, p, q);          // ibeta_general for a non-integer 0 < k < 1
+    if (up == 0.0) return exp(log_nb_density(k, alpha, p, q));
+    return up;
 }
 
 __device__ inline double nb_pmf(double k, double alpha, double p, double q)          // scipy.stats.nbinom.pmf

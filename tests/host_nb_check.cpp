@@ -10,6 +10,7 @@
 #define __device__
 using std::isinf;
 using std::isnan;
+using std::fma;
 static inline double __longlong_as_double(long long v)
 {
     double d;
@@ -59,5 +60,10 @@ void hc_llr(int model, const double *alpha, const double *theta, const double *p
 void hc_fisher2(const double *a, const double *b, int64_t n, double *out)
 {
     for (int64_t i = 0; i < n; ++i) out[i] = dig_nb::fisher2(a[i], b[i]);
+}
+
+void hc_chi2_sf(int df, const double *x, int64_t n, double *out)
+{
+    for (int64_t i = 0; i < n; ++i) out[i] = dig_nb::chi2_sf(x[i], df);
 }
 }
