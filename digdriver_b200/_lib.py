@@ -87,7 +87,7 @@ class ScanOpts(ctypes.Structure):
                 ("nsum_offset_words", _c.c_int32), ("peer_counts3_d", _c.c_void_p * 8), ("mc_counts3_d", _c.c_void_p)]
 
 
-SCAN_AUTO, SCAN_PER_BASE, SCAN_HEX_PLAIN, SCAN_HEX = 0, 1, 2, 3
+SCAN_AUTO, SCAN_PER_BASE, SCAN_HEX = 0, 1, 3
 
 _lib = None
 

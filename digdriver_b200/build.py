@@ -60,10 +60,7 @@ def build_library(force=False, verbose=False, extra_flags=(), out_path=None):
 
 
 if __name__ == "__main__":
-    if "--variant" in sys.argv:        # python -m digdriver_b200.build --variant NAME -DFLAG ...  (developer A/B builds)
-        i = sys.argv.index("--variant")
-        print(build_library(extra_flags=sys.argv[i + 2:], out_path=os.path.join(PKG_DIR, "libdigb200_%s.so" % sys.argv[i + 1])))
-    elif "--timing" in sys.argv:
+    if "--timing" in sys.argv:
         print(build_library(extra_flags=["-DDIG_LB_TIMING"], out_path=os.path.join(PKG_DIR, "libdigb200_timing.so")))
     else:
         print(build_library(force="--force" in sys.argv, verbose="-v" in sys.argv))

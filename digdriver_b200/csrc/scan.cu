@@ -278,177 +278,6 @@ __global__ void __launch_bounds__(THREADS, PRIVATE ? 3 : 3) scan_sym_kernel(
 }
 
 // ---------------------------------------------------------------------------------------
-// fused kernel: pentanucleotide AND trinucleotide tables of the same regions in one pass.
-//
-// The K=1024 scan runs at the shared-memory data-pipe limit, so a second scan for the trinucleotide
-// table (the one the element / gene stage needs) would cost another pass.  Instead the trinucleotide
-// row is the marginal of the pentanucleotide row over the two outer bases -- each lane already holds
-// exactly the 8 int4 chunks that sum to its two trinucleotide bins -- plus the few centres whose
-// 3-mer is valid while their 5-mer is not (an N exactly two bases away, the second base of a
-// chromosome, the last-but-one base): those are counted into a 64-bin correction histogram through
-// the cooperative path.
-// ---------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(THREADS, 3) scan_fused53_kernel(
-    const uint2 *__restrict__ p2v, const uint32_t *__restrict__ p2, const uint32_t *__restrict__ nmask,
-    int64_t n_words32, const int64_t *__restrict__ chrom_off, const int64_t *__restrict__ chrom_len,
-    const int32_t *__restrict__ reg_chrom, const int64_t *__restrict__ reg_start,
-    const int64_t *__restrict__ reg_end, int64_t n_reg, int32_t *__restrict__ counts5,
-    int32_t *__restrict__ counts3, unsigned long long *__restrict__ totals5,
-    unsigned long long *__restrict__ totals3, unsigned int tot_limit_kb)
-{
-    constexpr int K = 1024, K4 = 256, K3 = 64;
-    constexpr uint32_t HIST_BYTES = 4096u;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    __shared__ unsigned int cta_acc_kb;
-    __shared__ int tot3_s[K3];
-    __shared__ int corr_s[WARPS_PER_BLOCK][K3];
-
-    const int lane = threadIdx.x & 31;
-    const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
-    const uint32_t smem0 = (uint32_t)__cvta_generic_to_shared(smem_raw);
-    const uint32_t hist0 = (smem0 + K * 4u + HIST_BYTES - 1u) & ~(HIST_BYTES - 1u);
-    const uint32_t hist = hist0 + (uint32_t)warp * HIST_BYTES;
-    int *hist_p = reinterpret_cast<int *>(smem_raw + (hist - smem0));
-    int *tot_p = reinterpret_cast<int *>(smem_raw);
-    int *corr = corr_s[warp];
-    const uint32_t corr_addr = (uint32_t)__cvta_generic_to_shared(corr);
-
-    for (int k = threadIdx.x; k < K; k += THREADS) tot_p[k] = 0;
-    if (threadIdx.x < K3) tot3_s[threadIdx.x] = 0;
-    if (threadIdx.x == 0) cta_acc_kb = 0u;
-    for (uint32_t k = lane; k < HIST_BYTES / 4u; k += 32) hist_p[k] = 0;
-    corr[lane] = 0;
-    corr[lane + 32] = 0;
-    __syncthreads();
-
-    const int64_t gwarp = (int64_t)blockIdx.x * WARPS_PER_BLOCK + warp;
-    const int64_t nwarps = (int64_t)gridDim.x * WARPS_PER_BLOCK;
-
-    for (int64_t r = gwarp; r < n_reg; r += nwarps) {
-        const RegionSpan s5 = region_span(chrom_off, chrom_len, reg_chrom, reg_start, reg_end, r, 2, 2, 2, 2);
-        const RegionSpan s3 = region_span(chrom_off, chrom_len, reg_chrom, reg_start, reg_end, r, 1, 1, 1, 1);
-        if (s3.ge > s3.gs) {                                   // the 3-mer range contains the 5-mer range
-            const int64_t w0 = s3.gs >> 5;
-            const int nw = (int)(((s3.ge - 1) >> 5) - w0) + 1;
-            const int lo3 = (int)(s3.gs - (w0 << 5)), hi3 = (int)(s3.ge - (w0 << 5));
-            const int lo5 = (int)(s5.gs - (w0 << 5)), hi5 = (int)(s5.ge - (w0 << 5));
-            const uint2 *pv = p2v + w0;
-            const uint32_t *pn = nmask + w0;
-            const int64_t left = n_words32 - w0;
-            const int avail = left > 0x7fffffff ? 0x7fffffff : (int)left;
-            uint32_t carry_p = 0u, carry_n = 0xFFFFFFFFu;
-            if (w0 > 0) {
-                carry_p = __ldg(p2 + 2 * w0 - 1);
-                carry_n = __ldg(nmask + w0 - 1);
-            }
-            WordLoad nxt = load_word(pv, pn, lane, avail);
-            WordLoad nx2 = load_word(pv, pn, lane + 32, avail);
-            for (int rel0 = 0; rel0 < nw; rel0 += 32) {
-                const int rel = rel0 + lane;
-                const WordLoad cur = nxt;
-                nxt = nx2;
-                nx2 = load_word(pv, pn, rel + 64, avail);
-                const uint2 pw = cur.pw;
-                const uint32_t nm = cur.nm;
-                uint32_t prev_p = __shfl_up_sync(0xffffffffu, pw.y, 1);
-                uint32_t next_p = __shfl_down_sync(0xffffffffu, pw.x, 1);
-                uint32_t prev_n = __shfl_up_sync(0xffffffffu, nm, 1);
-                uint32_t next_n = __shfl_down_sync(0xffffffffu, nm, 1);
-                const uint32_t n0_p = __shfl_sync(0xffffffffu, nxt.pw.x, 0);
-                const uint32_t n0_n = __shfl_sync(0xffffffffu, nxt.nm, 0);
-                if (lane == 0) {
-                    prev_p = carry_p;
-                    prev_n = carry_n;
-                }
-                if (lane == 31) {
-                    next_p = n0_p;
-                    next_n = n0_n;
-                }
-                carry_p = __shfl_sync(0xffffffffu, pw.y, 31);
-                carry_n = __shfl_sync(0xffffffffu, nm, 31);
-                const int pos0 = rel << 5;                     // position of this word's first base, from w0
-                const uint32_t bad3 = nm | (nm << 1) | (next_n >> 31) | (nm >> 1) | (prev_n << 31);
-                const uint32_t bad5 = bad3 | (nm << 2) | (next_n >> 30) | (nm >> 2) | (prev_n << 30);
-                const uint32_t valid5 = range_mask(lo5 - pos0, hi5 - pos0) & ~bad5;
-                const uint32_t extra3 = range_mask(lo3 - pos0, hi3 - pos0) & ~bad3 & ~valid5;
-
-                const bool full = valid5 == 0xFFFFFFFFu;
-                if (full) Unroll<2, 2, 0, 2>::run(hist, prev_p, pw.x, pw.y, next_p);
-                uint32_t pm = __ballot_sync(0xffffffffu, (!full && valid5 != 0u) || extra3 != 0u);
-                while (pm) {
-                    const int j = __ffs(pm) - 1;
-                    pm &= pm - 1;
-                    const uint32_t a = __shfl_sync(0xffffffffu, prev_p, j);
-                    const uint32_t b0 = __shfl_sync(0xffffffffu, pw.x, j);
-                    const uint32_t b1 = __shfl_sync(0xffffffffu, pw.y, j);
-                    const uint32_t c = __shfl_sync(0xffffffffu, next_p, j);
-                    uint32_t v5 = __shfl_sync(0xffffffffu, valid5, j);
-                    const uint32_t v3 = __shfl_sync(0xffffffffu, extra3, j);
-                    if (v5 == 0xFFFFFFFFu) v5 = 0u;            // that lane already ran the unrolled path
-                    const uint32_t bit = 0x80000000u >> lane;
-                    if (v5 & bit) smem_inc((runtime_key<2, 2>(a, b0, b1, c, lane) << 2) | hist);
-                    if (v3 & bit) smem_inc(corr_addr + (runtime_key<1, 1>(a, b0, b1, c, lane) << 2));
-                }
-            }
-        }
-        __syncwarp();
-        bool tot_smem = totals5 != nullptr, tot_glob = false;
-        if (totals5 != nullptr) {
-            const unsigned int kb = (unsigned int)((s3.ge - s3.gs) >> 10) + 1u;
-            unsigned int old = 0u;
-            if (lane == 0) old = atomicAdd(&cta_acc_kb, kb);
-            old = __shfl_sync(0xffffffffu, old, 0);
-            if (old + kb > tot_limit_kb || old + kb < old) {
-                tot_smem = false;
-                tot_glob = true;
-            }
-        }
-        int4 *hist4 = reinterpret_cast<int4 *>(hist_p);
-        int4 *out4 = reinterpret_cast<int4 *>(counts5 + r * (int64_t)K);
-        int tri[2] = {0, 0};                                   // trinucleotide bins lane and lane + 32
-#pragma unroll
-        for (int j = 0; j < K4 / 32; ++j) {
-            const int cidx = j * 32 + lane;                    // = x0 * 64 + (x1 x2 x3); chunk = the 4 values of x4
-            const int4 v = hist4[cidx];
-            hist4[cidx] = make_int4(0, 0, 0, 0);
-            __stcs(out4 + cidx, v);
-            tri[j & 1] += (v.x + v.y) + (v.z + v.w);
-            if (tot_smem) {
-                atomicAdd(tot_p + 0 * K4 + cidx, v.x);
-                atomicAdd(tot_p + 1 * K4 + cidx, v.y);
-                atomicAdd(tot_p + 2 * K4 + cidx, v.z);
-                atomicAdd(tot_p + 3 * K4 + cidx, v.w);
-            }
-            if (tot_glob) {
-                if (v.x) atomicAdd(totals5 + 4 * cidx + 0, (unsigned long long)v.x);
-                if (v.y) atomicAdd(totals5 + 4 * cidx + 1, (unsigned long long)v.y);
-                if (v.z) atomicAdd(totals5 + 4 * cidx + 2, (unsigned long long)v.z);
-                if (v.w) atomicAdd(totals5 + 4 * cidx + 3, (unsigned long long)v.w);
-            }
-        }
-        int32_t *out3 = counts3 + r * (int64_t)K3;
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-            const int m = h * 32 + lane;
-            const int v = tri[h] + corr[m];
-            corr[m] = 0;
-            __stcs(out3 + m, v);
-            if (tot_smem && v) atomicAdd(tot3_s + m, v);
-            if (tot_glob && v) atomicAdd(totals3 + m, (unsigned long long)v);
-        }
-        __syncwarp();
-    }
-
-    if (totals5 == nullptr) return;
-    __syncthreads();
-    for (int k = threadIdx.x; k < K; k += THREADS) {
-        const int v = tot_p[k];
-        if (v) atomicAdd(totals5 + ((k % K4) * 4 + k / K4), (unsigned long long)v);
-    }
-    if (threadIdx.x < K3 && tot3_s[threadIdx.x]) atomicAdd(totals3 + threadIdx.x, (unsigned long long)tot3_s[threadIdx.x]);
-}
-
-// ---------------------------------------------------------------------------------------
 // generic kernel: any (n_up, n_down) with K <= 4096, any strand.  One lane per centre.
 // ---------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(THREADS) scan_generic_kernel(
@@ -563,31 +392,18 @@ extern "C" int dig_count_contexts_fused53(const uint32_t *packed2_d, const uint3
     DIG_CHECK_ARG((totals5_d == nullptr) == (totals3_d == nullptr), "pass both totals or neither");
     DIG_CHECK_ARG((reinterpret_cast<uintptr_t>(packed2_d) & 7u) == 0 && (reinterpret_cast<uintptr_t>(counts5_d) & 15u) == 0,
                   "packed2_d must be 8-byte and counts5_d 16-byte aligned");
-    DIG_CHECK_ARG(so.variant >= DIG_SCAN_AUTO && so.variant <= DIG_SCAN_HEX, "unknown scan variant");
+    DIG_CHECK_ARG(so.variant == DIG_SCAN_AUTO || so.variant == DIG_SCAN_HEX, "unknown scan variant (AUTO or HEX)");
+    const uint32_t *nsum = so.nsum_off > 0 ? nmask_d + so.nsum_off : nullptr;
     if (so.variant == DIG_SCAN_AUTO &&
-        scan_lb_usable(packed2_d, nmask_d, n_bases, counts5_d, so.workspace, so.workspace_bytes, n_reg))
-        return launch_scan_lb(packed2_d, nmask_d, so.nsum_off > 0 ? nmask_d + so.nsum_off : nullptr, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
+        scan_lb_usable(packed2_d, nmask_d, nsum, n_bases, counts5_d, so.workspace, so.workspace_bytes, n_reg))
+        return launch_scan_lb(packed2_d, nmask_d, nsum, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
                               n_reg, counts5_d, counts3_d, totals5_d, totals3_d, so.tot_limit_kb, so.workspace,
                               so.tile_window, (cudaStream_t)stream, so.n_peer, so.peer3, so.mc3);
-    DIG_CHECK_ARG(so.n_peer == 0, "peer_counts3_d needs the lane-bank kernel (workspace, 128-base aligned genome, variant AUTO)");
-    if (so.variant != DIG_SCAN_PER_BASE)
-        return launch_scan_hex(packed2_d, nmask_d, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
-                               n_reg, counts5_d, counts3_d, totals5_d, totals3_d, so.tot_limit_kb,
-                               so.variant == DIG_SCAN_HEX_PLAIN, nullptr, nullptr, (cudaStream_t)stream);
-    const size_t smem = 1024 * 4 + 4096 + (size_t)WARPS_PER_BLOCK * 4096;
-    static thread_local int blocks_per_sm = 0;
-    if (blocks_per_sm == 0) {
-        DIG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, scan_fused53_kernel, THREADS, smem));
-        if (blocks_per_sm < 1) blocks_per_sm = 1;
-    }
-    int64_t blocks = (int64_t)dig::sm_count() * blocks_per_sm;
-    const int64_t need = (n_reg + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
-    if (blocks > need) blocks = need;
-    scan_fused53_kernel<<<(unsigned)blocks, THREADS, smem, (cudaStream_t)stream>>>(
-        reinterpret_cast<const uint2 *>(packed2_d), packed2_d, nmask_d, (n_bases + 31) >> 5, chrom_off_d, chrom_len_d,
-        reg_chrom_d, reg_start_d, reg_end_d, n_reg, counts5_d, counts3_d, totals5_d, totals3_d, so.tot_limit_kb);
-    DIG_CHECK_LAUNCH();
-    return DIG_OK;
+    DIG_CHECK_ARG(so.n_peer == 0, "peer_counts3_d needs the lane-bank kernel (workspace, N summary, 128-base aligned genome, "
+                                  "variant AUTO)");
+    return launch_scan_hex(packed2_d, nmask_d, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
+                           n_reg, counts5_d, counts3_d, totals5_d, totals3_d, so.tot_limit_kb, nullptr, nullptr,
+                           (cudaStream_t)stream);
 }
 
 extern "C" int64_t dig_scan_workspace_bytes(int64_t n_reg) { return (int64_t)scan_lb_workspace_bytes(n_reg); }
@@ -608,26 +424,27 @@ extern "C" int dig_count_contexts(const uint32_t *packed2_d, const uint32_t *nma
                   "null pointer");
     DIG_CHECK_ARG((reinterpret_cast<uintptr_t>(packed2_d) & 7u) == 0 && (reinterpret_cast<uintptr_t>(counts_d) & 15u) == 0,
                   "packed2_d must be 8-byte and counts_d 16-byte aligned");
-    DIG_CHECK_ARG(so.variant >= DIG_SCAN_AUTO && so.variant <= DIG_SCAN_HEX, "unknown scan variant");
+    DIG_CHECK_ARG(so.variant == DIG_SCAN_AUTO || so.variant == DIG_SCAN_PER_BASE || so.variant == DIG_SCAN_HEX,
+                  "unknown scan variant");
     cudaStream_t st = (cudaStream_t)stream;
+    const uint32_t *nsum = so.nsum_off > 0 ? nmask_d + so.nsum_off : nullptr;
     if (n_up == 2 && n_down == 2 && reg_strand_d == nullptr && so.variant == DIG_SCAN_AUTO &&
-        scan_lb_usable(packed2_d, nmask_d, n_bases, counts_d, so.workspace, so.workspace_bytes, n_reg))
-        return launch_scan_lb(packed2_d, nmask_d, so.nsum_off > 0 ? nmask_d + so.nsum_off : nullptr, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
+        scan_lb_usable(packed2_d, nmask_d, nsum, n_bases, counts_d, so.workspace, so.workspace_bytes, n_reg))
+        return launch_scan_lb(packed2_d, nmask_d, nsum, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
                               n_reg, counts_d, nullptr, totals_d, nullptr, so.tot_limit_kb, so.workspace, so.tile_window, st);
     // (the lane-bank kernel works in batches of 32 regions, one CTA per batch: with fewer than two batches per SM -- e.g.
     // 3 100 windows of 1 Mb -- the per-warp kernel spreads the work better)
     if (n_up == 1 && n_down == 1 && reg_strand_d == nullptr && so.variant == DIG_SCAN_AUTO &&
         n_reg >= (int64_t)64 * dig::sm_count() &&
-        scan_lb_usable(packed2_d, nmask_d, n_bases, counts_d, so.workspace, so.workspace_bytes, n_reg))
-        return launch_scan_lb(packed2_d, nmask_d, so.nsum_off > 0 ? nmask_d + so.nsum_off : nullptr, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
+        scan_lb_usable(packed2_d, nmask_d, nsum, n_bases, counts_d, so.workspace, so.workspace_bytes, n_reg))
+        return launch_scan_lb(packed2_d, nmask_d, nsum, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
                               n_reg, nullptr, counts_d, nullptr, totals_d, so.tot_limit_kb, so.workspace, so.tile_window, st,
                               so.n_peer, so.peer3, so.mc3);
     DIG_CHECK_ARG(so.n_peer == 0, "peer_counts3_d needs the trinucleotide lane-bank kernel (n_up = n_down = 1, plus strand, "
-                                  "workspace, >= 64 regions per SM, variant AUTO)");
+                                  "workspace, N summary, >= 64 regions per SM, variant AUTO)");
     if (n_up == 2 && n_down == 2 && reg_strand_d == nullptr && so.variant != DIG_SCAN_PER_BASE)
         return launch_scan_hex(packed2_d, nmask_d, n_bases, chrom_off_d, chrom_len_d, reg_chrom_d, reg_start_d, reg_end_d,
-                               n_reg, counts_d, nullptr, totals_d, nullptr, so.tot_limit_kb,
-                               so.variant == DIG_SCAN_HEX_PLAIN, nullptr, nullptr, st);
+                               n_reg, counts_d, nullptr, totals_d, nullptr, so.tot_limit_kb, nullptr, nullptr, st);
     if (n_up == n_down && n_up <= 2) {
         switch (n_up) {
         case 0:

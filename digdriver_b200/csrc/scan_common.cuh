@@ -149,7 +149,7 @@ int launch_scan_hex(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, con
                     const int64_t *chrom_len, const int32_t *reg_chrom, const int64_t *reg_start,
                     const int64_t *reg_end, int64_t n_reg, int32_t *counts5, int32_t *counts3,
                     unsigned long long *totals5, unsigned long long *totals3, unsigned int tot_limit_kb,
-                    bool plain_flush, const int32_t *rlist, const int32_t *rlist_n, cudaStream_t stream);
+                    const int32_t *rlist, const int32_t *rlist_n, cudaStream_t stream);
 
 // scan.cu: trinucleotide table of the regions in a device-side list (per-warp kernel; the lane-bank kernel's redo list)
 int launch_scan_tri_list(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int64_t *chrom_off,
@@ -158,11 +158,12 @@ int launch_scan_tri_list(const uint32_t *p2, const uint32_t *nm, int64_t n_bases
                          unsigned int tot_limit_kb, const int32_t *rlist, const int32_t *rlist_n, cudaStream_t stream);
 
 // scan_lb.cu: the same tables through the lane-bank kernel (one window per lane, conflict-free atomics), followed by
-// launch_scan_hex over the regions it could not take.  `workspace` holds that list (scan_lb_workspace_bytes).  `nsum`
-// (nullable): the per-128-base N summary of nm (dig_nmask_summary); with it the kernel stages the bases alone.
+// launch_scan_hex over the regions it could not take.  `workspace` holds that list (scan_lb_workspace_bytes).  `nsum`:
+// the per-128-base N summary of nm (dig_nmask_summary); the kernel stages the bases alone and reads the mask words of
+// mixed spans only.  scan_lb_usable says whether the kernel can take a call (a summary and a workspace among others).
 size_t scan_lb_workspace_bytes(int64_t n_reg);
-bool scan_lb_usable(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int32_t *counts5, const void *workspace,
-                    size_t workspace_bytes, int64_t n_reg);
+bool scan_lb_usable(const uint32_t *p2, const uint32_t *nm, const uint32_t *nsum, int64_t n_bases, const int32_t *counts5,
+                    const void *workspace, size_t workspace_bytes, int64_t n_reg);
 int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, const uint32_t *nsum, int64_t n_bases, const int64_t *chrom_off,
                    const int64_t *chrom_len, const int32_t *reg_chrom, const int64_t *reg_start, const int64_t *reg_end,
                    int64_t n_reg, int32_t *counts5, int32_t *counts3, unsigned long long *totals5,

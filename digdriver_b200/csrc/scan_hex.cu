@@ -38,6 +38,8 @@ using namespace digscan;
 namespace {
 
 // 8 warps x 2 CTAs per SM at 128 registers: 6 x 3 and 10 x 2 (96 registers, spills) measured 10-17 % slower
+constexpr int HEX_WARPS = 8, HEX_MIN_CTAS = 2;
+constexpr int HEX_THREADS = HEX_WARPS * 32;
 constexpr uint32_t H6_BYTES = 8192u;     // 4096 x 16 bit, per warp, also its alignment
 constexpr uint32_t C5_BYTES = 2048u;     // 1024 x 16 bit single-pentanucleotide corrections
 constexpr uint32_t C3_BYTES = 256u;      // 64 x int32 trinucleotide corrections
@@ -85,7 +87,6 @@ struct HexUnroll<32> {
 
 // acc += both marginals of the warp's hexamer histogram (+ the single-pentanucleotide corrections),
 // leaving them zeroed.  Lane owns output chunks cidx = 32 j + lane (bins 4 cidx .. 4 cidx + 3), j < 8.
-template <bool EXCH>
 __device__ __forceinline__ void hex_flush(unsigned char *h6, uint32_t hist, unsigned char *c5, bool singles, int lane,
                                           int (&acc)[32])
 {
@@ -106,33 +107,21 @@ __device__ __forceinline__ void hex_flush(unsigned char *h6, uint32_t hist, unsi
         acc[4 * j + 3] += (int)(ty >> 16);
     }
     __syncwarp();
-    // ... then the first marginal (sum over the last base) with read-and-zero.  The 128-bit accesses are 32 B
-    // apart: lanes 0-3 / 4-7 of a quarter-warp take opposite halves first, which keeps the eight lanes on eight
+    // ... then the first marginal (sum over the last base) with read-and-zero (ATOMS.EXCH.128).  The 128-bit accesses
+    // are 32 B apart: lanes 0-3 / 4-7 of a quarter-warp take opposite halves first, which keeps the eight lanes on eight
     // distinct 16-byte bank groups
     const int s = (lane >> 2) & 1;
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
         const int cidx = j * 32 + lane;
-        uint4 r0, r1;
-        if constexpr (EXCH) {
-            r0 = smem_take128(hist + 32 * cidx + 16 * s);
-            r1 = smem_take128(hist + 32 * cidx + 16 * (s ^ 1));
-        } else {
-            r0 = *reinterpret_cast<const uint4 *>(h6 + 32 * cidx + 16 * s);
-            r1 = *reinterpret_cast<const uint4 *>(h6 + 32 * cidx + 16 * (s ^ 1));
-        }
+        const uint4 r0 = smem_take128(hist + 32 * cidx + 16 * s);
+        const uint4 r1 = smem_take128(hist + 32 * cidx + 16 * (s ^ 1));
         const uint32_t f0 = (r0.x + r0.y) & 0xFFFFu, f1 = (r0.z + r0.w) & 0xFFFFu;   // bins 2s, 2s + 1
         const uint32_t g0 = (r1.x + r1.y) & 0xFFFFu, g1 = (r1.z + r1.w) & 0xFFFFu;   // bins 2 - 2s, 3 - 2s
         acc[4 * j + 0] += (int)(s ? g0 : f0);
         acc[4 * j + 1] += (int)(s ? g1 : f1);
         acc[4 * j + 2] += (int)(s ? f0 : g0);
         acc[4 * j + 3] += (int)(s ? f1 : g1);
-    }
-    if constexpr (!EXCH) {
-        __syncwarp();
-        uint4 *z = reinterpret_cast<uint4 *>(h6);
-#pragma unroll
-        for (int k = 0; k < (int)(H6_BYTES / 512u); ++k) z[k * 32 + lane] = make_uint4(0u, 0u, 0u, 0u);
     }
     if (singles) {
 #pragma unroll
@@ -218,8 +207,8 @@ __device__ __forceinline__ HexRegion hex_setup(const HexRaw raw, const uint2 *__
     return g;
 }
 
-template <int HEX_WARPS, int MIN_CTAS, bool TRI, bool TOT, bool EXCH>
-__global__ void __launch_bounds__(HEX_WARPS * 32, MIN_CTAS) scan_hex_kernel(
+template <bool TRI, bool TOT>
+__global__ void __launch_bounds__(HEX_THREADS, HEX_MIN_CTAS) scan_hex_kernel(
     const uint2 *__restrict__ p2v, const uint32_t *__restrict__ p2, const uint32_t *__restrict__ nmask,
     int64_t n_words32, const int64_t *__restrict__ chrom_off, const int64_t *__restrict__ chrom_len,
     const int32_t *__restrict__ reg_chrom, const int64_t *__restrict__ reg_start,
@@ -228,7 +217,6 @@ __global__ void __launch_bounds__(HEX_WARPS * 32, MIN_CTAS) scan_hex_kernel(
     unsigned long long *__restrict__ totals3, unsigned int tot_limit_kb, uint32_t one,
     const int32_t *__restrict__ rlist, const int32_t *__restrict__ rlist_n)
 {
-    constexpr int HEX_THREADS = HEX_WARPS * 32;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
@@ -283,7 +271,7 @@ __global__ void __launch_bounds__(HEX_WARPS * 32, MIN_CTAS) scan_hex_kernel(
             int acc[32];
 #pragma unroll
             for (int i = 0; i < 32; ++i) acc[i] = 0;
-            if (scanned) hex_flush<EXCH>(h6, hist, c5, singles, lane, acc);
+            if (scanned) hex_flush(h6, hist, c5, singles, lane, acc);
             int tri[2] = {0, 0};
 #pragma unroll
             for (int j = 0; j < 8; ++j)
@@ -447,16 +435,15 @@ __global__ void __launch_bounds__(HEX_WARPS * 32, MIN_CTAS) scan_hex_kernel(
     }
 }
 
-template <int HEX_WARPS, int MIN_CTAS, bool TRI, bool TOT, bool EXCH>
-int launch_hex_cfg(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int64_t *chrom_off,
+template <bool TRI, bool TOT>
+int launch_hex(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int64_t *chrom_off,
                const int64_t *chrom_len, const int32_t *reg_chrom, const int64_t *reg_start, const int64_t *reg_end,
                int64_t n_reg, int32_t *counts5, int32_t *counts3, unsigned long long *totals5,
                unsigned long long *totals3, unsigned int tot_limit_kb, const int32_t *rlist, const int32_t *rlist_n,
                cudaStream_t stream)
 {
-    constexpr int HEX_THREADS = HEX_WARPS * 32;
     constexpr size_t HEX_SMEM = H6_BYTES + (size_t)HEX_WARPS * (H6_BYTES + C5_BYTES + C3_BYTES);
-    auto kern = scan_hex_kernel<HEX_WARPS, MIN_CTAS, TRI, TOT, EXCH>;
+    auto kern = scan_hex_kernel<TRI, TOT>;
     static thread_local int blocks_per_sm = 0;
     if (blocks_per_sm == 0) {
         DIG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HEX_SMEM));
@@ -474,45 +461,21 @@ int launch_hex_cfg(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, cons
     return DIG_OK;
 }
 
-template <bool TRI, bool TOT, bool EXCH>
-int launch_hex(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int64_t *chrom_off,
-               const int64_t *chrom_len, const int32_t *reg_chrom, const int64_t *reg_start, const int64_t *reg_end,
-               int64_t n_reg, int32_t *counts5, int32_t *counts3, unsigned long long *totals5,
-               unsigned long long *totals3, unsigned int tot_limit_kb, const int32_t *rlist, const int32_t *rlist_n,
-               cudaStream_t stream)
-{
-    return launch_hex_cfg<8, 2, TRI, TOT, EXCH>(p2, nm, n_bases, chrom_off, chrom_len, reg_chrom, reg_start, reg_end,
-                                                n_reg, counts5, counts3, totals5, totals3, tot_limit_kb, rlist, rlist_n,
-                                                stream);
-}
-
 }  // namespace
 
 namespace digscan {
 
 // counts3 == nullptr: pentanucleotide table only.  totals5 (and totals3 when counts3 is given) may be null.
-// plain_flush selects LDS + STS instead of ATOMS.EXCH.128 at write-out (A/B hook, same results).
 int launch_scan_hex(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int64_t *chrom_off,
                     const int64_t *chrom_len, const int32_t *reg_chrom, const int64_t *reg_start,
                     const int64_t *reg_end, int64_t n_reg, int32_t *counts5, int32_t *counts3,
                     unsigned long long *totals5, unsigned long long *totals3, unsigned int tot_limit_kb,
-                    bool plain_flush, const int32_t *rlist, const int32_t *rlist_n, cudaStream_t stream)
+                    const int32_t *rlist, const int32_t *rlist_n, cudaStream_t stream)
 {
-#define DIG_HEX_CALL(TRI, TOT, EXCH)                                                                                   \
-    return launch_hex<TRI, TOT, EXCH>(p2, nm, n_bases, chrom_off, chrom_len, reg_chrom, reg_start, reg_end, n_reg,    \
-                                      counts5, counts3, totals5, totals3, tot_limit_kb, rlist, rlist_n, stream)
-    const int sel = (counts3 != nullptr ? 4 : 0) | (totals5 != nullptr ? 2 : 0) | (plain_flush ? 0 : 1);
-    switch (sel) {
-    case 0: DIG_HEX_CALL(false, false, false);
-    case 1: DIG_HEX_CALL(false, false, true);
-    case 2: DIG_HEX_CALL(false, true, false);
-    case 3: DIG_HEX_CALL(false, true, true);
-    case 4: DIG_HEX_CALL(true, false, false);
-    case 5: DIG_HEX_CALL(true, false, true);
-    case 6: DIG_HEX_CALL(true, true, false);
-    default: DIG_HEX_CALL(true, true, true);
-    }
-#undef DIG_HEX_CALL
+    auto launch = counts3 != nullptr ? (totals5 != nullptr ? launch_hex<true, true> : launch_hex<true, false>)
+                                     : (totals5 != nullptr ? launch_hex<false, true> : launch_hex<false, false>);
+    return launch(p2, nm, n_bases, chrom_off, chrom_len, reg_chrom, reg_start, reg_end, n_reg, counts5, counts3, totals5,
+                  totals3, tot_limit_kb, rlist, rlist_n, stream);
 }
 
 }  // namespace digscan

@@ -17,11 +17,11 @@
 //     per-warp kernel (16-bit fields, flushed as needed) right after this one; so are regions longer than
 //     LB_MAX_CHUNKS chunks.
 //   * genome staging: the 16 consumer warps split each 2048-base chunk of every window into 128-base spans; the
-//     chunk (+ one 16-byte granule of halo) of each of the 32 windows is brought into shared memory by TMA bulk
-//     copies (cp.async.bulk, mbarrier completion), two stages deep (plus slots aliased onto the slice buffers; with
-//     the per-128-base N summary only the bases are staged, see lb_span_states); consumer warp w issues the copies of windows
-//     2w and 2w+1 (ptxas serialises per-lane bulk copies, so they are spread over the warps).  Window strides of
-//     33 / 17 granules keep the 128-bit shared-memory reads of a quarter-warp on distinct banks.
+//     packed bases of the chunk (+ one 16-byte granule of halo) of each of the 32 windows are brought into shared
+//     memory by TMA bulk copies (cp.async.bulk, mbarrier completion), three stages deep plus a slot aliased onto the
+//     slice buffers.  The N mask is not staged: each span's state (no N, all N, mixed) comes from the per-128-base N
+//     summary (lb_span_states), and only mixed spans read their mask words, from global memory.  The producer warps
+//     issue the copies (see lb_producer).
 //   * write-out: pentanucleotide m gets dp4a(row m) (hexamers that START with m) plus byte f of the rows
 //     a.bcde over a (hexamers that END with m = bcdef).  Thread (warp w, lane l) produces four consecutive bins
 //     of window l per 64-bin slice, rotated by lane so the 128-bit stores into the slice buffer are conflict-free;
@@ -51,36 +51,31 @@ constexpr int LB_CONS = LB_CW * 32;
 constexpr int LB_SPAN = 128;                       // bases per consumer thread per chunk
 constexpr int LB_CHUNK = LB_CW * LB_SPAN;          // 2048
 constexpr uint32_t LB_DSTRIDE = (LB_CHUNK + 64) / 4;     // 528 B of packed bases per window and stage (33 granules)
-constexpr uint32_t LB_MSTRIDE = (LB_CHUNK + 128) / 8;    // 272 B of N mask (17 granules)
 // Lanes 4r .. 4r+3 form group r and work on windows r, r+8, r+16, r+24 of the batch: in a regular tiling those four
 // strips sit at a fixed pitch (8 windows, a multiple of 128 bases), so ONE 2-D TMA box load brings all four.  A group's
 // strips are the rows of the box (written one after the other) and the group starts 128-byte aligned.
-// Bank layout of the strips: a consumer warp reads the same 32 (16) bytes of all 32 strips with 128-bit loads, eight
-// lanes per pass, so the eight strips of lanes 8q .. 8q+7 (two groups) must start in eight different 16-byte columns of
-// the 128-byte bank row.  Rows of 34 (18) granules put a group's four strips on columns 0, 2, 4, 6, and the strips of ODD
-// groups begin one granule into their rows (the box of an odd group is fetched 16 bytes early): columns 1, 3, 5, 7.
-// (With 33 / 17-granule rows and no shift both groups sat on columns 0-3: every such load took two passes, the single
-// word loads behind them eight: 2.6 k of the 15 k shared-memory wavefronts per batch.)
+// Bank layout of the strips: a consumer warp reads the same 32 bytes of all 32 strips with 128-bit loads, eight lanes
+// per pass, so the eight strips of lanes 8q .. 8q+7 (two groups) must start in eight different 16-byte columns of the
+// 128-byte bank row.  Rows of 34 granules put a group's four strips on columns 0, 2, 4, 6, and the strips of ODD groups
+// begin one granule into their rows (the box of an odd group is fetched 16 bytes early): columns 1, 3, 5, 7.
+// (With 33-granule rows and no shift both groups sat on columns 0-3: every such load took two passes, the single word
+// loads behind them eight.)
 constexpr uint32_t LB_DROW = LB_DSTRIDE + 16u;           // 544 B: row pitch in shared memory = width of the data box
-constexpr uint32_t LB_MROW = LB_MSTRIDE + 16u;           // 288 B
 constexpr uint32_t LB_DGROUP = 4u * LB_DROW;             // 2176 = 17 x 128
-constexpr uint32_t LB_MGROUP = 4u * LB_MROW;             // 1152 = 9 x 128
-static_assert(LB_DGROUP % 128u == 0u && LB_MGROUP % 128u == 0u, "groups start 128-byte aligned (TMA box destination)");
-constexpr uint32_t LB_MBASE = 8u * LB_DGROUP;            // mask strips follow the eight data groups
-constexpr uint32_t LB_STAGE_BYTES = 8u * (LB_DGROUP + LB_MGROUP);
+static_assert(LB_DGROUP % 128u == 0u, "groups start 128-byte aligned (TMA box destination)");
+constexpr uint32_t LB_STAGE = 8u * LB_DGROUP;            // 17408 B: the bases of one chunk of 32 windows
 __device__ __forceinline__ int lb_win(int lane) { return (lane >> 2) + 8 * (lane & 3); }    // window of the batch a lane owns
 __device__ __forceinline__ uint32_t lb_dgroup(int lane) { return (uint32_t)(lane >> 2) * LB_DGROUP; }
-__device__ __forceinline__ uint32_t lb_mgroup(int lane) { return LB_MBASE + (uint32_t)(lane >> 2) * LB_MGROUP; }
 __device__ __forceinline__ uint32_t lb_dstrip(int lane) { return lb_dgroup(lane) + (uint32_t)(lane & 3) * LB_DROW + (uint32_t)((lane >> 2) & 1) * 16u; }
-__device__ __forceinline__ uint32_t lb_mstrip(int lane) { return lb_mgroup(lane) + (uint32_t)(lane & 3) * LB_MROW + (uint32_t)((lane >> 2) & 1) * 16u; }
 constexpr int LB_MAX_CHUNKS = 16;                  // regions up to ~32 kb; longer ones go to the per-warp kernel
 constexpr int LB_MAX_CHUNKS_TRI = 1 << 18;         // trinucleotide-only mode counts in 32 bits: regions up to 536 Mb
 constexpr int LB_EXC_CAP = 508;
 
 constexpr uint32_t OFF_TAB = 0u;                                   // [1024 rows][32 lanes] words
-constexpr uint32_t OFF_STG = 131072u;
+constexpr uint32_t OFF_STG = 131072u;                              // three stages of LB_STAGE bytes
+constexpr uint32_t OFF_SUM = OFF_STG + 3u * LB_STAGE;              // [4 slots][32 windows] span-state words, 1 KB reserved
 constexpr uint32_t OUT_BYTES = 32u * 64u * 4u;                     // one 64-bin slice of 32 windows
-constexpr uint32_t OFF_OUT = OFF_STG + 2u * LB_STAGE_BYTES;
+constexpr uint32_t OFF_OUT = OFF_SUM + 1024u;
 constexpr int LB_NOUT = LB_WW;                                     // slice buffers in flight
 constexpr uint32_t OFF_TRI = OFF_OUT + LB_NOUT * OUT_BYTES;        // [64 bins][33] ints (padded: transposable)
 constexpr uint32_t TRI_BYTES = 64u * 33u * 4u;
@@ -90,95 +85,54 @@ constexpr uint32_t OFF_CNT = OFF_EXC + 2u * EXC_BYTES;             // pairs coun
 constexpr uint32_t OFF_CHK = OFF_CNT + 256u;                       // sum of table bytes per window
 constexpr uint32_t OFF_FLG = OFF_CHK + 128u;                       // batch verdict, writer warp 0 -> the others
 constexpr uint32_t OFF_BAR = OFF_FLG + 16u;
-constexpr uint32_t LB_SMEM = OFF_BAR + 256u;                       // 17 barriers of 8 bytes
+constexpr uint32_t LB_SMEM = OFF_BAR + 256u;                       // 19 barriers of 8 bytes
 static_assert(OFF_BAR % 16u == 0u, "barrier block alignment");
 static_assert(LB_SMEM <= 232448u, "shared memory budget");
+static_assert(OFF_SUM + 4u * 128u <= OFF_OUT && LB_STAGE <= LB_NOUT * OUT_BYTES, "staging ring layout");
 
-// With the per-128-base N summary (LbArgs::nsum) a stage holds the bases alone: 8 x LB_DGROUP = 17 KB instead of 26 KB, so
-// THREE stages fit where two stood, and a fourth ring slot is aliased onto the slice buffers as before.  The span states
-// of every window and slot (one word per window, see lb_span_states) sit in the 1 KB left between the third stage and
-// the slice buffers.  Every other offset is the same in both layouts.
-constexpr uint32_t LB_BSTAGE = 8u * LB_DGROUP;                    // 17408 B: a stage of bases only
-constexpr uint32_t OFF_SUM = OFF_STG + 3u * LB_BSTAGE;             // [4 slots][32 windows] span-state words
-static_assert(OFF_SUM + 4u * 128u <= OFF_OUT && LB_BSTAGE <= LB_NOUT * OUT_BYTES, "bases-only ring layout");
-
-enum { BAR_FULL = 0, BAR_EMPTY = 2, BAR_OUTFULL = 4, BAR_OUTEMPTY = 8, BAR_DONE = 12, BAR_CLEAN = 13 };
-
-// Third staging slot of the pentanucleotide modes.  Two stages are all that fits beside the 128 KB table and the four
-// slice buffers -- but the slice buffers (32 KB, directly behind the two stages) are idle while a batch is being counted,
-// and one stage is 26 KB.  Chunk kq of a batch goes to slot kq % 3, slot 2 being the slice buffers: chunks 0 and 1 of the
-// NEXT batch can still be fetched during the write-out (slots 0 and 1), and slot 2 is only filled once the last tile of
-// the previous batch has left the buffers (BAR_OUTFREE, one arrival per writer warp; waiting for BAR_DONE instead, which
-// comes after the table clearing and warp 0's closing work, held chunk 2 -- and the chunks queued behind it -- back by
-// ~2 k cycles) and is always read before the batch barrier that precedes the next write-out.  Inside a batch a chunk is then requested three chunks ahead instead of two.
-#ifndef DIG_LB_STAGE3
-#define DIG_LB_STAGE3 1
-#endif
-constexpr bool LB_ST3 = DIG_LB_STAGE3 != 0;
-// With the N summary (bases-only stages) the ring has FOUR slots, chunk kq going to slot kq % 4: slots 0-2 are real
-// stages and slot 3 is the slice buffers, under the same BAR_OUTFREE rule.
-enum { BAR_FULL2 = 14, BAR_EMPTY2 = 15, BAR_OUTFREE = 16, BAR_FULL3 = 17, BAR_EMPTY3 = 18 };   // OUTFREE: the four writer warps have shipped their last tile of the batch
-__device__ __forceinline__ uint32_t lb3_full(uint32_t stage)
-{
-    return stage < 2u ? (uint32_t)BAR_FULL + stage : (stage == 2u ? (uint32_t)BAR_FULL2 : (uint32_t)BAR_FULL3);
-}
-__device__ __forceinline__ uint32_t lb3_empty(uint32_t stage)
-{
-    return stage < 2u ? (uint32_t)BAR_EMPTY + stage : (stage == 2u ? (uint32_t)BAR_EMPTY2 : (uint32_t)BAR_EMPTY3);
-}
-// slots of the pentanucleotide ring, the last one being the slice buffers; stg0 = sbase + OFF_STG
-template <bool NS>
-struct LbSlots {
-    static constexpr uint32_t N = NS ? 4u : 3u;
-};
-template <bool NS>
+// The staging ring of the pentanucleotide modes has FOUR slots: three stages fit beside the 128 KB table and the four
+// slice buffers, and the slice buffers (32 KB) are idle while a batch is being counted, so they are the fourth.  Chunk kq
+// of a batch goes to slot kq % 4: chunks 0-2 of the NEXT batch can still be fetched during the write-out (slots 0-2), and
+// slot 3 is only filled once the last tile of the previous batch has left the buffers (BAR_OUTFREE, one arrival per
+// writer warp; waiting for BAR_DONE instead, which comes after the table clearing and warp 0's closing work, held that
+// chunk -- and the chunks queued behind it -- back by ~2 k cycles) and is always read before the batch barrier that
+// precedes the next write-out.
+constexpr uint32_t LB_NSLOT = 4u;
+// barriers: slot s of the ring is BAR_FULL + s / BAR_EMPTY + s, slice buffer i BAR_OUTFULL + i / BAR_OUTEMPTY + i;
+// OUTFREE: the four writer warps have shipped their last tile of the batch
+enum { BAR_FULL = 0, BAR_EMPTY = 4, BAR_OUTFULL = 8, BAR_OUTEMPTY = 12, BAR_DONE = 16, BAR_CLEAN = 17, BAR_OUTFREE = 18 };
+// slot of the pentanucleotide ring, the last one being the slice buffers; stg0 = sbase + OFF_STG
 __device__ __forceinline__ uint32_t lb_slot(uint32_t stg0, uint32_t stage)
 {
-    if constexpr (NS) return stage < 3u ? stg0 + stage * LB_BSTAGE : stg0 + (OFF_OUT - OFF_STG);
-    else return stg0 + stage * LB_STAGE_BYTES;                    // slot 2 = OFF_OUT
+    return stage < 3u ? stg0 + stage * LB_STAGE : stg0 + (OFF_OUT - OFF_STG);
 }
 __device__ __forceinline__ uint32_t lb_slot_sum(uint32_t stg0, uint32_t stage) { return stg0 + (OFF_SUM - OFF_STG) + stage * 128u; }
 
-// Staging ring per mode.  The pentanucleotide modes have room for two stages next to their 128 KB table and the slice
-// buffers; the trinucleotide-only mode (32 KB table, no slice buffers) runs FOUR, which hides the ~3 k cycles between a
-// stage's release and its refill (poll + issue + copy latency) behind three chunks of work instead of one.
-template <int GM>
-struct LbRing {
-    static constexpr uint32_t NST = 2u, LOG = 1u, STG0 = OFF_STG, FULL0 = BAR_FULL, EMPTY0 = BAR_EMPTY;
-};
+// Shared-memory layout of the trinucleotide-only kernel: two teams of eight consumer + two writer + two producer warps
+// work on alternate batches, each with its own table, two stages, row block, exception lists and barriers; a warp takes
+// two spans of every chunk.  While one team is at its batch barrier, in its write-out or waiting for a chunk, the other
+// one keeps the integer and shared-memory pipes busy -- the overlap of phases that the pentanucleotide modes cannot have
+// for lack of room for a second 128 KB table.  (One team of sixteen consumer warps with a four-stage ring measured
+// 0.606 ms against 0.507 ms for two teams.)
+// A stage holds the bases (LB_STAGE bytes), then the span-state words of its 32 windows (TriL::SUM); its pitch is the
+// measured layout's, with 9 KB unused behind the state words.
 constexpr uint32_t TRI_TAB_BYTES = 256u * 128u;                      // [256 4-mers][32 lanes] words
-template <>
-struct LbRing<2> {                                                   // trinucleotide-only, one team: four stages
-    static constexpr uint32_t NST = 4u, LOG = 2u, STG0 = TRI_TAB_BYTES, FULL0 = 0u, EMPTY0 = 4u;
-};
-template <>
-struct LbRing<3> {                                                   // trinucleotide-only, two teams: two stages each
-    static constexpr uint32_t NST = 2u, LOG = 1u, STG0 = 0u /* per team, see TriL */, FULL0 = 0u, EMPTY0 = 2u;
-};
-enum { TBAR_OUTFULL = 8, TBAR_DONE = 9, TBAR_CLEAN = 10 };           // barrier slots of the trinucleotide-only mode
-
-// Shared-memory layout of the trinucleotide-only kernel.  TEAMS = 1: the sixteen consumer warps work on one batch at a
-// time (table 32 KB, four stages).  TEAMS = 2: two teams of eight consumer + two writer + two producer warps work on
-// alternate batches, each with its own table, two stages, row block, exception lists and barriers; a warp then takes
-// two spans of every chunk.  While one team is at its batch barrier, in its write-out or waiting for a chunk, the
-// other one keeps the integer and shared-memory pipes busy -- the overlap of phases that the pentanucleotide modes
-// cannot have for lack of room for a second 128 KB table.
-template <int TEAMS>
 struct TriL {
-    static constexpr int GM = TEAMS == 1 ? 2 : 3;
+    static constexpr int TEAMS = 2;
     static constexpr int CW = LB_CW / TEAMS, WW = LB_WW / TEAMS, PW = LB_PW / TEAMS, SPW = TEAMS;     // warps per team, spans per warp
-    static constexpr uint32_t NST = LbRing<GM>::NST;
+    static constexpr uint32_t NST = 2u;                                                  // stages per team
+    static constexpr uint32_t STAGE = 26624u, SUM = LB_STAGE;                            // stage pitch, state words in a stage
     static constexpr uint32_t TAB = 0u;                                                  // + team * TRI_TAB_BYTES
-    static constexpr uint32_t STG = TEAMS * TRI_TAB_BYTES;                               // + team * NST * LB_STAGE_BYTES
-    static constexpr uint32_t TRI = STG + 4u * LB_STAGE_BYTES;                           // + team * TRI_BYTES
+    static constexpr uint32_t STG = TEAMS * TRI_TAB_BYTES;                               // + team * NST * STAGE
+    static constexpr uint32_t TRI = STG + TEAMS * NST * STAGE;                           // + team * TRI_BYTES
     static constexpr uint32_t EXC = TRI + TEAMS * TRI_BYTES;                             // + team * 2 * EXC_BYTES
     static constexpr uint32_t BAR = EXC + TEAMS * 2u * EXC_BYTES;                        // + team * 128
     static constexpr uint32_t SMEM = BAR + TEAMS * 128u;
-    static constexpr uint32_t B_OUTFULL = TEAMS == 1 ? TBAR_OUTFULL : 4u, B_DONE = TEAMS == 1 ? TBAR_DONE : 5u,
-                              B_CLEAN = TEAMS == 1 ? TBAR_CLEAN : 6u;
+    static constexpr uint32_t B_FULL = 0u, B_EMPTY = 2u, B_OUTFULL = 4u, B_DONE = 5u, B_CLEAN = 6u;
 };
-static_assert(TriL<2>::SMEM <= 232448u && TriL<1>::SMEM <= 232448u, "shared memory budget");
-static_assert(TriL<1>::BAR % 16u == 0u && TriL<2>::BAR % 16u == 0u, "barrier block alignment");
+static_assert(TriL::SMEM <= 232448u, "shared memory budget");
+static_assert(TriL::BAR % 16u == 0u, "barrier block alignment");
+static_assert(TriL::SUM + 128u <= TriL::STAGE, "trinucleotide stage layout");
 
 // which batches, barriers and stages a producer warp works for (one team = the whole CTA in the pentanucleotide modes)
 struct LbTeam {
@@ -496,7 +450,7 @@ __device__ __forceinline__ void lb_mask_global(const uint32_t *__restrict__ nmas
 struct LbArgs {
     const uint32_t *p2;
     const uint32_t *nmask;
-    const uint32_t *nsum;     // per-128-base N summary (kernels instantiated with NS = true only)
+    const uint32_t *nsum;     // per-128-base N summary of nmask (lb_span_states)
     int64_t n_bases;
     const int64_t *chrom_off;
     const int64_t *chrom_len;
@@ -515,7 +469,7 @@ struct LbArgs {
     uint32_t top;             // = 0x01000000 (see field_inc)
     uint32_t zero;            // = 0
     int64_t tile_w;           // > 0: the caller says the regions tile chromosomes with windows of this size (a multiple of 16)
-    int64_t dshift, mshift;   // element offsets of the second row phase of the input tensor maps
+    int64_t dshift;           // element offset of the second row phase of the input tensor maps
     unsigned long long *timing;   // DIG_LB_TIMING builds only: phase counters (cycles summed over consumer warps)
     // fused all-gather of the trinucleotide rows (range-sharded runs, dig_scan_opts::peer_counts3_d): n_peer > 0 sends
     // every row to the same place in each rank's buffer -- one multimem store through the NVSwitch multicast alias when
@@ -557,19 +511,20 @@ __device__ __forceinline__ int lb_chunk_order(int kq, int nch) { return kq == 0 
 // The chunk sequence of a CTA is the concatenation of the chunks of its batches (each batch in lb_chunk_order).  In the
 // trinucleotide-only rings chunk number ci lands in stage ci & (NST - 1) once the chunk that used the stage before has
 // been read into registers by all consumer warps of the team; in the pentanucleotide modes chunk kq of a batch lands in
-// slot kq % 3 (kq % 4 with the N summary; the last slot = the slice buffers, see BAR_FULL2 / BAR_OUTFREE above), with one
-// fill-parity bit per slot.
+// slot kq % 4 (the last slot = the slice buffers, see LB_NSLOT above), with one fill-parity bit per slot.
+// With the bases, the producer lane of a window stores the states of the chunk's sixteen spans (lb_span_states).
 //   * Regular group (the four windows lie at a pitch of 8 tile windows in one chromosome, nothing clipped): the group
-//     leader issues TWO 2-D TMA box loads per chunk (4 rows x 528 B of bases, 4 rows x 272 B of mask) through tensor
-//     maps that view each genome array as rows of one pitch (lb_input_maps).
-//   * Anything else: every lane issues two 1-D bulk copies for its own window.  ptxas serialises per-lane bulk copies
+//     leader issues ONE 2-D TMA box load per chunk (4 rows x 544 B of bases) through tensor maps that view the packed
+//     genome as rows of one pitch (lb_input_maps).
+//   * Anything else: every lane issues a 1-D bulk copy for its own window.  ptxas serialises per-lane bulk copies
 //     (ELECT + five R2UR broadcasts, ~25 cycles per copy at SM level whatever the number of issuing warps), which
-//     is what the box path avoids: 16 operations per chunk instead of 64.
+//     is what the box path avoids: 8 operations per chunk instead of 32.
 struct LbMaps {
-    CUtensorMap d[2], m[2];   // bases / mask, each with two row phases (a box must not cross the end of a row)
+    CUtensorMap d[2];         // packed bases, two row phases (a box must not cross the end of a row)
 };
 
-template <int GM, bool NS>
+// GM: 0 / 1 = the pentanucleotide modes (four-slot ring), 2 = trinucleotide only (one team's two-stage ring)
+template <int GM>
 __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps, const LbTeam T, int pw, int lane)
 {
     const uint32_t bar = T.bar;
@@ -577,14 +532,13 @@ __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps,
     const int m = lane & 3;                                // row of the group's box
     const bool mine = (lane >> T.lane_shift) == pw;
     uint32_t ci = 0u;
-    constexpr bool ST3 = LB_ST3 && GM < 2;                 // three (NS: four) slots, the last one aliasing the slice buffers
-    constexpr uint32_t NSL = LbSlots<NS>::N;
+    constexpr bool PENTA = GM < 2;
     uint32_t uses = 0u, pbi = 0u;                          // bit s of uses: parity of the number of fills of slot s
     for (int64_t b = T.b0; b < n_batches; b += T.bstep, ++pbi) {
         const LbGeom g = lb_geom<GM>(b * 32 + lb_win(lane), A.n_reg, A.chrom_off, A.chrom_len, A.reg_chrom, A.reg_start, A.reg_end);
         const int nch = warp_max(g.nch);
         uint32_t st3 = 0u;
-        if constexpr (ST3) {
+        if constexpr (PENTA) {
             // batch pbi - 2 is closed (it practically always is): the parity wait for batch pbi - 1 below cannot alias
             if (pbi >= 2u) mbar_wait_idle(bar + 8u * BAR_OUTFREE, pbi & 1u);
         }
@@ -598,88 +552,76 @@ __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps,
                           g.O + (int64_t)g.nch * LB_CHUNK + 128 <= A.n_bases;      // every staged strip lies inside the arrays
         const uint32_t okm = __ballot_sync(0xffffffffu, fits);
         const bool regular = ((okm >> lead) & 0xFu) == 0xFu;
-        // Box coordinates of chunk 0 (element = uint32; a row of the data view holds 8 W bases = W / 2 elements, of the
-        // mask view W / 4): the two divisions are done once per batch, the chunk loop only adds.  The producers share
-        // the issue slots with sixteen consumer warps that saturate the integer pipe, so every instruction in the
-        // chunk loop delays the data.
-        const uint32_t ped = (uint32_t)(A.tile_w >> 1), pem = (uint32_t)(A.tile_w >> 2);
-        uint32_t xd0 = 0u, yd0 = 0u, xm0 = 0u, ym0 = 0u;
+        // Box coordinates of chunk 0 (element = uint32; a row of the view holds 8 W bases = W / 2 elements): the division
+        // is done once per batch, the chunk loop only adds.  The producers share the issue slots with sixteen consumer
+        // warps that saturate the integer pipe, so every instruction in the chunk loop delays the data.
+        const uint32_t ped = (uint32_t)(A.tile_w >> 1);
+        uint32_t xd0 = 0u, yd0 = 0u;
         if (regular && m == 0) {
-            const uint32_t ed = (uint32_t)(O0 >> 4), em = (uint32_t)(O0 >> 5);       // n_bases < 2^35 on this path
+            const uint32_t ed = (uint32_t)(O0 >> 4);                                  // n_bases < 2^35 on this path
             yd0 = ed / ped; xd0 = ed - yd0 * ped;
-            ym0 = em / pem; xm0 = em - ym0 * pem;
         }
         for (int kq = 0; kq < nch; ++kq, ++ci) {
             const int k = lb_chunk_order(kq, nch);
-            using R = LbRing<GM>;
             uint32_t stage, fpar, full_i, empty_i;
-            if constexpr (ST3) {
+            if constexpr (PENTA) {
                 stage = st3;
-                st3 = st3 == NSL - 1u ? 0u : st3 + 1u;
+                st3 = st3 == LB_NSLOT - 1u ? 0u : st3 + 1u;
                 fpar = (uses >> stage) & 1u;
                 uses ^= 1u << stage;
-                full_i = lb3_full(stage);
-                empty_i = lb3_empty(stage);
+                full_i = BAR_FULL + stage;
+                empty_i = BAR_EMPTY + stage;
             } else {
-                stage = ci & (R::NST - 1u);
-                fpar = (ci >> R::LOG) & 1u;
-                full_i = R::FULL0 + stage;
-                empty_i = R::EMPTY0 + stage;
+                stage = ci & (TriL::NST - 1u);
+                fpar = (ci >> 1) & 1u;
+                full_i = TriL::B_FULL + stage;
+                empty_i = TriL::B_EMPTY + stage;
             }
             // span states of this window's chunk: read (read-only data) before the wait for the slot hides the load
             uint32_t sw = 0u;
-            if constexpr (NS) {
-                if (mine && k < g.nch) sw = lb_span_states(A.nsum, A.n_bases, g.O + (int64_t)k * LB_CHUNK);
-            }
+            if (mine && k < g.nch) sw = lb_span_states(A.nsum, A.n_bases, g.O + (int64_t)k * LB_CHUNK);
             LB_T(t_e0);
             mbar_wait_idle(bar + 8u * empty_i, fpar ^ 1u);
-            if constexpr (ST3) {
+            if constexpr (PENTA) {
                 // the slice buffers are free once the previous batch's last tiles have left them
-                if (stage == NSL - 1u && pbi >= 1u) mbar_wait_idle(bar + 8u * BAR_OUTFREE, (pbi - 1u) & 1u);
+                if (stage == LB_NSLOT - 1u && pbi >= 1u) mbar_wait_idle(bar + 8u * BAR_OUTFREE, (pbi - 1u) & 1u);
             }
             LB_T(t_e1);
             const uint32_t full = bar + 8u * full_i;
-            const uint32_t stg = ST3 ? lb_slot<NS>(T.stg0, stage) : T.stg0 + stage * LB_STAGE_BYTES;
-            if constexpr (NS) {
-                // the state word goes where the mask strips went (trinucleotide-only rings, whose stages keep their size)
-                // or into the state block of the pentanucleotide ring; this lane's FULL arrival below releases it
-                if (mine) sts32((ST3 ? lb_slot_sum(T.stg0, stage) : stg + LB_MBASE) + (uint32_t)lb_win(lane) * 4u, sw);
-            }
+            const uint32_t stg = PENTA ? lb_slot(T.stg0, stage) : T.stg0 + stage * TriL::STAGE;
+            // the state word goes into the state block of the pentanucleotide ring or behind the bases of a trinucleotide
+            // stage; this lane's FULL arrival below releases it
+            if (mine) sts32((PENTA ? lb_slot_sum(T.stg0, stage) : stg + TriL::SUM) + (uint32_t)lb_win(lane) * 4u, sw);
             if (!mine) {
                 // another producer warp's window
             } else if (regular && k < g.nch) {
                 if (m == 0) {
-                    // chunk k starts k * 2048 bases = 128 k (64 k) elements further: at most one row wrap (W >= 4096)
-                    uint32_t xd = xd0 + 128u * (uint32_t)k, yd = yd0, xm = xm0 + 64u * (uint32_t)k, ym = ym0;
+                    // chunk k starts k * 2048 bases = 128 k elements further: at most one row wrap (W >= 4096)
+                    uint32_t xd = xd0 + 128u * (uint32_t)k, yd = yd0;
                     if (xd >= ped) { xd -= ped; ++yd; }
-                    if (xm >= pem) { xm -= pem; ++ym; }
                     // odd groups: the box starts one granule (four elements) early, see the bank layout above; a start
                     // before the row only reads zeros into a lead-in nobody looks at
                     const int lead = ((lane >> 2) & 1) * 4;
-                    int bxd = (int)xd - lead, bxm = (int)xm - lead, sd = 0, sm = 0;
+                    int bxd = (int)xd - lead, sd = 0;
                     if (bxd + (int)(LB_DROW / 4) > (int)ped) { bxd -= (int)A.dshift; sd = 1; }     // the box would cross the row end:
-                    if (bxm + (int)(LB_MROW / 4) > (int)pem) { bxm -= (int)A.mshift; sm = 1; }     // same row of the shifted view
-                    mbar_arrive_tx(full, 4u * (NS ? LB_DROW : LB_DROW + LB_MROW));
+                                                                                                   // same row of the shifted view
+                    mbar_arrive_tx(full, 4u * LB_DROW);
                     tensor_g2s(&maps->d[sd], stg + lb_dgroup(lane), bxd, (int)yd, full);
-                    if constexpr (!NS) tensor_g2s(&maps->m[sm], stg + lb_mgroup(lane), bxm, (int)ym, full);
                 } else {
                     mbar_arrive(full);
                 }
             } else if (k < g.nch) {
                 const int64_t G0 = g.O + (int64_t)k * LB_CHUNK;              // first staged base: multiple of 128, >= -128
-                int64_t dsrc = G0 >> 2, msrc = G0 >> 3;
-                uint32_t ddst = stg + lb_dstrip(lane), mdst = stg + lb_mstrip(lane);
-                int64_t dbytes = LB_DSTRIDE, mbytes = LB_MSTRIDE;
+                int64_t dsrc = G0 >> 2;
+                uint32_t ddst = stg + lb_dstrip(lane);
+                int64_t dbytes = LB_DSTRIDE;
                 if (G0 < 0) {                                                // no base before the genome is ever needed
                     dsrc = 0; ddst += 32u; dbytes -= 32;
-                    msrc = 0; mdst += 16u; mbytes -= 16;
                 }
-                const int64_t davail = (A.n_bases >> 2) - dsrc, mavail = (A.n_bases >> 3) - msrc;
+                const int64_t davail = (A.n_bases >> 2) - dsrc;
                 if (dbytes > davail) dbytes = davail;
-                if (mbytes > mavail) mbytes = mavail;
-                mbar_arrive_tx(full, (uint32_t)(NS ? dbytes : dbytes + mbytes));
+                mbar_arrive_tx(full, (uint32_t)dbytes);
                 bulk_g2s(ddst, reinterpret_cast<const unsigned char *>(A.p2) + dsrc, (uint32_t)dbytes, full);
-                if constexpr (!NS) bulk_g2s(mdst, reinterpret_cast<const unsigned char *>(A.nmask) + msrc, (uint32_t)mbytes, full);
             } else {
                 mbar_arrive(full);
             }
@@ -710,10 +652,9 @@ __device__ __forceinline__ void lb_producer(const LbArgs &A, const LbMaps *maps,
 // ahead for the slice buffers' OUTEMPTY barriers -- a barrier look is a round trip through the shared-memory pipe behind
 // the other warps' atomics.  Measured on one box, twice each: 0.925 ms without, 0.933-0.936 ms with the FULL probe,
 // 0.941-0.944 ms with the OUTEMPTY probe: the extra shared-memory operation costs more than the hidden latency.
-template <bool TRI, bool NS>
+template <bool TRI>
 __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int warp, int lane)
 {
-    constexpr uint32_t NSL = LbSlots<NS>::N;
     const uint32_t bar = sbase + OFF_BAR;
     const uint32_t tabl = sbase + OFF_TAB + (uint32_t)lane * 4u;
     const int64_t n_batches = (A.n_reg + 31) >> 5;
@@ -744,26 +685,18 @@ __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int
         uint32_t st3 = 0u;
         for (int kq = 0; kq < nch; ++kq, ++cit) {
             const int k = lb_chunk_order(kq, nch);
-            uint32_t stage, fpar, full_i, empty_i;
-            if constexpr (LB_ST3) {                        // slot kq % 3 (NS: kq % 4, see BAR_FULL2); the producers count the same way
-                stage = st3;
-                st3 = st3 == NSL - 1u ? 0u : st3 + 1u;
-                fpar = (uses >> stage) & 1u;
-                uses ^= 1u << stage;
-                full_i = lb3_full(stage);
-                empty_i = lb3_empty(stage);
-            } else {
-                stage = cit & 1u;
-                fpar = (cit >> 1) & 1u;
-                full_i = BAR_FULL + stage;
-                empty_i = BAR_EMPTY + stage;
-            }
+            // slot kq % 4 (see LB_NSLOT); the producers count the same way
+            const uint32_t stage = st3;
+            st3 = st3 == LB_NSLOT - 1u ? 0u : st3 + 1u;
+            const uint32_t fpar = (uses >> stage) & 1u;
+            uses ^= 1u << stage;
+            const uint32_t full_i = BAR_FULL + stage, empty_i = BAR_EMPTY + stage;
             LB_T(t_a);
             mbar_wait(bar + 8u * full_i, fpar);
             LB_T(t_b);
             LB_ACC(0, t_a, t_b);
             LB_ACC((kq == 0 ? 8 : (kq == 1 ? 9 : 10)), t_a, t_b);
-            const uint32_t stg = LB_ST3 ? lb_slot<NS>(sbase + OFF_STG, stage) : sbase + OFF_STG + stage * LB_STAGE_BYTES;
+            const uint32_t stg = lb_slot(sbase + OFF_STG, stage);
             {
                 // a span that holds no centre of any lane's window (the lead-in span, the tail of the last chunk)
                 const int base0 = k * LB_CHUNK + warp * LB_SPAN;
@@ -774,26 +707,14 @@ __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int
                 }
             }
             const uint32_t dptr = stg + lb_dstrip(lane) + (uint32_t)warp * 32u;
-            uint32_t D[9], M[5] = {0u, 0u, 0u, 0u, 0u}, sst = 0u;
-            uint32_t dep;
-            {
-                const uint4 a = lds128(dptr), c = lds128(dptr + 16u);
-                D[0] = a.x; D[1] = a.y; D[2] = a.z; D[3] = a.w;
-                D[4] = c.x; D[5] = c.y; D[6] = c.z; D[7] = c.w;
-                D[8] = lds32(dptr + 32u);
-                if constexpr (NS) {
-                    // this span's state (lb_span_states): one word per window, written by its producer lane
-                    const uint32_t sa = LB_ST3 ? lb_slot_sum(sbase + OFF_STG, stage) : stg + LB_MBASE;
-                    sst = (lds32(sa + (uint32_t)lb_win(lane) * 4u) >> (2 * warp)) & 3u;
-                    dep = (D[0] | D[4]) ^ (D[8] | sst);
-                } else {
-                    const uint32_t mptr = stg + lb_mstrip(lane) + (uint32_t)warp * 16u;
-                    const uint4 m = lds128(mptr);
-                    M[0] = m.x; M[1] = m.y; M[2] = m.z; M[3] = m.w;
-                    M[4] = lds32(mptr + 16u);
-                    dep = (D[0] | D[4]) ^ (D[8] | M[0]) ^ M[4];
-                }
-            }
+            uint32_t D[9], M[5] = {0u, 0u, 0u, 0u, 0u};
+            const uint4 a = lds128(dptr), c = lds128(dptr + 16u);
+            D[0] = a.x; D[1] = a.y; D[2] = a.z; D[3] = a.w;
+            D[4] = c.x; D[5] = c.y; D[6] = c.z; D[7] = c.w;
+            D[8] = lds32(dptr + 32u);
+            // this span's state (lb_span_states): one word per window, written by its producer lane
+            const uint32_t sst = (lds32(lb_slot_sum(sbase + OFF_STG, stage) + (uint32_t)lb_win(lane) * 4u) >> (2 * warp)) & 3u;
+            const uint32_t dep = (D[0] | D[4]) ^ (D[8] | sst);
             // the stage may be refilled as soon as all sixteen warps have arrived: only after the loads have RETURNED
             // (one register of each load instruction is enough: a warp's load instruction releases its scoreboard when
             // the data of ALL lanes has been written, so lane 0's dependence covers the warp)
@@ -809,21 +730,14 @@ __device__ __forceinline__ void lb_consumer(const LbArgs &A, uint32_t sbase, int
             LB_T(t_p0);
             const int base = k * LB_CHUNK + warp * LB_SPAN;                  // local base 0 relative to the origin
             const int lo5 = g.lo5 - base, hi5 = g.hi5 - base;                // centre c (local base index) valid: lo5 <= c < hi5
-            const uint32_t any_n = NS ? sst : M[0] | M[1] | M[2] | M[3] | (M[4] & 0xF0000000u);
             uint32_t PV[4] = {0u, 0u, 0u, 0u};
-#ifdef DIG_LB_UNIFORM_PATH
-            if (__all_sync(0xffffffffu, any_n == 0u && lo5 <= 2 && hi5 >= 130)) {
-#else
             // per lane, although a warp whose lanes disagree runs both bodies one after the other: sending the whole warp
             // through the predicated body instead was measured 9 % slower (1.041 vs 0.954 ms at hg19 scale)
-            if (any_n == 0u && lo5 <= 2 && hi5 >= 130) {
-#endif
+            if (sst == 0u && lo5 <= 2 && hi5 >= 130) {
                 lb_pairs<false>(D, tabl, A.k32, top_r, PV);
                 npairs += 64u;
-            } else if (k < g.nch && (!NS || sst != 3u)) {                    // (an all-N span has no valid centre)
-                if constexpr (NS) {
-                    if (sst != 0u) lb_mask_global(A.nmask, A.n_bases, g.O + base, M);       // mixed: rare, N-run edges
-                }
+            } else if (k < g.nch && sst != 3u) {                             // (an all-N span has no valid centre)
+                if (sst != 0u) lb_mask_global(A.nmask, A.n_bases, g.O + base, M);          // mixed: rare, N-run edges
                 const int lo3 = g.lo3 - base, hi3 = g.hi3 - base;
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
@@ -1020,9 +934,7 @@ __device__ __forceinline__ void lb_writer(const LbArgs &A, const CUtensorMap *tm
             if (lane == 0) {
                 bulk_wait_read<0>();                                         // the tile has left shared memory
                 mbar_arrive_after_loads(bar + 8u * (BAR_OUTEMPTY + q), dep, A.zero);
-                if constexpr (LB_ST3) {
-                    if (s4 == 3) mbar_arrive_after_loads(bar + 8u * BAR_OUTFREE, dep, A.zero);
-                }
+                if (s4 == 3) mbar_arrive_after_loads(bar + 8u * BAR_OUTFREE, dep, A.zero);
             }
             __syncwarp();
         }
@@ -1136,16 +1048,14 @@ __device__ __forceinline__ void lb_pairs4(const uint32_t (&D)[9], uint32_t tabl,
     }
 }
 
-template <int TEAMS, bool NS>
 __device__ __forceinline__ void lb_consumer_tri(const LbArgs &A, uint32_t sbase, int team, int warp, int lane)
 {
-    using L = TriL<TEAMS>;                                     // `warp` = index inside the team
-    using R = LbRing<L::GM>;
+    using L = TriL;                                            // `warp` = index inside the team
     const uint32_t bar = sbase + L::BAR + (uint32_t)team * 128u;
     const uint32_t tabl = sbase + L::TAB + (uint32_t)team * TRI_TAB_BYTES + (uint32_t)lane * 4u;
-    const uint32_t stg0 = sbase + L::STG + (uint32_t)team * R::NST * LB_STAGE_BYTES;
+    const uint32_t stg0 = sbase + L::STG + (uint32_t)team * L::NST * L::STAGE;
     const uint32_t trib = sbase + L::TRI + (uint32_t)team * TRI_BYTES;
-    const int64_t b0 = (int64_t)blockIdx.x * TEAMS + team, bstep = (int64_t)gridDim.x * TEAMS;
+    const int64_t b0 = (int64_t)blockIdx.x * L::TEAMS + team, bstep = (int64_t)gridDim.x * L::TEAMS;
     const int64_t n_batches = (A.n_reg + 31) >> 5;
     const uint32_t k128 = A.k32 << 2;
     uint32_t cit = 0u, bi = 0u;
@@ -1171,42 +1081,31 @@ __device__ __forceinline__ void lb_consumer_tri(const LbArgs &A, uint32_t sbase,
         }
         for (int kq = 0; kq < nch; ++kq, ++cit) {
             const int k = lb_chunk_order(kq, nch);                           // the order the producers stage the chunks in
-            const uint32_t stage = cit & (R::NST - 1u);
+            const uint32_t stage = cit & (L::NST - 1u);
             LB_T(t_a);
-            mbar_wait(bar + 8u * (R::FULL0 + stage), (cit >> R::LOG) & 1u);
+            mbar_wait(bar + 8u * (L::B_FULL + stage), (cit >> 1) & 1u);
             LB_T(t_b);
             LB_ACC(0, t_a, t_b);
-            const uint32_t stg = stg0 + stage * LB_STAGE_BYTES;
+            const uint32_t stg = stg0 + stage * L::STAGE;
             if (kq == 0) gnext = lb_geom2<2>(nact, nc, nrs, nre, A.chrom_off, A.chrom_len);
 #pragma unroll 1
           for (int sp = 0; sp < L::SPW; ++sp) {                             // the warp's spans of this chunk
             const int span = warp + sp * L::CW;
             if (!__any_sync(0xffffffffu, k < g.nch && g.lo3 - (k * LB_CHUNK + span * LB_SPAN) < 130 &&
                                              g.hi3 - (k * LB_CHUNK + span * LB_SPAN) > 2)) {
-                if (lane == 0) mbar_arrive(bar + 8u * (R::EMPTY0 + stage));   // no centre of any lane's window in this span
+                if (lane == 0) mbar_arrive(bar + 8u * (L::B_EMPTY + stage));  // no centre of any lane's window in this span
                 continue;
             }
             const uint32_t dptr = stg + lb_dstrip(lane) + (uint32_t)span * 32u;
-            uint32_t D[9], M[5] = {0u, 0u, 0u, 0u, 0u}, sst = 0u;
-            uint32_t dep;
-            {
-                const uint4 a = lds128(dptr), c = lds128(dptr + 16u);
-                D[0] = a.x; D[1] = a.y; D[2] = a.z; D[3] = a.w;
-                D[4] = c.x; D[5] = c.y; D[6] = c.z; D[7] = c.w;
-                D[8] = lds32(dptr + 32u);
-                if constexpr (NS) {                                          // span state (lb_span_states), in the mask's place
-                    sst = (lds32(stg + LB_MBASE + (uint32_t)lb_win(lane) * 4u) >> (2 * span)) & 3u;
-                    dep = (D[0] | D[4]) ^ (D[8] | sst);
-                } else {
-                    const uint32_t mptr = stg + lb_mstrip(lane) + (uint32_t)span * 16u;
-                    const uint4 m = lds128(mptr);
-                    M[0] = m.x; M[1] = m.y; M[2] = m.z; M[3] = m.w;
-                    M[4] = lds32(mptr + 16u);
-                    dep = (D[0] | D[4]) ^ (D[8] | M[0]) ^ M[4];
-                }
-            }
+            uint32_t D[9], M[5] = {0u, 0u, 0u, 0u, 0u};
+            const uint4 a = lds128(dptr), c = lds128(dptr + 16u);
+            D[0] = a.x; D[1] = a.y; D[2] = a.z; D[3] = a.w;
+            D[4] = c.x; D[5] = c.y; D[6] = c.z; D[7] = c.w;
+            D[8] = lds32(dptr + 32u);
+            const uint32_t sst = (lds32(stg + L::SUM + (uint32_t)lb_win(lane) * 4u) >> (2 * span)) & 3u;     // lb_span_states
+            const uint32_t dep = (D[0] | D[4]) ^ (D[8] | sst);
             __syncwarp();
-            if (lane == 0) mbar_arrive_after_loads(bar + 8u * (R::EMPTY0 + stage), dep, A.zero);
+            if (lane == 0) mbar_arrive_after_loads(bar + 8u * (L::B_EMPTY + stage), dep, A.zero);
             if (!clean) {
                 LB_T(t_c);
                 mbar_wait(bar + 8u * L::B_CLEAN, (bi - 1u) & 1u);
@@ -1217,14 +1116,11 @@ __device__ __forceinline__ void lb_consumer_tri(const LbArgs &A, uint32_t sbase,
             LB_T(t_p0);
             const int base = k * LB_CHUNK + span * LB_SPAN;
             const int lo3 = g.lo3 - base, hi3 = g.hi3 - base;                // centre c (local base index) valid: lo3 <= c < hi3
-            const uint32_t any_n = NS ? sst : M[0] | M[1] | M[2] | M[3] | (M[4] & 0xF0000000u);
             uint32_t PV[4] = {0u, 0u, 0u, 0u};
-            if (any_n == 0u && lo3 <= 2 && hi3 >= 130) {
+            if (sst == 0u && lo3 <= 2 && hi3 >= 130) {
                 lb_pairs4<false>(D, tabl, k128, PV);
-            } else if (k < g.nch && (!NS || sst != 3u)) {
-                if constexpr (NS) {
-                    if (sst != 0u) lb_mask_global(A.nmask, A.n_bases, g.O + base, M);
-                }
+            } else if (k < g.nch && sst != 3u) {
+                if (sst != 0u) lb_mask_global(A.nmask, A.n_bases, g.O + base, M);
 #pragma unroll
                 for (int j = 0; j < 4; ++j) {
                     // bit 31 - t of word j <-> centre at local base 32 j + t + 2, its trinucleotide = bases 32 j + t + 1 .. + 3
@@ -1251,9 +1147,8 @@ __device__ __forceinline__ void lb_consumer_tri(const LbArgs &A, uint32_t sbase,
         if (nch == 0) gnext = lb_geom2<2>(nact, nc, nrs, nre, A.chrom_off, A.chrom_len);
         if (!clean) mbar_wait(bar + 8u * L::B_CLEAN, (bi - 1u) & 1u);
         LB_T(t_s0);
-        if constexpr (TEAMS == 1) cons_sync();                               // every 4-mer of the batch is in the table
-        else if (team == 0) asm volatile("bar.sync 1, %0;" ::"n"(L::CW * 32) : "memory");
-        else asm volatile("bar.sync 3, %0;" ::"n"(L::CW * 32) : "memory");
+        if (team == 0) asm volatile("bar.sync 1, %0;" ::"n"(L::CW * 32) : "memory");         // every 4-mer of the batch
+        else asm volatile("bar.sync 3, %0;" ::"n"(L::CW * 32) : "memory");                   // is in the team's table
         LB_T(t_sa);
         LB_ACC(3, t_s0, t_sa);
         mbar_wait(bar + 8u * L::B_DONE, (bi & 1u) ^ 1u);                     // writer warp 0 has stored and re-zeroed the row block
@@ -1286,12 +1181,12 @@ __device__ __forceinline__ void lb_consumer_tri(const LbArgs &A, uint32_t sbase,
 #endif
 }
 
-template <bool TOT, int TEAMS>
+template <bool TOT>
 __device__ __forceinline__ void lb_writer_tri(const LbArgs &A, uint32_t sbase, int team, int q, int lane)
 {
-    using L = TriL<TEAMS>;
+    using L = TriL;
     const uint32_t bar = sbase + L::BAR + (uint32_t)team * 128u;
-    const int64_t b0 = (int64_t)blockIdx.x * TEAMS + team, bstep = (int64_t)gridDim.x * TEAMS;
+    const int64_t b0 = (int64_t)blockIdx.x * L::TEAMS + team, bstep = (int64_t)gridDim.x * L::TEAMS;
     const int64_t n_batches = (A.n_reg + 31) >> 5;
     uint32_t bi = 0u;
     unsigned int tot3[2] = {0u, 0u};
@@ -1374,11 +1269,10 @@ __device__ __forceinline__ void lb_writer_tri(const LbArgs &A, uint32_t sbase, i
     }
 }
 
-template <bool TOT, int TEAMS, bool NS>
+template <bool TOT>
 __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_tri_kernel(const LbArgs A, const __grid_constant__ LbMaps imaps)
 {
-    using L = TriL<TEAMS>;
-    using R = LbRing<L::GM>;
+    using L = TriL;
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     const uint32_t sbase = (uint32_t)__cvta_generic_to_shared(smem_raw);
     const int lane = threadIdx.x & 31;
@@ -1386,11 +1280,11 @@ __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_tri_kernel(const LbArgs
     if ((sbase & 127u) != 0u) __trap();
     for (uint32_t i = threadIdx.x; i < L::BAR / 16u; i += LB_THREADS) sts128(sbase + i * 16u, 0u, 0u, 0u, 0u);
     if (threadIdx.x == 0) {
-        for (int t = 0; t < TEAMS; ++t) {
+        for (int t = 0; t < L::TEAMS; ++t) {
             const uint32_t bar = sbase + L::BAR + (uint32_t)t * 128u;
-            for (uint32_t st = 0; st < R::NST; ++st) {
-                mbar_init(bar + 8u * (R::FULL0 + st), 32u);
-                mbar_init(bar + 8u * (R::EMPTY0 + st), LB_CW);              // sixteen spans per chunk, one arrival each
+            for (uint32_t st = 0; st < L::NST; ++st) {
+                mbar_init(bar + 8u * (L::B_FULL + st), 32u);
+                mbar_init(bar + 8u * (L::B_EMPTY + st), LB_CW);             // sixteen spans per chunk, one arrival each
             }
             mbar_init(bar + 8u * L::B_OUTFULL, L::CW);                      // all consumer warps of the team, per batch
             mbar_init(bar + 8u * L::B_DONE, 1u);
@@ -1402,19 +1296,19 @@ __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_tri_kernel(const LbArgs
     __syncthreads();
     if (warp >= LB_CW + LB_WW) {
         const int pw = warp - LB_CW - LB_WW, team = pw / L::PW;
-        lb_producer<L::GM, NS>(A, &imaps,
-                           LbTeam{(int64_t)blockIdx.x * TEAMS + team, (int64_t)gridDim.x * TEAMS, sbase + L::BAR + (uint32_t)team * 128u,
-                                  sbase + L::STG + (uint32_t)team * R::NST * LB_STAGE_BYTES, TEAMS == 1 ? 3 : 4},
-                           pw % L::PW, lane);
+        lb_producer<2>(A, &imaps,
+                       LbTeam{(int64_t)blockIdx.x * L::TEAMS + team, (int64_t)gridDim.x * L::TEAMS, sbase + L::BAR + (uint32_t)team * 128u,
+                              sbase + L::STG + (uint32_t)team * L::NST * L::STAGE, 4},
+                       pw % L::PW, lane);
     } else if (warp >= LB_CW) {
         const int ww = warp - LB_CW;
-        lb_writer_tri<TOT, TEAMS>(A, sbase, ww / L::WW, ww % L::WW, lane);
+        lb_writer_tri<TOT>(A, sbase, ww / L::WW, ww % L::WW, lane);
     } else {
-        lb_consumer_tri<TEAMS, NS>(A, sbase, warp / L::CW, warp % L::CW, lane);
+        lb_consumer_tri(A, sbase, warp / L::CW, warp % L::CW, lane);
     }
 }
 
-template <bool TRI, bool TOT, bool NS>
+template <bool TRI, bool TOT>
 __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_kernel(const LbArgs A, const __grid_constant__ CUtensorMap tmap,
                                                                 const __grid_constant__ LbMaps imaps)
 {
@@ -1427,14 +1321,11 @@ __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_kernel(const LbArgs A, 
     for (uint32_t i = threadIdx.x; i < OFF_BAR / 16u; i += LB_THREADS) sts128(sbase + i * 16u, 0u, 0u, 0u, 0u);
     if (threadIdx.x == 0) {
         const uint32_t bar = sbase + OFF_BAR;
-        mbar_init(bar + 8u * (BAR_FULL + 0), 32u);
-        mbar_init(bar + 8u * (BAR_FULL + 1), 32u);
-        mbar_init(bar + 8u * (BAR_EMPTY + 0), LB_CW);
-        mbar_init(bar + 8u * (BAR_EMPTY + 1), LB_CW);
-        mbar_init(bar + 8u * BAR_FULL2, 32u);
-        mbar_init(bar + 8u * BAR_EMPTY2, LB_CW);
-        mbar_init(bar + 8u * BAR_FULL3, 32u);
-        mbar_init(bar + 8u * BAR_EMPTY3, LB_CW);
+#pragma unroll
+        for (uint32_t st = 0; st < LB_NSLOT; ++st) {
+            mbar_init(bar + 8u * (BAR_FULL + st), 32u);
+            mbar_init(bar + 8u * (BAR_EMPTY + st), LB_CW);
+        }
         mbar_init(bar + 8u * BAR_OUTFREE, LB_WW);
 #pragma unroll
         for (int i = 0; i < LB_NOUT; ++i) {
@@ -1448,10 +1339,10 @@ __global__ void __launch_bounds__(LB_THREADS, 1) scan_lb_kernel(const LbArgs A, 
     }
     __syncthreads();
     if (warp >= LB_CW + LB_WW)
-        lb_producer<TRI, NS>(A, &imaps, LbTeam{(int64_t)blockIdx.x, (int64_t)gridDim.x, sbase + OFF_BAR, sbase + LbRing<TRI>::STG0, 3},
+        lb_producer<TRI>(A, &imaps, LbTeam{(int64_t)blockIdx.x, (int64_t)gridDim.x, sbase + OFF_BAR, sbase + OFF_STG, 3},
                          warp - LB_CW - LB_WW, lane);
     else if (warp >= LB_CW) lb_writer<TRI, TOT>(A, &tmap, sbase, warp - LB_CW, lane);
-    else lb_consumer<TRI, NS>(A, sbase, warp, lane);
+    else lb_consumer<TRI>(A, sbase, warp, lane);
 }
 
 typedef CUresult (*LbEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
@@ -1492,66 +1383,54 @@ int lb_tensor_map(CUtensorMap *tmap, int32_t *counts5, int64_t n_reg)
     return lb_encode(tmap, CU_TENSOR_MAP_DATA_TYPE_INT32, counts5, 1024u, (uint64_t)n_reg, 4096u, 64u, 32u);
 }
 
-// The two genome arrays as rows of 8 tile windows (8 W bases: 2 W bytes of packed bases, W bytes of mask), so that the
-// strips of windows r, r + 8, r + 16, r + 24 of a batch are the rows of one [4][strip] box.  A box must not run over the
-// end of a row, hence a second view of each array shifted by about half a row.  Returns the tile size actually usable
-// (0: no box path) through A.
+// The packed bases as rows of 8 tile windows (8 W bases = 2 W bytes), so that the strips of windows r, r + 8, r + 16,
+// r + 24 of a batch are the rows of one [4][strip] box.  A box must not run over the end of a row, hence a second view
+// shifted by half a row.  Returns the tile size actually usable (0: no box path) through A.
 int lb_input_maps(LbMaps *maps, LbArgs &A, int64_t tile_w)
 {
     A.tile_w = 0;
-    A.dshift = A.mshift = 0;
+    A.dshift = 0;
     memset(maps, 0, sizeof(*maps));
     if (tile_w < 4096 || (tile_w & 15) != 0 || tile_w > (int64_t)LB_MAX_CHUNKS * LB_CHUNK || A.n_bases >= ((int64_t)1 << 35))
         return DIG_OK;
-    const uint64_t dbytes = (uint64_t)A.n_bases >> 2, mbytes = (uint64_t)A.n_bases >> 3;
-    const uint64_t dpitch = 2u * (uint64_t)tile_w, mpitch = (uint64_t)tile_w;      // bytes per row
-    const uint64_t dsh = (dpitch / 2) & ~(uint64_t)15, msh = (mpitch / 2) & ~(uint64_t)15;
-    if (dbytes <= dsh + dpitch || mbytes <= msh + mpitch) return DIG_OK;           // tiny genome: not worth a map
+    const uint64_t dbytes = (uint64_t)A.n_bases >> 2;
+    const uint64_t dpitch = 2u * (uint64_t)tile_w;                                 // bytes per row
+    const uint64_t dsh = (dpitch / 2) & ~(uint64_t)15;
+    if (dbytes <= dsh + dpitch) return DIG_OK;                                     // tiny genome: not worth a map
     const unsigned char *p2b = reinterpret_cast<const unsigned char *>(A.p2);
-    const unsigned char *nmb = reinterpret_cast<const unsigned char *>(A.nmask);
     int rc = lb_encode(&maps->d[0], CU_TENSOR_MAP_DATA_TYPE_UINT32, p2b, dpitch / 4, (dbytes + dpitch - 1) / dpitch, dpitch,
                        LB_DROW / 4, 4u);
     if (rc == DIG_OK)
         rc = lb_encode(&maps->d[1], CU_TENSOR_MAP_DATA_TYPE_UINT32, p2b + dsh, dpitch / 4, (dbytes - dsh + dpitch - 1) / dpitch,
                        dpitch, LB_DROW / 4, 4u);
-    if (rc == DIG_OK)
-        rc = lb_encode(&maps->m[0], CU_TENSOR_MAP_DATA_TYPE_UINT32, nmb, mpitch / 4, (mbytes + mpitch - 1) / mpitch, mpitch,
-                       LB_MROW / 4, 4u);
-    if (rc == DIG_OK)
-        rc = lb_encode(&maps->m[1], CU_TENSOR_MAP_DATA_TYPE_UINT32, nmb + msh, mpitch / 4, (mbytes - msh + mpitch - 1) / mpitch,
-                       mpitch, LB_MROW / 4, 4u);
     if (rc != DIG_OK) return rc;
     A.tile_w = tile_w;
     A.dshift = (int64_t)(dsh / 4);
-    A.mshift = (int64_t)(msh / 4);
     return DIG_OK;
 }
 
-#ifndef DIG_LB_TRI_TEAMS
-#define DIG_LB_TRI_TEAMS 2
-#endif
-template <bool TOT, bool NS>
+template <bool TOT>
 int launch_lb_tri(const LbArgs &A, const LbMaps &imaps, cudaStream_t stream)
 {
-    constexpr int TEAMS = DIG_LB_TRI_TEAMS;
-    auto kern = scan_lb_tri_kernel<TOT, TEAMS, NS>;
+    constexpr int TEAMS = TriL::TEAMS;
+    auto kern = scan_lb_tri_kernel<TOT>;
     static thread_local bool attr_set = false;
     if (!attr_set) {
-        DIG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TriL<TEAMS>::SMEM));
+        DIG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TriL::SMEM));
         attr_set = true;
     }
     const int64_t n_batches = (A.n_reg + 31) >> 5;
     int64_t blocks = dig::sm_count();
     if (blocks > (n_batches + TEAMS - 1) / TEAMS) blocks = (n_batches + TEAMS - 1) / TEAMS;
-    kern<<<(unsigned)blocks, LB_THREADS, TriL<TEAMS>::SMEM, stream>>>(A, imaps);
+    kern<<<(unsigned)blocks, LB_THREADS, TriL::SMEM, stream>>>(A, imaps);
     DIG_CHECK_LAUNCH();
     return DIG_OK;
 }
 
-template <bool TRI, bool TOT, bool NS>
+template <bool TRI, bool TOT>
 int launch_lb(const LbArgs &A, const CUtensorMap &tmap, const LbMaps &imaps, cudaStream_t stream)
 {
-    auto kern = scan_lb_kernel<TRI, TOT, NS>;
+    auto kern = scan_lb_kernel<TRI, TOT>;
     static thread_local bool attr_set = false;
     if (!attr_set) {
         DIG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)LB_SMEM));
@@ -1576,10 +1455,10 @@ size_t scan_lb_workspace_bytes(int64_t n_reg) { return lb_list_bytes(n_reg) + 12
 size_t scan_lb_workspace_bytes(int64_t n_reg) { return lb_list_bytes(n_reg); }
 #endif
 
-bool scan_lb_usable(const uint32_t *p2, const uint32_t *nm, int64_t n_bases, const int32_t *counts5, const void *workspace,
-                    size_t workspace_bytes, int64_t n_reg)
+bool scan_lb_usable(const uint32_t *p2, const uint32_t *nm, const uint32_t *nsum, int64_t n_bases, const int32_t *counts5,
+                    const void *workspace, size_t workspace_bytes, int64_t n_reg)
 {
-    return workspace != nullptr && workspace_bytes >= scan_lb_workspace_bytes(n_reg) && (n_bases & 127) == 0 &&
+    return nsum != nullptr && workspace != nullptr && workspace_bytes >= scan_lb_workspace_bytes(n_reg) && (n_bases & 127) == 0 &&
            (reinterpret_cast<uintptr_t>(p2) & 15u) == 0 && (reinterpret_cast<uintptr_t>(nm) & 15u) == 0 &&
            (reinterpret_cast<uintptr_t>(counts5) & 15u) == 0 && (reinterpret_cast<uintptr_t>(workspace) & 15u) == 0 &&
            n_reg > 0 && n_reg < (int64_t)0x7fffffe0;
@@ -1623,10 +1502,7 @@ int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, const uint32_t *nsum,
     if (counts5 == nullptr) {
         // trinucleotide table alone: 4-mer pairs in 32-bit lane-bank counters, then the per-warp kernel over the list
         // (regions beyond LB_MAX_CHUNKS_TRI chunks, batches whose exception list overflowed)
-        if (nsum != nullptr)
-            rc = totals3 != nullptr ? launch_lb_tri<true, true>(A, imaps, stream) : launch_lb_tri<false, true>(A, imaps, stream);
-        else
-            rc = totals3 != nullptr ? launch_lb_tri<true, false>(A, imaps, stream) : launch_lb_tri<false, false>(A, imaps, stream);
+        rc = totals3 != nullptr ? launch_lb_tri<true>(A, imaps, stream) : launch_lb_tri<false>(A, imaps, stream);
         if (rc != DIG_OK) return rc;
         rc = launch_scan_tri_list(p2, nm, n_bases, chrom_off, chrom_len, reg_chrom, reg_start, reg_end, n_reg, counts3,
                                   totals3, tot_limit_kb, fb_list, fb_count, stream);
@@ -1636,20 +1512,13 @@ int launch_scan_lb(const uint32_t *p2, const uint32_t *nm, const uint32_t *nsum,
         }
         return rc;
     }
-    if (nsum != nullptr) {
-        if (counts3 != nullptr)
-            rc = totals5 != nullptr ? launch_lb<true, true, true>(A, tmap, imaps, stream) : launch_lb<true, false, true>(A, tmap, imaps, stream);
-        else
-            rc = totals5 != nullptr ? launch_lb<false, true, true>(A, tmap, imaps, stream) : launch_lb<false, false, true>(A, tmap, imaps, stream);
-    } else {
-        if (counts3 != nullptr)
-            rc = totals5 != nullptr ? launch_lb<true, true, false>(A, tmap, imaps, stream) : launch_lb<true, false, false>(A, tmap, imaps, stream);
-        else
-            rc = totals5 != nullptr ? launch_lb<false, true, false>(A, tmap, imaps, stream) : launch_lb<false, false, false>(A, tmap, imaps, stream);
-    }
+    if (counts3 != nullptr)
+        rc = totals5 != nullptr ? launch_lb<true, true>(A, tmap, imaps, stream) : launch_lb<true, false>(A, tmap, imaps, stream);
+    else
+        rc = totals5 != nullptr ? launch_lb<false, true>(A, tmap, imaps, stream) : launch_lb<false, false>(A, tmap, imaps, stream);
     if (rc != DIG_OK) return rc;
     rc = launch_scan_hex(p2, nm, n_bases, chrom_off, chrom_len, reg_chrom, reg_start, reg_end, n_reg, counts5, counts3,
-                         totals5, totals3, tot_limit_kb, false, fb_list, fb_count, stream);
+                         totals5, totals3, tot_limit_kb, fb_list, fb_count, stream);
     if (rc == DIG_OK && A.n_peer > 0) {
         lb_publish_redo_kernel<<<8, 256, 0, stream>>>(A);
         DIG_CHECK_LAUNCH();

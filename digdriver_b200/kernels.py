@@ -98,7 +98,8 @@ def count_contexts(genome, reg_chrom, reg_start, reg_end, n_up=1, n_down=1, stra
         out = torch.empty((n, K), dtype=torch.int32, device=dev)
     if want_totals and totals is None:
         totals = torch.zeros(K, dtype=torch.int64, device=dev)
-    lane_bank = (n_up, n_down) in ((2, 2), (1, 1)) and st is None and variant == _lib.SCAN_AUTO
+    lane_bank = ((n_up, n_down) in ((2, 2), (1, 1)) and st is None and variant == _lib.SCAN_AUTO
+                 and getattr(genome, "nsum", None) is not None)
     opts, opts_ref, workspace = _scan_opts(dev, n if lane_bank else 0, variant, totals_limit_kb,
                                            workspace if lane_bank else None,
                                            _tile_hint(reg_start, reg_end, tile_window) if lane_bank else 0,
@@ -130,7 +131,7 @@ def count_contexts_fused53(genome, reg_chrom, reg_start, reg_end, want_totals=Fa
     if want_totals and totals5 is None:
         totals5 = torch.zeros(1024, dtype=torch.int64, device=dev)
         totals3 = torch.zeros(64, dtype=torch.int64, device=dev)
-    lane_bank = variant == _lib.SCAN_AUTO
+    lane_bank = variant == _lib.SCAN_AUTO and getattr(genome, "nsum", None) is not None
     opts, opts_ref, workspace = _scan_opts(dev, n if lane_bank else 0, variant, totals_limit_kb,
                                            workspace if lane_bank else None,
                                            _tile_hint(reg_start, reg_end, tile_window) if lane_bank else 0,

@@ -75,13 +75,14 @@ int dig_pack_genome(const uint8_t *ascii_d, int64_t n_bases, uint32_t *packed2_d
  *
  * opts (nullable = all defaults) carries the per-call knobs; the library keeps no scan state between calls:
  *   workspace_d / workspace_bytes  caller-owned device scratch of dig_scan_workspace_bytes(n_reg) bytes, 16-byte
- *        aligned, contents irrelevant.  With it, pentanucleotide plus-strand scans (this call with n_up = n_down = 2
- *        and no strands, and dig_count_contexts_fused53) run the lane-bank kernel (csrc/scan_lb.cu: one window per
- *        lane, conflict-free shared-memory atomics, TMA staging); the scratch holds the device-side list of regions
- *        that kernel hands to the per-warp kernel (regions longer than ~32 kb, batches whose 8-bit counters
- *        overflowed).  Without it (or when n_bases is not a multiple of 128 / the arrays are not 16-byte aligned)
- *        the per-warp kernels run; results are identical.
- *   variant          DIG_SCAN_AUTO, or one specific kernel family for A/B measurements and tests
+ *        aligned, contents irrelevant.  With it AND the N summary (nsum_offset_words below), pentanucleotide
+ *        plus-strand scans (this call with n_up = n_down = 2 and no strands, and dig_count_contexts_fused53) and
+ *        trinucleotide plus-strand scans of >= 64 regions per SM run the lane-bank kernel (csrc/scan_lb.cu: one window
+ *        per lane, conflict-free shared-memory atomics, TMA staging); the scratch holds the device-side list of regions
+ *        that kernel hands to the per-warp kernel (regions longer than it takes, batches whose counters overflowed).
+ *        Without either (or when n_bases is not a multiple of 128 / the arrays are not 16-byte aligned) the per-warp
+ *        kernels run: identical results, slower.
+ *   variant          DIG_SCAN_AUTO, or one per-warp kernel family, which tests compare the lane-bank kernel against
  *   totals_limit_kb  0 = default; kilobases folded into 32-bit partial totals before they move to totals_d
  *   tile_window      0 = unknown.  > 0: a HINT that the regions are the reference's window tiling (DataExtractor.py:70-77:
  *        consecutive windows of this size from 0 in every chromosome, in order).  The lane-bank kernel then fetches the
@@ -90,9 +91,8 @@ int dig_pack_genome(const uint8_t *ascii_d, int64_t n_bases, uint32_t *packed2_d
  *        never correctness.  Used when it is a multiple of 16 and >= 4096.
  */
 #define DIG_SCAN_AUTO 0        /* lane-bank kernel when usable, else per-warp hexamer pairs, else per-base */
-#define DIG_SCAN_PER_BASE 1    /* one shared-memory atomic per base (scan.cu) */
-#define DIG_SCAN_HEX_PLAIN 2   /* per-warp hexamer pairs, LDS/STS flush */
-#define DIG_SCAN_HEX 3         /* per-warp hexamer pairs, ATOMS.EXCH.128 flush (scan_hex.cu) */
+#define DIG_SCAN_PER_BASE 1    /* one shared-memory atomic per base (scan.cu); dig_count_contexts only */
+#define DIG_SCAN_HEX 3         /* per-warp hexamer pairs (scan_hex.cu); any other value is DIG_ERR_ARG */
 typedef struct dig_scan_opts {
     void *workspace_d;
     int64_t workspace_bytes;
@@ -109,11 +109,11 @@ typedef struct dig_scan_opts {
      * only (DIG_ERR_ARG otherwise).  The caller orders the ranks afterwards (a device barrier) before reading. */
     int32_t n_peer_counts3;
     /* Per-128-base N summary of nmask_d (dig_nmask_summary): 0 = none.  > 0: the summary starts this many uint32 words
-     * after nmask_d, in the same allocation (a multiple of 4, at least dig_nmask_words(n_bases)).  With it the
-     * lane-bank kernel stages the packed bases alone (no mask) and reads each 128-base span's state -- no N, all N, or
+     * after nmask_d, in the same allocation (a multiple of 4, at least dig_nmask_words(n_bases)).  The lane-bank kernel
+     * needs it: it stages the packed bases alone (no mask) and reads each 128-base span's state -- no N, all N, or
      * mixed -- from the summary; only mixed spans read their mask words, from global memory.  The summary must describe
-     * nmask_d as it is at the time of the call (rebuild the part that covers any mask words you rewrite).  Results are
-     * identical with and without it. */
+     * nmask_d as it is at the time of the call (rebuild the part that covers any mask words you rewrite).  Without it
+     * the per-warp kernels run, with identical results. */
     int32_t nsum_offset_words;
     void *peer_counts3_d[8];
     void *mc_counts3_d;

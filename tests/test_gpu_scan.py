@@ -202,11 +202,12 @@ def test_fused_penta_tri_scan_matches_two_scans(dev, oracle, gold_dev_genome):
     assert np.array_equal(t5.cpu().numpy(), want5.sum(axis=0)) and np.array_equal(t3.cpu().numpy(), want3.sum(axis=0))
 
 
-def test_hexamer_pair_scan_adversarial(dev, oracle):
+def test_hexamer_pair_scan_adversarial_and_rejected_variants(dev, oracle):
     """scan_hex.cu counts pentanucleotides through hexamer pairs at even positions; this drives the parts
     that differ from the per-base kernels: pairs with a single valid centre (N every few bases, odd
     region boundaries, odd chromosome ends), 16-bit packed counters on homopolymers longer than one
-    flush interval (98 304 bases), regions shorter than one pair, and the register totals."""
+    flush interval (98 304 bases), regions shorter than one pair, and the register totals.  The retired variants
+    (variant 2, the per-base kernel of the fused scan) are rejected with DIG_ERR_ARG."""
     import ctypes
     from digdriver_b200 import kernels, _lib
     from digdriver_b200.genome import Genome, DeviceGenome
@@ -238,8 +239,8 @@ def test_hexamer_pair_scan_adversarial(dev, oracle):
     want5, _ = oracle.count_regions(seq, dg.chrom_off, dg.chrom_len, chrom, start, end, 2, 2)
     want3, _ = oracle.count_regions(seq, dg.chrom_off, dg.chrom_len, chrom, start, end, 1, 1)
     # lane-bank kernel (+ its redo list: the homopolymer overflows 8-bit fields, long regions exceed its chunk
-    # limit), per-warp hexamer kernel with ATOMS.EXCH.128 flush and with plain LDS/STS flush
-    for variant in (_lib.SCAN_AUTO, _lib.SCAN_HEX, _lib.SCAN_HEX_PLAIN):
+    # limit) and the per-warp hexamer kernel
+    for variant in (_lib.SCAN_AUTO, _lib.SCAN_HEX):
         for limit in (0, 64):                        # 64 kb: the register totals spill to global many times
             kw = dict(variant=variant, totals_limit_kb=limit)
             c5, c3, t5, t3 = kernels.count_contexts_fused53(dg, chrom, start, end, want_totals=True, **kw)
@@ -253,9 +254,14 @@ def test_hexamer_pair_scan_adversarial(dev, oracle):
             assert np.array_equal(p5.cpu().numpy(), want5) and np.array_equal(pt.cpu().numpy(), want5.sum(axis=0))
             q5, _ = kernels.count_contexts(dg, chrom, start, end, 2, 2, **kw)
             assert np.array_equal(q5.cpu().numpy(), want5)
-    # the per-base kernels stay available and agree
-    c5, c3, _, _ = kernels.count_contexts_fused53(dg, chrom, start, end, variant=_lib.SCAN_PER_BASE)
-    assert np.array_equal(c5.cpu().numpy(), want5) and np.array_equal(c3.cpu().numpy(), want3)
+    # the per-base kernels stay available and agree; the fused scan has none, and 2 names no variant
+    p5, _ = kernels.count_contexts(dg, chrom, start, end, 2, 2, variant=_lib.SCAN_PER_BASE)
+    assert np.array_equal(p5.cpu().numpy(), want5)
+    for variant in (_lib.SCAN_PER_BASE, 2):
+        with pytest.raises(_lib.DigError):
+            kernels.count_contexts_fused53(dg, chrom, start, end, variant=variant)
+    with pytest.raises(_lib.DigError):
+        kernels.count_contexts(dg, chrom, start, end, 2, 2, variant=2)
     # trinucleotide-only lane-bank kernel (4-mer pairs): it takes over from 64 regions per SM, so the same adversarial
     # set is repeated (and shuffled, so that every batch of 32 mixes chromosomes, lengths and parities); whole
     # chromosomes of 300 kb run through ~150 chunks per lane while their batch neighbours have one
@@ -272,7 +278,7 @@ def test_hexamer_pair_scan_adversarial(dev, oracle):
     assert np.array_equal(k3b.cpu().numpy(), want_big)
     # the same shuffled set through the FUSED lane-bank kernel, four times over: every CTA then works through several
     # consecutive batches whose chunk counts differ (0 to 16 chunks, long regions on the redo list), which is what the
-    # three-slot staging ring (slot kq % 3, the third slot aliased onto the slice buffers, one fill parity per slot) and
+    # four-slot staging ring (slot kq % 4, the fourth slot aliased onto the slice buffers, one fill parity per slot) and
     # its hand-offs across batch boundaries have to survive; twice, with and without register-total spills
     reps5 = 4 * reps
     order5 = np.random.default_rng(11).permutation(reps5 * len(chrom))

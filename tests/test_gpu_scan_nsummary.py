@@ -1,9 +1,9 @@
 """The per-128-base N summary (dig_nmask_summary) and the lane-bank scan that stages bases only when it has one.
 
-The summary is checked against a NumPy definition; the scan with the summary against the same scan without it
-(nsum_offset_words = 0: the mask is staged as before) and against the CPU oracle, on N layouts chosen to hit every case of the
-span-state rule: N runs starting and ending at every offset mod 128, single N in the four halo bases of the next block,
-windows inside N runs, N lead-ins, chromosome ends."""
+The summary is checked against a NumPy definition; the lane-bank scan, which runs only with the summary, against the
+same call without it (nsum_offset_words = 0: the per-warp kernels run) and against the CPU oracle, on N layouts chosen to
+hit every case of the span-state rule: N runs starting and ending at every offset mod 128, single N in the four halo
+bases of the next block, windows inside N runs, N lead-ins, chromosome ends."""
 import numpy as np
 import pytest
 import torch
@@ -125,6 +125,7 @@ def adv(oracle):
 
 
 def _both(dg, fn):
+    """fn() with the genome's summary (lane-bank kernel) and without it (per-warp kernels)."""
     nsum = dg.nsum
     try:
         with_sum = fn()

@@ -31,7 +31,7 @@ def launches(path):
     if any("scan_lb_kernel" in n for n, _ in names):
         is_scan = lambda n: "scan_lb_kernel" in n       # noqa: E731  (its redo pass, scan_hex_kernel, belongs to the same step)
     else:
-        is_scan = lambda n: "scan_fused53_kernel" in n or "scan_sym_kernel<2" in n or "scan_hex_kernel" in n   # noqa: E731
+        is_scan = lambda n: "scan_sym_kernel<2" in n or "scan_hex_kernel" in n   # noqa: E731
     big = max([v for n, v in names if is_scan(n)] or [0.0])
     # a step = one whole-genome scan (the per-chromosome scans of the e2e leg are much shorter) and what follows it,
     # up to the next scan or pack launch; the last COMPLETE one is reported (-c may cut the run anywhere)
