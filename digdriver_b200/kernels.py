@@ -433,7 +433,12 @@ def gene_scale_sums(mu, sigma, P, pi_indel, obs, cgc_mask=None, tp53=-1, stream=
 
 def gene_burden_test(mu, sigma, P, pi_indel, obs, nsamp, sums, n_syn, scale_factor=None, stream=None):
     """All 13 NB tests + Fisher per gene in one launch pair.  Returns float64 [27, E] (rows: GENE_OUT_ROWS).
-    n_syn=None: the synonymous count is sums[3] on the device (multi-GPU path, no host read)."""
+    n_syn=None: the synonymous count is sums[3] on the device (multi-GPU path, no host read), so without a
+    scale_factor sums must hold four values; gene_scale_sums returns three, and the caller appends the count."""
+    need = 4 if n_syn is None and scale_factor is None else 3
+    if sums.numel() < need:
+        raise ValueError("gene_burden_test: sums has %d values, the kernel reads %d (n_syn=None takes the synonymous "
+                         "count from sums[3])" % (sums.numel(), need))
     dev = mu.device
     E = mu.numel()
     out = torch.empty((len(GENE_OUT_ROWS), E), dtype=torch.float64, device=dev)

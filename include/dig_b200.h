@@ -319,7 +319,8 @@ int dig_fisher_combine2(const double *p1_d, const double *p2_d, int64_t n, doubl
  *   genic_driver_tools.py:158-159 (ELT_SIZE / R_SIZE for elements, :334-335) from the int64 outputs of
  *   dig_element_transfer, in one launch.
  * dig_gene_burden_test: cj = n_syn / sums[0] (or scale_factor when it is not NaN), t_indel = sums[2] / sums[1];
- *   a NaN n_syn means "read it from sums_d[3]" (the all-reduced value of a multi-GPU run, never copied to the host);
+ *   a NaN n_syn means "read it from sums_d[3]" (the all-reduced value of a multi-GPU run, never copied to the host):
+ *   sums_d then holds 4 values (dig_gene_scale_sums writes 3; the caller appends the count), otherwise 3;
  *   out_d [27, n_gene] rows: 0-5 EXP_{SYN,MIS,NONS,SPL,TRUNC,NONSYN}, 6-11 PVAL_*_BURDEN, 12-17
  *   PVAL_*_BURDEN_SAMPLE, 18 EXP_INDEL, 19 PVAL_INDEL_BURDEN, 20 PVAL_MUT_BURDEN (Fisher of TRUNC and INDEL),
  *   21 ALPHA, 22 THETA (scaled by cj), 23 THETA_INDEL, 24 Pi_INDEL, 25 Pi_TRUNC, 26 Pi_NONSYN.
