@@ -178,15 +178,18 @@ def expected_mutations_by_context(train_idx, test_idx, f_model, N=1, key_prefix=
 
 def _mutation_starts(tabix):
     """The reference reads mutations through pysam.TabixFile (absent here): accept a DataFrame with CHROM / START
-    columns, a (chrom, start) array pair, or a path to a mutation file readable by data_tools.read_mutation_file."""
+    columns, a (chrom, start) array pair, or a path to a mutation file readable by data_tools.read_mutation_file.
+    Chromosome names come back without a leading 'chr' in every form."""
     import pandas as pd
     if isinstance(tabix, (str, bytes)):
         from ..data_tools import mutation_tools
         tabix = mutation_tools.read_mutation_file(tabix, drop_sex=False)
     if isinstance(tabix, pd.DataFrame):
-        return tabix.CHROM.astype(str).str.replace("^chr", "", regex=True).values, tabix.START.values.astype(np.int64)
-    chrom, start = tabix
-    return np.asarray(chrom).astype(str), np.asarray(start, dtype=np.int64)
+        chrom, start = tabix.CHROM.values, tabix.START.values
+    else:
+        chrom, start = tabix
+    return (pd.Series(np.asarray(chrom)).astype(str).str.replace("^chr", "", regex=True).values,
+            np.asarray(start, dtype=np.int64))
 
 
 def nb_model(d_pr, idx, mu_lst, sigma_lst, f_tabix, f_fasta, n_up=2, n_down=2, binsize=50, collapse=False):
@@ -213,7 +216,8 @@ def nb_model(d_pr, idx, mu_lst, sigma_lst, f_tabix, f_fasta, n_up=2, n_down=2, b
                                 n_up=n_up, n_down=n_down, binsize=binsize)
     nb = np.diff(out["bin_ptr"])
     rep = lambda v: np.repeat(np.asarray(v), nb)
-    df = pd.DataFrame({"CHROM": rep([int(c) if c.isdigit() else c for c in chroms]),
+    # an object array keeps 'X' a string and '3' an int in one column (a plain array would make every label a string)
+    df = pd.DataFrame({"CHROM": rep(np.array([int(c) if c.isdigit() else c for c in chroms], dtype=object)),
                        "POS": out["pos"].cpu().numpy(), "OBS": out["obs"].cpu().numpy().astype(np.float64),
                        "EXP": out["exp"].cpu().numpy(), "PVAL": out["pval"].cpu().numpy(),
                        "Pi": out["pt"].cpu().numpy(), "MU": rep(mu), "SIGMA": rep(sigma)})

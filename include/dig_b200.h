@@ -391,6 +391,12 @@ int dig_site_test(const int32_t *site_chrom_d, const int64_t *site_start_d, cons
  *   ceil(n_positions / binsize), positions being the centres dig_count_contexts walks.  norm_d NULL = unnormalised
  *   (normed=False); pt_d / exp_d / pos_d may be NULL.
  * dig_nb_pvalue_exact replaces nb_model.nb_pvalue_exact(k, alpha, p) (nb_model.py:298-314) element-wise.
+ * Accuracy (tests/test_gpu_position_exact.py): norm is within (4^klen / 32 + 6) u of the correctly rounded dot product
+ *   (lane-strided sums, possibly FMA-contracted); pt = sum over the bin, position by position, of
+ *   __ddiv_rn(S_prob[k-mer], norm), exp = pt*mu, alpha = (mu*mu)/(sigma*sigma), theta = (sigma*sigma)/mu and
+ *   p = 1/(pt*theta + 1) are each rounded once in that order, so they are reproducible bit for bit from norm; pval
+ *   is within 1e-8 (log10) of a high-precision reference and within 1e-12 of dig_nb_pvalue_exact(obs, alpha, p), whose
+ *   inline copy the compiler contracts differently; obs, pos and the bin layout are exact.
  */
 int dig_region_prob_norm(const int32_t *counts_d, const double *s_prob_d, int64_t n_reg, int n_ctx, double *norm_d,
                          void *stream);

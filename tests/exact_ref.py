@@ -1,4 +1,4 @@
-"""Exact host references for the test stage (numpy and math.fsum only).
+"""Exact host references for the test stage and the per-position test (numpy and math.fsum only).
 
 A float64 kernel result is judged against the correctly rounded value of the same real-number expression, so a
 bound in units of u = 2^-53 measures the kernel's own rounding and nothing else:
@@ -8,6 +8,8 @@ bound in units of u = 2^-53 measures the kernel's own rounding and nothing else:
 - warp_dot_model(a, B): the summation order of the warp kernels (K6, dig_window_denominators) in numpy.
 - gene_transfer_ref(...): K6 gene / element mode with every sum exact.
 - tabulate_genes_ref(...): K5 gene mode from np.unique.
+- position_layout_ref, kmer_keys_ref, position_norm_ref, position_model_ref, position_obs_ref: K8's centres and bins,
+  k-mer keys, exact normaliser, arithmetic in the kernel's order, and observed counts and positions.
 """
 import math
 
@@ -45,15 +47,17 @@ def exact_dot(a, B):
 
 
 _LIMB = 21                                # |R| < 2^31 times a 21-bit limb stays below 2^52 per product
+_COLS = 2048                             # columns per int64 matrix product: 2048 * 2^31 * 2^21 = 2^63
 
 
 def exact_dot_int(a, R):
-    """Correctly rounded sum_j a[j] * R[i, j] for an integer matrix R (|R| < 2^31, at most 2048 columns) and finite a
+    """Correctly rounded sum_j a[j] * R[i, j] for an integer matrix R (|R| < 2^31, any number of columns) and finite a
     whose result is a normal float64.  Every a_j is an integer multiple of 2^e0 (e0 = the smallest exponent of its
-    last significand bit), so the sum is 2^e0 times an integer, formed exactly from int64 products of 21-bit limbs."""
+    last significand bit), so the sum is 2^e0 times an integer, formed exactly from int64 products of 21-bit limbs
+    over blocks of at most 2048 columns and combined as Python integers."""
     a = np.asarray(a, dtype=np.float64)
     R = np.atleast_2d(np.asarray(R))
-    assert R.dtype.kind in "iu" and R.shape[1] == a.size and a.size <= 2048
+    assert R.dtype.kind in "iu" and R.shape[1] == a.size
     R = R.astype(np.int64)
     assert R.size == 0 or np.abs(R).max() < 2 ** 31
     assert np.all(np.isfinite(a))
@@ -70,8 +74,11 @@ def exact_dot_int(a, R):
     for k in range(n_limb):
         # signed limbs: M_j = sum_k sign_j limb_jk 2^(21 k)
         limb = np.array([(1 if v >= 0 else -1) * ((abs(v) >> (_LIMB * k)) & mask) for v in M], dtype=np.int64)
-        s = R @ limb                                         # |s| < 2048 * 2^52: exact in int64
-        total = total + (s.astype(object) << (_LIMB * k))
+        if not limb.any():
+            continue
+        for c0 in range(0, a.size, _COLS):
+            s = R[:, c0:c0 + _COLS] @ limb[c0:c0 + _COLS]    # |s| < 2048 * 2^52: exact in int64
+            total = total + (s.astype(object) << (_LIMB * k))
     # Python's int / int is correctly rounded
     if e0 >= 0:
         return np.array([float(t << e0) for t in total])
@@ -203,3 +210,102 @@ def tabulate_genes_ref(gene, sample, cls, n_gene, cap=None):
     nsamp = np.zeros((n_gene, 7), dtype=np.int64)
     np.add.at(nsamp, kg, flags.astype(np.int64))
     return obs, nsamp
+
+
+# ---------------------------------------------------------------- K8: the per-position / per-bin hotspot test
+
+def position_layout_ref(chrom_len, reg_chrom, reg_start, reg_end, n_up, n_down, binsize):
+    """Per region: its first centre (chromosome coordinate), its number of positions and its number of bins, and the
+    CSR bin_ptr [n_reg + 1].  The rules of fetch_sequence (sequence_tools.py:21-29) and count_sequence_context
+    (:65-78): START == 0 becomes n_up; the fetched string is [START - n_up, END + n_down), which faidx clips at the
+    chromosome end (empty when it starts at or past the end); its centres are the bases with n_up bases before and
+    n_down after them inside the string."""
+    n = len(reg_chrom)
+    first, n_pos = np.zeros(n, dtype=np.int64), np.zeros(n, dtype=np.int64)
+    for r in range(n):
+        L = int(chrom_len[int(reg_chrom[r])])
+        start, end = int(reg_start[r]), int(reg_end[r])
+        if start == 0:
+            start = n_up
+        assert start >= n_up, "0 < START < n_up: the reference raises"
+        f0, f1 = start - n_up, end + n_down
+        f0, f1 = min(f0, L), min(f1, L)
+        first[r] = f0 + n_up
+        n_pos[r] = max(f1 - f0 - n_up - n_down, 0)
+    n_bin = (n_pos + binsize - 1) // binsize
+    return first, n_pos, n_bin, np.concatenate([[0], np.cumsum(n_bin)]).astype(np.int64)
+
+
+_CODE = np.full(256, -1, dtype=np.int64)
+for _i, _b in enumerate(b"ACGT"):
+    _CODE[_b] = _i
+    _CODE[_b | 0x20] = _i                    # the synthetic genome is half lower case: the reference upper-cases it
+
+
+def kmer_keys_ref(ascii, off, centres, n_up, n_down):
+    """(key, valid) of the k-mer [c - n_up, c + n_down] of every centre c: key = its base-4 index with the first
+    base most significant (mk_context_sequences order), valid = all of its bases are one of ACGTacgt.
+    ascii[i] is the base at coordinate off + i."""
+    ascii = np.asarray(ascii, dtype=np.uint8)
+    idx = np.asarray(centres, dtype=np.int64) - off - n_up
+    key = np.zeros(idx.shape, dtype=np.int64)
+    valid = np.ones(idx.shape, dtype=bool)
+    for j in range(n_up + n_down + 1):
+        c = _CODE[ascii[idx + j]]
+        valid &= c >= 0
+        key = key * 4 + np.maximum(c, 0)
+    return key, valid
+
+
+def position_norm_ref(s_prob, key, valid, region, n_reg):
+    """The exact normaliser of every region: the correctly rounded sum_k counts[r, k] s_prob[k], with the context
+    counts tabulated from the reference keys (region[i] = region of position i).  Returns (norm, counts)."""
+    K = len(s_prob)
+    counts = np.bincount(region[valid] * K + key[valid], minlength=n_reg * K).reshape(n_reg, K)
+    return exact_dot_int(s_prob, counts), counts
+
+
+def position_model_ref(s_prob, key, valid, n_pos, norm, mu, sigma, binsize):
+    """K8's arithmetic in the kernel's order, for regions whose positions are concatenated in key / valid (n_pos
+    each): q = s_prob[key] / norm (0 for an invalid k-mer), pt = q summed position by position over each bin (the last
+    bin padded with +0.0), exp = pt mu, alpha = (mu mu) / (sigma sigma), theta = (sigma sigma) / mu and
+    p = 1 / (pt theta + 1), every operation rounded once.  Given the kernel's own norm this is bit-identical to it.
+    Returns dict(pt, exp, alpha, p) per bin (alpha repeated over the region's bins)."""
+    n_pos = np.asarray(n_pos, dtype=np.int64)
+    n_bin = (n_pos + binsize - 1) // binsize
+    reg = np.repeat(np.arange(len(n_pos)), n_pos)
+    within = np.arange(len(reg)) - np.repeat(np.cumsum(n_pos) - n_pos, n_pos)
+    bin_of = np.repeat(np.cumsum(n_bin) - n_bin, n_pos) + within // binsize
+    with np.errstate(divide="ignore", invalid="ignore"):
+        q = np.where(valid, np.asarray(s_prob)[key], 0.0) / np.asarray(norm)[reg]
+    Q = np.zeros(int(n_bin.sum()) * binsize)
+    Q[bin_of * binsize + within % binsize] = q
+    Q = Q.reshape(-1, binsize)
+    pt = np.zeros(Q.shape[0])
+    for j in range(binsize):
+        pt = pt + Q[:, j]
+    m, s = np.repeat(np.asarray(mu, dtype=np.float64), n_bin), np.repeat(np.asarray(sigma, dtype=np.float64), n_bin)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        theta = (s * s) / m
+        return dict(pt=pt, exp=pt * m, alpha=(m * m) / (s * s), p=1.0 / (pt * theta + 1.0), q=q, bin_of=bin_of)
+
+
+def position_obs_ref(mut_chrom, mut_start, reg_chrom, first, n_pos, bin_ptr, binsize):
+    """obs per bin (mutation rows whose (chromosome, START) is a position of the bin, duplicates counted) and pos per
+    bin (the mean of its positions, first + b binsize + (n_in_bin - 1) / 2, exact in float64)."""
+    keys, cnt = np.unique((np.asarray(mut_chrom, dtype=np.int64) << 32) | np.asarray(mut_start, dtype=np.int64),
+                          return_counts=True)
+    rc = np.asarray(reg_chrom, dtype=np.int64)
+    lo = np.searchsorted(keys, (rc << 32) | first)
+    hi = np.searchsorted(keys, (rc << 32) | (first + n_pos))
+    nh = hi - lo
+    reg = np.repeat(np.arange(len(rc)), nh)
+    k = np.repeat(lo, nh) + np.arange(int(nh.sum())) - np.repeat(np.cumsum(nh) - nh, nh)
+    obs = np.zeros(int(bin_ptr[-1]), dtype=np.int64)
+    np.add.at(obs, bin_ptr[reg] + ((keys[k] & 0xFFFFFFFF) - first[reg]) // binsize, cnt[k])
+    n_bin = np.diff(bin_ptr)
+    reg_b = np.repeat(np.arange(len(rc)), n_bin)
+    b = np.arange(int(bin_ptr[-1])) - bin_ptr[reg_b]
+    n_in = np.minimum(binsize, n_pos[reg_b] - b * binsize)
+    pos = (first[reg_b] + b * binsize).astype(np.float64) + 0.5 * (n_in - 1).astype(np.float64)
+    return obs, pos

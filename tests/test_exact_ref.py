@@ -181,3 +181,115 @@ def test_burden_test_rejects_short_sums_before_launch():
         kernels.gene_burden_test(f, f, P, f, obs, nsamp, torch.zeros(2, dtype=torch.float64), 10.0)
     with pytest.raises(ValueError, match="sums"):
         kernels.gene_burden_test(f, f, P, f, obs, nsamp, torch.zeros(2, dtype=torch.float64), None, scale_factor=1.0)
+
+
+# ---------------------------------------------------------------- K8: the per-position test references
+
+def test_exact_dot_int_beyond_2048_columns_matches_fraction():
+    """K = 4096 (n_up + n_down = 5) needs two 2048-column blocks, combined as Python integers."""
+    rng = np.random.default_rng(7)
+    a = rng.lognormal(np.log(1e-6), 1.0, 4096)
+    a[rng.choice(4096, 40, replace=False)] = 0.0
+    R = rng.integers(0, 10_001, (6, 4096))
+    R[1] = 0
+    R[2, :2048] = 0                                          # only the second block
+    R[3] = rng.integers(0, 2 ** 31 - 1, 4096)                # every block's int64 sum near its limit
+    want = np.array([_frac_dot(a, R[i]) for i in range(len(R))])
+    assert np.array_equal(X.exact_dot_int(a, R), want)
+    assert np.array_equal(X.exact_dot_int(a[:2048], R[:, :2048]), [_frac_dot(a[:2048], R[i, :2048]) for i in range(6)])
+
+
+SHAPES = [(u, d) for u in range(6) for d in range(6) if u + d <= 5]
+
+
+@pytest.fixture(scope="module")
+def small_genome(oracle):
+    """Three chromosomes of the synthetic genome (half lower case) with N runs and an IUPAC base written in."""
+    lengths = [3001, 2048, 1777]
+    seqs = [oracle.synth_genome(1_000_000 * (c + 1), n, 11) for c, n in enumerate(lengths)]
+    seqs[0][500:640] = ord("N")
+    seqs[1][0:3] = ord("n")
+    seqs[1][1200:1207] = ord("N")
+    seqs[2][900] = ord("R")
+    seqs[2][1770:] = ord("N")
+    return seqs, np.array(lengths, dtype=np.int64)
+
+
+def _small_regions(lengths):
+    rows = [(0, 0, 40), (0, 480, 660), (0, 505, 600), (0, 630, 700), (0, 2950, 3001), (0, 2990, 3100),
+            (1, 0, 1), (1, 5, 6), (1, 1190, 1220), (1, 2040, 2048), (1, 2048, 2100), (1, 2100, 2200),
+            (2, 0, 250), (2, 880, 920), (2, 1700, 1900), (2, 10, 11), (2, 100, 400), (2, 150, 350)]
+    return np.array(rows, dtype=np.int64)
+
+
+@pytest.mark.parametrize("u,d", SHAPES)
+def test_position_refs_match_oracle(small_genome, oracle, u, d):
+    """Layout, k-mer keys and unnormalised probabilities against the oracle's line-faithful base_probabilities, and
+    obs / pos against its position_test, region by region on three chromosomes."""
+    seqs, lengths = small_genome
+    regs = _small_regions(lengths)
+    regs = regs[(regs[:, 1] == 0) | (regs[:, 1] >= u)]
+    rng = np.random.default_rng(100 + 6 * u + d)
+    s_prob = rng.lognormal(np.log(1e-6), 1.0, 4 ** (u + d + 1))
+    mut_c = rng.integers(0, 3, 3000)
+    mut_s = rng.integers(0, 3100, 3000)
+    for binsize in (1, 7):
+        first, n_pos, n_bin, ptr = X.position_layout_ref(lengths, regs[:, 0], regs[:, 1], regs[:, 2], u, d, binsize)
+        obs, pos = X.position_obs_ref(mut_c, mut_s, regs[:, 0], first, n_pos, ptr, binsize)
+        for r, (c, s, e) in enumerate(regs):
+            probs, poss = oracle.base_probabilities(seqs[c], int(s), int(e), s_prob, u, d, normed=False)
+            assert np.array_equal(first[r] + np.arange(n_pos[r]), poss), (u, d, r)
+            key, valid = X.kmer_keys_ref(seqs[c], 0, poss, u, d)
+            assert np.array_equal(np.where(valid, s_prob[key], 0.0), probs), (u, d, r)
+            if binsize == 1 or (u, d) in ((2, 2), (0, 5), (5, 0)):
+                _, wpos, wobs, _, _ = oracle.position_test(seqs[c], int(s), int(e), 10.0, 3.0, s_prob,
+                                                           mut_s[mut_c == c], u, d, binsize)
+                a, b = ptr[r], ptr[r + 1]
+                assert b - a == len(wpos)
+                assert np.array_equal(obs[a:b], wobs) and np.array_equal(pos[a:b], wpos), (u, d, binsize, r)
+
+
+def test_kmer_keys_first_base_most_significant():
+    seq = np.frombuffer(b"ACGTacgtNAC", dtype=np.uint8)
+    key, valid = X.kmer_keys_ref(seq, 100, np.array([101, 106, 109]), 1, 1)
+    assert key[0] == 0 * 16 + 1 * 4 + 2 and key[1] == 1 * 16 + 2 * 4 + 3
+    assert valid.tolist() == [True, True, False]
+
+
+@pytest.mark.parametrize("binsize", [2, 7, 50, 10_000, 10_001])
+def test_sequential_pt_model_within_bound(binsize):
+    """The kernel-order pt (a left-to-right sum over the bin) is within (binsize - 1) u of the exact sum of the same
+    quotients; bins of 1 are exact."""
+    import math
+    rng = np.random.default_rng(binsize)
+    n_pos = rng.integers(1, 3 * binsize, 40)
+    n_pos[0] = binsize
+    n_pos[1] = 1
+    K = 1024
+    s_prob = rng.lognormal(np.log(1e-6), 1.0, K)
+    key = rng.integers(0, K, int(n_pos.sum()))
+    valid = rng.random(key.size) > 0.05
+    norm = rng.lognormal(np.log(1e-2), 1.0, len(n_pos))
+    m = X.position_model_ref(s_prob, key, valid, n_pos, norm, np.full(40, 5.0), np.full(40, 2.0), binsize)
+    q, bin_of = m["q"], m["bin_of"]
+    order = np.argsort(bin_of, kind="stable")
+    edges = np.concatenate([[0], np.cumsum(np.bincount(bin_of, minlength=len(m["pt"])))])
+    exact = np.array([math.fsum(q[order[a:b]]) for a, b in zip(edges[:-1], edges[1:])])
+    err = X._rel_err_u(m["pt"], exact)
+    print("\nbinsize %d: sequential pt within %.2f u of the exact sum (bound %d u)" % (binsize, err.max(), binsize - 1))
+    assert err.max() <= binsize - 1
+    one = X.position_model_ref(s_prob, key, valid, n_pos, norm, np.full(40, 5.0), np.full(40, 2.0), 1)
+    assert np.array_equal(one["pt"], q)
+
+
+def test_nb_model_mutation_names_are_matched_without_chr():
+    """Mutation rows name chromosomes with or without 'chr', as a DataFrame or as a (chrom, start) pair: both forms
+    reach nb_model with the bare name, which it matches against the genome's names stripped of 'chr'."""
+    import pandas as pd
+    from digdriver_b200.sequence_model import nb_model as nb
+    want = ["1", "2", "22", "X"]
+    for names in (["chr1", "2", "chr22", "X"], ["1", "chr2", "22", "chrX"]):
+        c, s = nb._mutation_starts(pd.DataFrame({"CHROM": names, "START": [5, 6, 7, 8]}))
+        assert list(c) == want and list(s) == [5, 6, 7, 8]
+        c, s = nb._mutation_starts((np.array(names), np.array([5, 6, 7, 8])))
+        assert list(c) == want and list(s) == [5, 6, 7, 8]
