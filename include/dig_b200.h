@@ -563,6 +563,14 @@ int dig_annotate_snvs(const uint32_t *packed2_d, const uint32_t *nmask_d, int64_
  * dig_snv_codons: per (mutation, gene) pair of the interval join against the CDS blocks (as dig_annotate_snvs),
  *   codon_out_d int64 = the codon whose site the SNV is (position, REF and ALT; mut_ref_d / mut_alt_d uint8 0..3 as
  *   written), slot_out_d uint8 = its slot; -1 / 255 when it is no site of that gene.
+ * Accuracy (tests/test_gpu_codon_exact.py, 20 000 genes on a 3.1 Gb genome, 1 M cohort rows): K9a's L and flags,
+ *   K9b's classes, every field of K9c, K9d's codon and slot, and N_WIN, R_SIZE and FLAG of K10 are exact.  MU, R_OBS
+ *   and SIGMA = sqrt of the sum of fl(std * std) are sequential float64 sums from 0.0 over the window set in ascending
+ *   window order, and pi_num the sum of d_pr[bin] in slot order, so all four are reproducible bit for bit; pi_sum is one
+ *   correctly rounded division of pi_num by the sequential sum of the per-window denominators, bit-identical given
+ *   dig_window_denominators' output, and within 31 u of nonc_model's P_SUM for the same one-codon site set (the
+ *   correctly rounded numerator over the correctly rounded denominator): 16 u per window denominator, 2 u for the
+ *   sum over windows, 8 u for pi_num, 1 u for the division and 3 u for the reference's own roundings.
  */
 int dig_codon_sites(const uint32_t *packed2_d, const uint32_t *nmask_d, int64_t n_bases, const int64_t *chrom_off_d,
                     const int64_t *chrom_len_d, int n_chrom, const int32_t *gene_chrom_d, const int8_t *gene_strand_d,

@@ -10,6 +10,8 @@ bound in units of u = 2^-53 measures the kernel's own rounding and nothing else:
 - tabulate_genes_ref(...): K5 gene mode from np.unique.
 - position_layout_ref, kmer_keys_ref, position_norm_ref, position_model_ref, position_obs_ref: K8's centres and bins,
   k-mer keys, exact normaliser, arithmetic in the kernel's order, and observed counts and positions.
+- cds_engine(...): the gene annotation and codon rules over a whole gene set, vectorised; from it cds_table_ref (K9a),
+  annotate_ref (K9b), codon_records_ref (K9c), snv_codons_ref (K9d); codon_transfer_ref (K10) from the codon records.
 """
 import math
 
@@ -50,40 +52,56 @@ _LIMB = 21                                # |R| < 2^31 times a 21-bit limb stays
 _COLS = 2048                             # columns per int64 matrix product: 2048 * 2^31 * 2^21 = 2^63
 
 
+def int_limbs(a, limb=_LIMB):
+    """Integer form of finite float64 a: a_j = sum_k limbs[k, j] 2^(limb k) 2^e0 exactly, with signed limbs of `limb`
+    bits (int64 [n_limb, len(a)]).  Returns (limbs, e0)."""
+    a = np.asarray(a, dtype=np.float64)
+    assert np.all(np.isfinite(a))
+    nz = a != 0
+    if not nz.any():
+        return np.zeros((1, a.size), np.int64), 0
+    f, ex = np.frexp(a)                                      # a = f 2^ex, 0.5 <= |f| < 1
+    m = (f * 2.0 ** 53).astype(np.int64)                     # exact: a = m 2^(ex - 53)
+    e0 = int((ex - 53)[nz].min())
+    M = [int(mj) << int(xj - 53 - e0) if mj else 0 for mj, xj in zip(m, ex)]   # a_j = M_j 2^e0, Python ints
+    n_limb = max(abs(v).bit_length() for v in M) // limb + 1
+    mask = (1 << limb) - 1
+    limbs = np.array([[(1 if v >= 0 else -1) * ((abs(v) >> (limb * k)) & mask) for v in M] for k in range(n_limb)],
+                     dtype=np.int64)
+    return limbs, e0
+
+
+def limbs_to_float(S, e0, limb=_LIMB):
+    """Correctly rounded float64 of sum_k S[:, k] 2^(limb k) 2^e0 (S [n, n_limb] of integers, int64 or Python ints),
+    through Python integers: Python's int / int is correctly rounded."""
+    S = np.atleast_2d(np.asarray(S))
+    total = np.zeros(S.shape[0], dtype=object)
+    for k in range(S.shape[1]):
+        total = total + (S[:, k].astype(object) << (limb * k))
+    if e0 >= 0:
+        return np.array([float(t << e0) for t in total], dtype=np.float64)
+    return (total / (1 << -e0)).astype(np.float64)
+
+
 def exact_dot_int(a, R):
     """Correctly rounded sum_j a[j] * R[i, j] for an integer matrix R (|R| < 2^31, any number of columns) and finite a
-    whose result is a normal float64.  Every a_j is an integer multiple of 2^e0 (e0 = the smallest exponent of its
-    last significand bit), so the sum is 2^e0 times an integer, formed exactly from int64 products of 21-bit limbs
-    over blocks of at most 2048 columns and combined as Python integers."""
+    whose result is a normal float64.  Every a_j is an integer multiple of 2^e0 (int_limbs), so the sum is 2^e0 times
+    an integer, formed exactly from int64 products of 21-bit limbs over blocks of at most 2048 columns and combined as
+    Python integers (limbs_to_float)."""
     a = np.asarray(a, dtype=np.float64)
     R = np.atleast_2d(np.asarray(R))
     assert R.dtype.kind in "iu" and R.shape[1] == a.size
     R = R.astype(np.int64)
     assert R.size == 0 or np.abs(R).max() < 2 ** 31
-    assert np.all(np.isfinite(a))
-    nz = a != 0
-    if not nz.any():
-        return np.zeros(R.shape[0])
-    f, ex = np.frexp(a)                                      # a = f 2^ex, 0.5 <= |f| < 1
-    m = (f * 2.0 ** 53).astype(np.int64)                     # exact: a = m 2^(ex - 53)
-    e0 = int((ex - 53)[nz].min())
-    M = [int(mj) << int(xj - 53 - e0) if mj else 0 for mj, xj in zip(m, ex)]   # a_j = M_j 2^e0, Python ints
-    n_limb = max(abs(v).bit_length() for v in M) // _LIMB + 1
-    mask = (1 << _LIMB) - 1
-    total = np.zeros(R.shape[0], dtype=object)
-    for k in range(n_limb):
-        # signed limbs: M_j = sum_k sign_j limb_jk 2^(21 k)
-        limb = np.array([(1 if v >= 0 else -1) * ((abs(v) >> (_LIMB * k)) & mask) for v in M], dtype=np.int64)
+    limbs, e0 = int_limbs(a)
+    S = np.zeros((R.shape[0], len(limbs)), dtype=object)
+    for k, limb in enumerate(limbs):
         if not limb.any():
             continue
         for c0 in range(0, a.size, _COLS):
             s = R[:, c0:c0 + _COLS] @ limb[c0:c0 + _COLS]    # |s| < 2048 * 2^52: exact in int64
-            total = total + (s.astype(object) << (_LIMB * k))
-    # Python's int / int is correctly rounded
-    if e0 >= 0:
-        return np.array([float(t << e0) for t in total])
-    den = 1 << -e0
-    return np.array([t / den for t in total])
+            S[:, k] = S[:, k] + s.astype(object)
+    return limbs_to_float(S, e0)
 
 
 def butterfly(x):
@@ -309,3 +327,316 @@ def position_obs_ref(mut_chrom, mut_start, reg_chrom, first, n_pos, bin_ptr, bin
     n_in = np.minimum(binsize, n_pos[reg_b] - b * binsize)
     pos = (first[reg_b] + b * binsize).astype(np.float64) + 0.5 * (n_in - 1).astype(np.float64)
     return obs, pos
+
+
+# ---------------------------------------------------------------- K9a-K9d, K10: gene annotation and the codon test
+#
+# One vectorised engine restates the annotation rules of csrc/cdsannot.cu and the codon rules of csrc/codon.cu
+# (DESIGN.md section 5) for a whole gene set: transcripts are the genes' inclusive blocks, reversed on minus-strand
+# genes; bases come from the caller's reader (host bytes of each gene's span plus one base either side); amino acids
+# from NCBI table 1 with the consequence rules of oracle/cds_annot.py; essential-splice positions from
+# oracle/cds_annot.splice_positions, gene by gene.  Every output is an integer or a float64 sum in a stated order.
+
+_NO = 255                                  # no site / no hit / a codon with an N
+_ACGT = "ACGT"
+
+
+def _codon_tables():
+    """aa[c] (ASCII) of the 64 codons in ACGT index order (first base most significant), and the consequence code
+    cons[c_ref, c_alt]: 0 Synonymous, 1 Missense, 2 Nonsense, 5 Stop_loss (the DIG_CDS_* codes)."""
+    from oracle import cds_annot as O
+    names = [a + b + c for a in _ACGT for b in _ACGT for c in _ACGT]
+    aa = np.array([ord(O.CODON_TABLE[n]) for n in names], dtype=np.uint8)
+    stop = aa == ord("*")
+    cons = np.where(stop[None, :], 2, np.where(stop[:, None], 5, 1)).astype(np.uint8)
+    cons[aa[:, None] == aa[None, :]] = 0
+    return aa, cons
+
+
+_AA64, _CONS64 = _codon_tables()
+_BASE_CODE = np.full(256, 4, dtype=np.uint8)
+for _i, _b in enumerate(b"ACGT"):
+    _BASE_CODE[_b] = _BASE_CODE[_b | 0x20] = _i
+
+
+def _gene_dict(strand, ptr, bs, be, e):
+    return {"strand": int(strand[e]), "blocks": list(zip(bs[ptr[e]:ptr[e + 1]].tolist(), be[ptr[e]:ptr[e + 1]].tolist()))}
+
+
+def cds_engine(read, chrom_len, genes, donor=(1, 2, 5), acceptor=(1, 2), chunk=2000):
+    """The annotation and codon rules over every gene.  read(c, lo, n) returns the n bytes of chromosome c (genome
+    index) from position lo; genes = (chrom, strand, ptr, blk_start, blk_end) with inclusive, strictly ascending blocks.
+    Returns a dict: T [E] (CDS length), PTR [E+1] (floor(T / 3) codons per gene), per codon POS [n, 3], CC [n] (codon
+    code 16 b0 + 4 b1 + b2 of the transcript bases, 255 with an N), BIN / CLASS [n, 9], REF_AA [n], N_SITES [n]; per
+    gene L [E, 192, 4] (int64) and FLAGS [E]; SPLICE_KEY (sorted gene << 32 | position of every essential-splice
+    position).  Genes are processed `chunk` at a time, so only that many spans are in memory at once."""
+    from oracle import cds_annot as O
+    chrom, strand, ptr, bs, be = (np.asarray(x) for x in genes)
+    ptr, bs, be = ptr.astype(np.int64), bs.astype(np.int64), be.astype(np.int64)
+    chrom_len = np.asarray(chrom_len, dtype=np.int64)
+    E = len(chrom)
+    blen = be - bs + 1
+    owner = np.repeat(np.arange(E), np.diff(ptr))
+    T = np.bincount(owner, weights=blen, minlength=E).astype(np.int64)
+    nc = T // 3
+    cptr = np.concatenate([[0], np.cumsum(nc)]).astype(np.int64)
+    n = int(cptr[-1])
+    out = {"T": T, "PTR": cptr, "POS": np.zeros((n, 3), np.int64), "CC": np.zeros(n, np.uint8),
+           "BIN": np.full((n, 9), _NO, np.uint8), "CLASS": np.full((n, 9), _NO, np.uint8),
+           "REF_AA": np.zeros(n, np.uint8), "N_SITES": np.zeros(n, np.uint8),
+           "L": np.zeros((E, 192, 4), np.int64), "FLAGS": np.zeros(E, np.int32)}
+    rc = revcomp64()
+    splice_keys = []
+    for g0 in range(0, E, chunk):
+        g1 = min(g0 + chunk, E)
+        ge = np.arange(g0, g1)
+        Lc = chrom_len[chrom[ge]]
+        lo = np.maximum(bs[ptr[ge]] - 1, 0)
+        hi = np.minimum(be[ptr[ge + 1] - 1] + 2, Lc)
+        code = _BASE_CODE[np.concatenate([np.asarray(read(int(chrom[e]), int(a), int(b - a)), dtype=np.uint8)
+                                          for e, a, b in zip(ge, lo, hi)])]
+        boff = np.concatenate([[0], np.cumsum(hi - lo)])[:-1] - lo        # buffer index of (gene, p) = boff + p
+        # CDS bases in genomic order, then their transcript index
+        b0, b1 = ptr[g0], ptr[g1]
+        bl = blen[b0:b1]
+        nb = int(bl.sum())
+        blk = np.repeat(np.arange(b0, b1), bl)
+        gpos = bs[blk] + np.arange(nb) - np.repeat(np.cumsum(bl) - bl, bl)
+        gown = owner[blk]
+        loc = gown - g0
+        Tg = T[ge]
+        tstart = np.concatenate([[0], np.cumsum(Tg)])[:-1]
+        i_in_gene = np.arange(nb) - tstart[loc]
+        minus_b = strand[gown] < 0
+        tx = tstart[loc] + np.where(minus_b, Tg[loc] - 1 - i_in_gene, i_in_gene)
+        # transcript-ordered base, context and position
+        idx = boff[loc] + gpos
+        Lb = chrom_len[chrom[gown]]
+        has_ctx = (gpos >= 1) & (gpos + 1 < Lb)
+        i0, i2 = np.where(has_ctx, idx - 1, idx), np.where(has_ctx, idx + 1, idx)
+        t3 = np.stack([code[i0], code[idx], code[i2]], axis=1).astype(np.int64)
+        ok = has_ctx & (t3 < 4).all(axis=1)
+        ctx_g = 16 * t3[:, 0] + 4 * t3[:, 1] + t3[:, 2]
+        ctx = np.where(ok, np.where(minus_b, rc[np.where(ok, ctx_g, 0)], ctx_g), -1)
+        base = t3[:, 1]
+        tb = np.where(base < 4, np.where(minus_b, 3 - base, base), 4)
+        TB, CTX, TPOS = (np.empty(nb, np.int64) for _ in range(3))
+        TB[tx], CTX[tx], TPOS[tx] = tb, ctx, gpos
+        # codons
+        ncg = nc[ge]
+        cown = np.repeat(np.arange(g1 - g0), ncg)
+        k = np.arange(int(ncg.sum())) - np.repeat(np.cumsum(ncg) - ncg, ncg)
+        ti = tstart[cown][:, None] + 3 * k[:, None] + np.arange(3)[None, :]
+        cb, cx = TB[ti], CTX[ti]
+        has_n = (cb >= 4).any(axis=1)
+        cc = np.where(has_n, 0, 16 * cb[:, 0] + 4 * cb[:, 1] + cb[:, 2])
+        sl = slice(int(cptr[g0]), int(cptr[g1]))
+        out["POS"][sl] = TPOS[ti]
+        out["CC"][sl] = np.where(has_n, _NO, cc)
+        out["REF_AA"][sl] = np.where(has_n, 0, _AA64[cc])
+        bins = np.full((len(k), 9), _NO, np.int64)
+        clss = np.full((len(k), 9), _NO, np.int64)
+        Lg = np.zeros((g1 - g0) * 768, np.int64)
+        for j in range(3):
+            shift = 2 * (2 - j)
+            for r in range(3):
+                a = r + (r >= cb[:, j])
+                new = (cc & ~(3 << shift)) | (a << shift)
+                cls = _CONS64[cc, new].astype(np.int64)
+                live = ~has_n & (cx[:, j] >= 0)
+                b = 3 * cx[:, j] + r
+                inL = live & (cls != 5)
+                Lg += np.bincount(cown[inL] * 768 + b[inL] * 4 + cls[inL], minlength=len(Lg))
+                site = live & ((cls == 1) | (cls == 2))
+                bins[site, 3 * j + r] = b[site]
+                clss[site, 3 * j + r] = cls[site]
+        out["BIN"][sl], out["CLASS"][sl] = bins, clss
+        out["N_SITES"][sl] = (bins != _NO).sum(axis=1)
+        # flags: the trailing partial codon counts for the N flag but not for the stop flag
+        flags = np.where(Tg % 3 != 0, 1, 0)
+        nown = np.repeat(np.arange(g1 - g0), Tg)
+        flags |= np.where(np.bincount(nown[TB >= 4], minlength=g1 - g0) > 0, 2, 0)
+        stop = ~has_n & (_AA64[cc] == ord("*")) & (k < ncg[cown] - 1)
+        flags |= np.where(np.bincount(cown[stop], minlength=g1 - g0) > 0, 4, 0)
+        out["FLAGS"][g0:g1] = flags
+        # essential-splice positions, gene by gene from the plain-Python rule
+        se, sp = [], []
+        for e in ge:
+            q = O.splice_positions(_gene_dict(strand, ptr, bs, be, e), donor, acceptor)
+            se += [e] * len(q)
+            sp += q
+        se, sp = np.asarray(se, np.int64), np.asarray(sp, np.int64)
+        splice_keys.append((se << 32) | sp)
+        sl_loc = se - g0
+        si = boff[sl_loc] + sp
+        sLc = chrom_len[chrom[se]]
+        sok = (sp >= 1) & (sp + 1 < sLc)
+        s3 = np.stack([code[np.where(sok, si - 1, si)], code[si], code[np.where(sok, si + 1, si)]], axis=1).astype(np.int64)
+        sok &= (s3 < 4).all(axis=1)
+        sctx = 16 * s3[:, 0] + 4 * s3[:, 1] + s3[:, 2]
+        sctx = np.where(strand[se] < 0, rc[sctx & 63], sctx)
+        for r in range(3):
+            Lg += np.bincount(sl_loc[sok] * 768 + (3 * sctx[sok] + r) * 4 + 3, minlength=len(Lg))
+        out["L"][g0:g1] = Lg.reshape(-1, 192, 4)
+    out["SPLICE_KEY"] = np.sort(np.concatenate(splice_keys)) if splice_keys else np.zeros(0, np.int64)
+    return out
+
+
+def cds_table_ref(eng):
+    """K9a: L [E, 192, 4] (Synonymous, Missense, Nonsense, Essential_Splice) as float64, and the flags."""
+    return eng["L"].astype(np.float64), eng["FLAGS"]
+
+
+def codon_records_ref(eng):
+    """K9c: PTR, POS [n, 3], BIN / CLASS [n, 9], REF_AA, N_SITES."""
+    return {k: eng[k] for k in ("PTR", "POS", "BIN", "CLASS", "REF_AA", "N_SITES")}
+
+
+def _transcript_index(genes, T, e, p):
+    """Transcript index of position p in gene e (arrays), -1 where p is not a CDS base of that gene."""
+    chrom, strand, ptr, bs, be = genes
+    ptr, bs, be = (np.asarray(x, dtype=np.int64) for x in (ptr, bs, be))
+    e, p = np.asarray(e, dtype=np.int64), np.asarray(p, dtype=np.int64)
+    owner = np.repeat(np.arange(len(ptr) - 1, dtype=np.int64), np.diff(ptr))
+    blen = be - bs + 1
+    before = np.concatenate([[0], np.cumsum(blen)])[:-1] - np.concatenate([[0], np.cumsum(T)])[:-1][owner]
+    b = np.searchsorted((owner << 32) | bs, (e << 32) | p, side="right") - 1
+    bc = np.clip(b, 0, max(len(bs) - 1, 0))
+    hit = (b >= ptr[e]) & (b < ptr[e + 1]) & (p <= be[bc]) & (p >= bs[bc])
+    i = before[bc] + p - bs[bc]
+    t = np.where(np.asarray(strand)[e] < 0, T[e] - 1 - i, i)
+    return np.where(hit, t, -1)
+
+
+def _codon_of(eng, genes, e, p):
+    """(codon index or -1, phase j, transcript base of p or 4) of position p in gene e."""
+    t = _transcript_index(genes, eng["T"], e, p)
+    k = np.where(t >= 0, t // 3, 0)
+    ok = (t >= 0) & (k < np.diff(eng["PTR"])[e])
+    ci = np.where(ok, eng["PTR"][e] + k, -1)
+    cc = np.where(ok, eng["CC"][np.maximum(ci, 0)], _NO).astype(np.int64)
+    j = np.where(ok, t - 3 * k, 0)
+    tb = np.where(cc != _NO, (cc >> (2 * (2 - j))) & 3, 4)
+    return np.where(cc != _NO, ci, -1), j, tb, cc
+
+
+def annotate_ref(eng, genes, pair_gene, pos, alt):
+    """K9b: class of the SNV (genomic ALT 0..3, anything else none) at pos in gene pair_gene: the coding consequence
+    of a countable coding site (complete codon free of N), else 3 at an essential-splice position, else 255."""
+    strand = np.asarray(genes[1])
+    e, p, alt = (np.asarray(x, dtype=np.int64) for x in (pair_gene, pos, alt))
+    ci, j, tb, cc = _codon_of(eng, genes, e, p)
+    a = np.where(strand[e] < 0, 3 - alt, alt)
+    coding = (ci >= 0) & (alt < 4) & (a != tb)
+    shift = 2 * (2 - j)
+    new = (np.where(cc == _NO, 0, cc) & ~(3 << shift)) | (np.clip(a, 0, 3) << shift)
+    cls = np.where(coding, _CONS64[np.where(cc == _NO, 0, cc), new], _NO)
+    key = (e << 32) | p
+    sk = eng["SPLICE_KEY"]
+    at = np.searchsorted(sk, key)
+    splice = (at < len(sk)) & (sk[np.minimum(at, max(len(sk) - 1, 0))] == key) if len(sk) else np.zeros(len(e), bool)
+    incds = _transcript_index(genes, eng["T"], e, p) >= 0
+    cls = np.where(~incds & splice & (alt < 4), 3, cls)
+    return cls.astype(np.uint8)
+
+
+def snv_codons_ref(eng, genes, pair_gene, pos, ref, alt):
+    """K9d: (codon, slot) of the SNV (genomic REF / ALT codes) at pos in gene pair_gene: a site only when REF and ALT
+    are bases, differ, REF equals the genome's base and the slot holds a bin; (-1, 255) otherwise."""
+    strand = np.asarray(genes[1])
+    e, p, ref, alt = (np.asarray(x, dtype=np.int64) for x in (pair_gene, pos, ref, alt))
+    ci, j, tb, _ = _codon_of(eng, genes, e, p)
+    minus = strand[e] < 0
+    rt, at = np.where(minus, 3 - ref, ref), np.where(minus, 3 - alt, alt)
+    ok = (ci >= 0) & (ref < 4) & (alt < 4) & (ref != alt) & (rt == tb)
+    slot = 3 * j + np.where(at > tb, at - 1, at)
+    slot = np.where(ok, slot, 0)
+    ok &= eng["BIN"][np.maximum(ci, 0), slot] != _NO
+    return np.where(ok, ci, -1), np.where(ok, slot, _NO).astype(np.uint8)
+
+
+def window_rows(win_map_off, win_map, chrom_num, wn):
+    """Row of window number wn of chromosome number chrom_num in the dense window map, -1 where absent."""
+    off = np.asarray(win_map_off, dtype=np.int64)
+    c, wn = np.asarray(chrom_num, dtype=np.int64), np.asarray(wn, dtype=np.int64)
+    inr = (c >= 0) & (c < len(off) - 1) & (wn >= 0)
+    cc = np.where(inr, c, 0)
+    inr &= wn < off[cc + 1] - off[cc]
+    return np.where(inr, np.asarray(win_map)[np.where(inr, off[cc] + wn, 0)], -1).astype(np.int64)
+
+
+def codon_transfer_ref(rec, gene_chrom_num, gene_strand, window, win_map_off, win_map, win_counts, y_pred, std, y_true,
+                       flag, d_pr, denom_plus=None, denom_minus=None, exact=True):
+    """K10 per codon from its window set: the sorted distinct floor(p / window) of the bases that carry a site, each
+    looked up in the window map of the gene's chromosome NUMBER.  Exact: N_WIN (windows found), R_SIZE (their 64
+    counts summed), FLAG (OR), MISSING (a window of the set is absent).  Sequential float64 sums from 0.0 in ascending
+    window order: MU, SIGMA = sqrt(sum fl(s s)), R_OBS; PI_NUM = sum of d_pr[bin] in slot order.  PI_SUM (with the
+    given per-window denominators, by strand) = fl(PI_NUM / their sequential sum): the kernel's order.  PI_SUM_EXACT =
+    fl(sum d_pr[bin]) / fl(sum_j d_pr[j] R[j / 3]) with both sums correctly rounded and R the strand-ordered sum of the
+    window counts -- nonc_model's P_SUM for a one-codon site set.  Codons without sites are all zero; MU, SIGMA,
+    PI_SUM and PI_SUM_EXACT are NaN for a codon with a missing window.  exact=False skips PI_SUM_EXACT."""
+    ptr, pos, bins = rec["PTR"], rec["POS"], rec["BIN"].astype(np.int64)
+    n = len(bins)
+    gene = np.repeat(np.arange(len(ptr) - 1), np.diff(ptr))
+    minus = np.asarray(gene_strand)[gene] < 0
+    cnum = np.asarray(gene_chrom_num, dtype=np.int64)[gene]
+    has = (bins != _NO).reshape(n, 3, 3).any(axis=2)
+    tested = has.any(axis=1)
+    BIG = np.iinfo(np.int64).max
+    w = np.sort(np.where(has, pos // window, BIG), axis=1)
+    valid = w != BIG
+    valid[:, 1:] &= w[:, 1:] != w[:, :-1]
+    rows = np.where(valid, window_rows(win_map_off, win_map, cnum[:, None], np.where(valid, w, 0)), -1)
+    present = valid & (rows >= 0)
+    missing = (valid & (rows < 0)).any(axis=1)
+    y_pred, std, y_true = (np.asarray(x, dtype=np.float64) for x in (y_pred, std, y_true))
+    flag = np.asarray(flag).astype(bool)
+    counts = np.asarray(win_counts, dtype=np.int64)
+    rsum = counts.sum(axis=1)
+    mu, var, ro = np.zeros(n), np.zeros(n), np.zeros(n)
+    den = np.zeros(n)
+    fl = np.zeros(n, bool)
+    rsize = np.zeros(n, np.int64)
+    for u in range(3):
+        m, r = present[:, u], np.maximum(rows[:, u], 0)
+        mu = np.where(m, mu + y_pred[r], mu)
+        var = np.where(m, var + std[r] * std[r], var)
+        ro = np.where(m, ro + y_true[r], ro)
+        fl |= m & flag[r]
+        rsize += np.where(m, rsum[r], 0)
+        if denom_plus is not None:
+            den = np.where(m, den + np.where(minus, denom_minus[r], denom_plus[r]), den)
+    dp = np.concatenate([np.asarray(d_pr, dtype=np.float64), [0.0]])
+    b9 = np.where(bins == _NO, 192, bins)
+    num = np.zeros(n)
+    for s in range(9):
+        num = num + dp[b9[:, s]]
+    nw = present.sum(axis=1)
+    out = {"N_WIN": nw, "R_SIZE": rsize, "FLAG": fl, "MISSING": missing & tested, "R_OBS": ro, "PI_NUM": num}
+    nan = np.full(n, np.nan)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        out["MU"] = np.where(missing, nan, mu)
+        out["SIGMA"] = np.where(missing, nan, np.sqrt(var))
+        if denom_plus is not None:
+            out["PI_SUM"] = np.where(missing, nan, np.where(nw > 0, num / den, 0.0))
+    if not exact:
+        return out
+    # nonc_model's P_SUM: exact numerator and denominator, each rounded once, one division
+    limbs, e0 = int_limbs(dp[:192])
+    limbs193 = np.concatenate([limbs, np.zeros((len(limbs), 1), np.int64)], axis=1)
+    S_num = np.stack([limbs193[k][b9].sum(axis=1) for k in range(len(limbs))], axis=1)
+    g64 = limbs.reshape(len(limbs), 64, 3).sum(axis=2)               # sum_r limb[3 c + r]: R[j / 3] groups by c
+    rc = revcomp64()
+    Wp = np.stack([counts @ g64[k] for k in range(len(limbs))], axis=1)
+    Wm = np.stack([counts @ g64[k][rc] for k in range(len(limbs))], axis=1)
+    S_den = np.zeros((n, len(limbs)), np.int64)
+    for u in range(3):
+        m, r = present[:, u], np.maximum(rows[:, u], 0)
+        S_den += np.where(m[:, None], np.where(minus[:, None], Wm[r], Wp[r]), 0)
+    sel = np.flatnonzero(tested & ~missing)
+    exact = np.zeros(n)
+    if len(sel):
+        with np.errstate(divide="ignore", invalid="ignore"):
+            exact[sel] = limbs_to_float(S_num[sel], e0) / limbs_to_float(S_den[sel], e0)
+    out["PI_SUM_EXACT"] = np.where(missing, nan, exact)
+    return out

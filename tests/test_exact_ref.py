@@ -293,3 +293,249 @@ def test_nb_model_mutation_names_are_matched_without_chr():
         assert list(c) == want and list(s) == [5, 6, 7, 8]
         c, s = nb._mutation_starts((np.array(names), np.array([5, 6, 7, 8])))
         assert list(c) == want and list(s) == [5, 6, 7, 8]
+
+
+# ---------------------------------------------------------------- K9a-K9d, K10: the annotation and codon engine
+
+@pytest.fixture(scope="module")
+def cds_small(oracle):
+    """The 3.3 Mb genome and gene set of the small GPU fixtures (test_gpu_cds_annotation, test_gpu_codon) plus the
+    constructed edge set of the gene-set-size codon test, placed on the small genome."""
+    from digdriver_b200 import genome as G, pipeline
+    from oracle import cds_annot as O
+    from test_gpu_cds_annotation import LENGTHS, SEED, _as_dicts, _ascending, _concat, _edge_genes, _subset, _trim3
+    from codon_edges import edge_gene_set, n_runs
+    off, _ = G._layout(LENGTHS)
+    seqs = [oracle.synth_genome(int(o), int(n), SEED) for o, n in zip(off, LENGTHS)]
+    syn = pipeline.synth_genes(700, LENGTHS, 10_000, seed=3)
+    edge = edge_gene_set(LENGTHS, [n_runs(s) for s in seqs], 10_000, small=True)
+    genes = _concat(_trim3(_subset(syn, _ascending(*syn[2:]))), _edge_genes(), edge)
+    eng = X.cds_engine(lambda c, lo, n: seqs[c][lo:lo + n], LENGTHS, genes)
+    return dict(seqs=seqs, chroms=[O.Chrom(s) for s in seqs], genes=genes, dicts=_as_dicts(genes), eng=eng,
+                lengths=LENGTHS, n_edge=len(edge[0]) + 12)
+
+
+def test_engine_codons_match_the_plain_rules(cds_small):
+    """Every codon of every gene against tests/codon_oracle.codon_sites: position, amino acid, each slot's bin and
+    class; codons with an N have no sites and amino acid 0."""
+    import codon_oracle as C
+    from oracle import cds_annot as O
+    rec = X.codon_records_ref(cds_small["eng"])
+    ptr = rec["PTR"]
+    n_site = 0
+    for e, gd in enumerate(cds_small["dicts"]):
+        T = sum(t - s + 1 for s, t in gd["blocks"])
+        assert ptr[e + 1] - ptr[e] == T // 3
+        want = {c["codon"]: c for c in C.codon_sites(cds_small["chroms"][gd["chrom"]], gd)}
+        tpos = O.transcript_positions(gd)
+        for k in range(T // 3):
+            i = ptr[e] + k
+            assert tuple(rec["POS"][i]) == tuple(tpos[3 * k:3 * k + 3]), (e, k)
+            wc = want.get(k + 1)
+            bins, cls = np.full(9, 255), np.full(9, 255)
+            if wc is None:
+                assert rec["REF_AA"][i] == 0, (e, k)
+            else:
+                assert chr(rec["REF_AA"][i]) == wc["ref_aa"], (e, k)
+                for slot, _, _, _, b, name in wc["sites"]:
+                    bins[slot], cls[slot] = b, O.CLASS_CODE[name]
+            assert np.array_equal(rec["BIN"][i], bins) and np.array_equal(rec["CLASS"][i], cls), (e, k)
+            assert rec["N_SITES"][i] == (bins != 255).sum()
+            n_site += int((bins != 255).sum())
+    assert n_site > 500_000
+
+
+def test_engine_tables_match_the_plain_rules(cds_small):
+    from oracle import cds_annot as O
+    L, flags = X.cds_table_ref(cds_small["eng"])
+    for e, gd in enumerate(cds_small["dicts"]):
+        W, wf = O.gene_table(cds_small["chroms"][gd["chrom"]], gd)
+        assert wf == flags[e] and np.array_equal(W[:, :4], L[e]), e
+    assert (flags & O.FLAG_N).any() and (flags & O.FLAG_STOP).any() and (flags & O.FLAG_LENGTH).any()
+    assert L[:, :, 3].sum() > 0
+
+
+def _every_snv(cds_small, genes_idx, flank=7):
+    """(gene, position, genomic REF code, ALT code 0..4) of every base of each gene's blocks widened by `flank` (the
+    CDS, the splice positions and the intronic bases around them), every ALT."""
+    chrom, strand, ptr, bs, be = cds_small["genes"]
+    out = []
+    for e in genes_idx:
+        L = int(cds_small["lengths"][chrom[e]])
+        p = np.unique(np.concatenate([np.arange(max(s - flank, 0), min(t + flank + 1, L))
+                                      for s, t in zip(bs[ptr[e]:ptr[e + 1]], be[ptr[e]:ptr[e + 1]])]))
+        ref = X._BASE_CODE[cds_small["seqs"][chrom[e]][p]].astype(np.int64)
+        for a in range(5):
+            out.append(np.stack([np.full(len(p), e), p, ref, np.full(len(p), a)], axis=1))
+    return np.concatenate(out)
+
+
+def test_engine_snv_classes_and_codon_matches(cds_small):
+    """annotate_ref against oracle/cds_annot.snv_class, and snv_codons_ref against the codon oracle's sites, for every
+    SNV (REF as on the genome, and a wrong REF) at every position of a sample of genes and of the edge set."""
+    import codon_oracle as C
+    from oracle import cds_annot as O
+    eng, genes, dicts = cds_small["eng"], cds_small["genes"], cds_small["dicts"]
+    E = len(dicts)
+    rng = np.random.default_rng(8)
+    pick = np.unique(np.concatenate([rng.choice(E - cds_small["n_edge"], 40, replace=False),
+                                     np.arange(E - cds_small["n_edge"], E)]))
+    pick = [e for e in pick if genes[2][e + 1] - genes[2][e] < 1000]
+    snv = _every_snv(cds_small, pick)
+    e, p, ref, alt = snv.T
+    cls = X.annotate_ref(eng, genes, e, p, alt)
+    good_ref = (ref < 4) & (alt != ref)
+    ci, slot = X.snv_codons_ref(eng, genes, e, p, ref, alt)
+    wrong = (ref + 1 + rng.integers(0, 3, len(ref))) % 4
+    ci_w, _ = X.snv_codons_ref(eng, genes, e, p, np.where(ref < 4, wrong, ref), alt)
+    n_checked = 0
+    for g in pick:
+        gd = dicts[g]
+        ch = cds_small["chroms"][gd["chrom"]]
+        cache = (O.coding_sites(ch, gd), set(O.splice_positions(gd)))
+        sites = {}
+        ptr = eng["PTR"]
+        for c in C.codon_sites(ch, gd):
+            for slot_, pp, r_, a_, _, _ in c["sites"]:
+                sites[(pp, "ACGT".index(a_))] = (ptr[g] + c["codon"] - 1, slot_)
+        for i in np.flatnonzero(e == g):
+            a = int(alt[i])
+            want = O.snv_class(ch, gd, int(p[i]), "ACGT"[a], _cache=cache) if a < 4 else None
+            assert cls[i] == (255 if want is None else O.CLASS_CODE[want]), (g, p[i], a)
+            ws = sites.get((int(p[i]), a)) if good_ref[i] else None
+            assert (ci[i], slot[i]) == ((-1, 255) if ws is None else ws), (g, p[i], a)
+            assert ci_w[i] == -1
+            n_checked += 1
+    assert n_checked > 200_000 and (cls == 3).sum() > 100 and (ci >= 0).sum() > 50_000
+
+
+def _transfer_case(rng, n_codon=4000, n_win_chrom=60, W=1000):
+    """Random codon records over two chromosomes (numbers 1 and 2) of n_win_chrom windows each: one to three site
+    bases per codon in up to three windows, both strands; log-normal window parameters and d_pr."""
+    from digdriver_b200 import kernels
+    idx = np.array([(c, w * W) for c in (1, 2) for w in range(n_win_chrom)], dtype=np.int64)
+    off, wmap = kernels.build_window_map(idx[:, 0], idx[:, 1], W, 3)
+    nw = len(idx)
+    counts = rng.integers(0, 2000, (nw, 64)).astype(np.int32)
+    yp = rng.lognormal(np.log(10.0), 3.0, nw)
+    sd = rng.lognormal(np.log(3.0), 3.0, nw)
+    yt = np.round(rng.lognormal(np.log(20.0), 2.0, nw))
+    fl = rng.random(nw) < 0.2
+    d_pr = rng.lognormal(np.log(1e-6), 3.0, 192)
+    E = n_codon // 40
+    ptr = np.arange(E + 1, dtype=np.int64) * 40
+    gchrom = rng.integers(1, 3, E)
+    gstrand = np.where(rng.random(E) < 0.5, -1, 1).astype(np.int8)
+    start = rng.integers(0, (n_win_chrom - 3) * W, n_codon)
+    pos = start[:, None] + np.sort(rng.integers(0, 2 * W, (n_codon, 3)), axis=1)
+    bins = rng.integers(0, 192, (n_codon, 9)).astype(np.uint8)
+    bins[rng.random((n_codon, 9)) < 0.4] = 255
+    bins[::97] = 255                                          # codons without sites
+    rec = {"PTR": ptr, "POS": pos, "BIN": bins}
+    return rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr
+
+
+def test_codon_transfer_ref_matches_a_plain_loop():
+    """The vectorised K10 reference against a per-codon loop over codon_oracle.window_set's rule."""
+    import math
+    rng = np.random.default_rng(9)
+    rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr = _transfer_case(rng)
+    wmap = wmap.copy()
+    wmap[off[2] + 7] = -1                                     # a missing window
+    sub, rc = np.arange(192) // 3, X.revcomp64()
+    den_p = X.exact_dot_int(d_pr, counts[:, sub])
+    den_m = X.exact_dot_int(d_pr, counts[:, rc][:, sub])
+    ref = X.codon_transfer_ref(rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr, den_p, den_m)
+    n_miss = 0
+    for i in range(len(rec["BIN"])):
+        e = i // 40
+        b = rec["BIN"][i].astype(int)
+        sites = [(s, int(rec["POS"][i][s // 3])) for s in range(9) if b[s] != 255]
+        wins = sorted({p // W for _, p in sites})
+        rows = [int(wmap[off[gchrom[e]] + w]) if w < off[gchrom[e] + 1] - off[gchrom[e]] else -1 for w in wins]
+        have = [r for r in rows if r >= 0]
+        miss = len(have) < len(rows)
+        n_miss += miss
+        mu = var = ro = den = num = 0.0
+        for r in have:
+            mu += yp[r]
+            var += sd[r] * sd[r]
+            ro += yt[r]
+            den += den_m[r] if gstrand[e] < 0 else den_p[r]
+        for s, _ in sites:
+            num += d_pr[b[s]]
+        assert ref["N_WIN"][i] == len(have) and ref["MISSING"][i] == miss
+        assert ref["R_SIZE"][i] == sum(int(counts[r].sum()) for r in have)
+        assert ref["FLAG"][i] == any(fl[r] for r in have) and ref["R_OBS"][i] == ro and ref["PI_NUM"][i] == num
+        if not sites:
+            assert ref["MU"][i] == 0 and ref["PI_SUM"][i] == 0 and ref["PI_SUM_EXACT"][i] == 0
+        elif miss:
+            assert np.isnan(ref["MU"][i]) and np.isnan(ref["SIGMA"][i]) and np.isnan(ref["PI_SUM"][i])
+        else:
+            assert ref["MU"][i] == mu and ref["SIGMA"][i] == math.sqrt(var) and ref["PI_SUM"][i] == num / den
+            if i % 8 == 0:
+                R = sum(counts[r].astype(np.int64) for r in have)
+                R = R[rc] if gstrand[e] < 0 else R
+                D = X.exact_dot_int(d_pr, R[sub][None, :])[0]
+                assert ref["PI_SUM_EXACT"][i] == math.fsum(d_pr[b[s]] for s, _ in sites) / D
+    assert n_miss > 10
+
+
+def test_pi_sum_exact_matches_fraction():
+    from fractions import Fraction
+    rng = np.random.default_rng(10)
+    rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr = _transfer_case(rng, n_codon=400)
+    ref = X.codon_transfer_ref(rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr)
+    rc, sub = X.revcomp64(), np.arange(192) // 3
+    n = 0
+    for i in range(len(rec["BIN"])):
+        e = i // 40
+        b = [int(x) for x in rec["BIN"][i] if x != 255]
+        if not b:
+            continue
+        wins = sorted({int(rec["POS"][i][s // 3]) // W for s in range(9) if rec["BIN"][i][s] != 255})
+        R = sum(counts[int(wmap[off[gchrom[e]] + w])].astype(np.int64) for w in wins)
+        R = R[rc] if gstrand[e] < 0 else R
+        num = float(sum(Fraction(float(d_pr[j])) for j in b))
+        den = float(sum(Fraction(float(d_pr[j])) * int(R[sub[j]]) for j in range(192)))
+        assert ref["PI_SUM_EXACT"][i] == num / den, i
+        n += 1
+    assert n > 300
+
+
+# B, the bound of |kernel-order PI_SUM - PI_SUM_EXACT| in u, for nonnegative data:
+#   kernel denominator: each per-window denominator within 16 u of its exact value, then at most 2 additions of
+#     positive terms: relative error <= 16 + 2 = 18 u;
+#   kernel numerator: at most 8 additions of positive terms: <= 8 u;
+#   kernel division: 1 u;  PI_SUM_EXACT: numerator and denominator rounded once each and one division: 3 u.
+#   B = 18 + 8 + 1 + 3 = 30 u to first order; the second-order terms are below 1e-12 u, so B = 31 u.
+PI_SUM_BOUND_U = 31
+
+
+@pytest.fixture(scope="module")
+def transfer_model_case():
+    rng = np.random.default_rng(11)
+    case = _transfer_case(rng, n_codon=40_000, n_win_chrom=400)
+    rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr = case
+    sub, rc = np.arange(192) // 3, X.revcomp64()
+    return case, X.warp_dot_model(d_pr, counts[:, sub]), X.warp_dot_model(d_pr, counts[:, rc][:, sub])
+
+
+def test_kernel_order_pi_sum_within_bound(transfer_model_case):
+    """PI_SUM in the kernel's order, fed denominators in the warp kernel's order, is within B of PI_SUM_EXACT."""
+    (rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr), dp, dm = transfer_model_case
+    ref = X.codon_transfer_ref(rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr, dp, dm)
+    t = ref["N_WIN"] > 0
+    assert (ref["N_WIN"] == 3).sum() > 100
+    err = X._rel_err_u(ref["PI_SUM"][t], ref["PI_SUM_EXACT"][t])
+    print("\nkernel-order PI_SUM: worst %.2f u of PI_SUM_EXACT (B = %d u)" % (err.max(), PI_SUM_BOUND_U))
+    assert err.max() <= PI_SUM_BOUND_U
+
+
+def test_pi_sum_bound_rejects_plus_denominators_everywhere(transfer_model_case):
+    (rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr), dp, dm = transfer_model_case
+    ref = X.codon_transfer_ref(rec, gchrom, gstrand, W, off, wmap, counts, yp, sd, yt, fl, d_pr, dp, dp)
+    t = ref["N_WIN"] > 0
+    err = X._rel_err_u(ref["PI_SUM"][t], ref["PI_SUM_EXACT"][t])
+    print("\ndenom_plus for every gene: worst %.3g u" % err.max())
+    assert err.max() > 1e3 * PI_SUM_BOUND_U
